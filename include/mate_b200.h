@@ -17,7 +17,9 @@
  *   - "dev" pointers are device pointers owned by the caller (e.g. PyTorch tensors) on the
  *     device the handle was created for; "host" pointers are ordinary host memory;
  *   - batched I/O is row-major [B, N, D] float32 in the reference's feature order
- *     (mate/environment.py:908-983, mate/constants.py:267-300);
+ *     (mate/environment.py:908-983, mate/constants.py:267-300); the observation rows
+ *     (the ``float* cam_obs / tgt_obs`` arguments) may instead be float16 per handle, see
+ *     mate_b200_set_observation_format: the arguments then address buffers of that type;
  *   - a handle is not re-entrant; different handles are independent (one per GPU);
  *   - step/reset/observe enqueue work on the given stream and never synchronise the host.
  */
@@ -150,10 +152,21 @@ int mate_b200_destroy(MateSim* sim);
 /* Observation row widths: Dc, Dt (constants.py:267-300). */
 int mate_b200_obs_dims(const MateSim* sim, int32_t* cam_dim, int32_t* tgt_dim);
 
+/* Element type of the observation rows this handle writes: MATE_OBS_FORMAT_F32 (the default) or MATE_OBS_FORMAT_F16.
+ * The float16 rows are the float32 rows of the same call rounded once to nearest even; the simulation, the masks, the
+ * registered observation wrappers, rewards, done, auxiliary outputs and actions are unchanged (float32).  After
+ * MATE_OBS_FORMAT_F16 the `float* cam_obs / tgt_obs` arguments of mate_b200_reset, _step, _observe and _step_host
+ * address float16 buffers of the same shapes (cast the pointers), and mate_b200_transform_observations is refused
+ * (register the wrappers with mate_b200_set_observation_ops instead).  Allowed only before the handle's first reset,
+ * step, step_host or observe (MATE_ESTATE afterwards); an unknown code is MATE_EINVAL. */
+#define MATE_OBS_FORMAT_F32 0
+#define MATE_OBS_FORMAT_F16 1
+int mate_b200_set_observation_format(MateSim* sim, int32_t format);
+
 /* MultiAgentTracking.reset (environment.py:679-834) for the envs with env_mask[b] != 0
  * (dev, NULL = all); Philox streams keyed on (seed, global env index, episode id).
  * Writes the first joint observation of the reset envs (other rows are rewritten with
- * their current observation). */
+ * their current observation); cam_obs / tgt_obs in the handle's observation format. */
 int mate_b200_reset(MateSim* sim, const uint8_t* env_mask, uint64_t seed,
                     float* cam_obs, float* tgt_obs, void* stream);
 
@@ -167,7 +180,7 @@ int mate_b200_seed(MateSim* sim, const uint8_t* env_mask, uint64_t seed, void* s
 /* MultiAgentTracking.step (environment.py:590-676) for all envs: _simulate,
  * _update_view, _assign_goals, joint_observation, reward/done.
  *   cam_act [B,Nc,2], tgt_act [B,Nt,2] float32 dev (finite);
- *   cam_obs [B,Nc,Dc], tgt_obs [B,Nt,Dt] float32 dev;
+ *   cam_obs [B,Nc,Dc], tgt_obs [B,Nt,Dt] dev, float32 or float16 (mate_b200_set_observation_format);
  *   rewards [B,2] float32 dev = (camera_team_reward, target_team_reward);
  *   done [B] uint8 dev. */
 int mate_b200_step(MateSim* sim, const float* cam_act, const float* tgt_act,
@@ -176,7 +189,8 @@ int mate_b200_step(MateSim* sim, const float* cam_act, const float* tgt_act,
                    void* stream);
 
 /* joint_observation() of the current state without stepping (_update_view +
- * joint_observation, environment.py:1356-1388, 908-983); used after set_state. */
+ * joint_observation, environment.py:1356-1388, 908-983); used after set_state.  cam_obs / tgt_obs in the
+ * handle's observation format. */
 int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs,
                       const MateStepAux* aux, const MateReplay* replay, void* stream);
 
@@ -192,7 +206,7 @@ int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs,
  * (INTEGRATION.md), compacted: non-zero 16-byte chunks only, or -- with MATE_STEP_HOST_ROWS_KEPT -- only the 64-byte
  * groups that differ from the previous call's rows; host threads of the library put them in place before the call
  * returns.  The buffers hold the same bytes in every case.  Row buffers must be 4-byte aligned (16-byte aligned for full
- * speed). */
+ * speed) and of the handle's observation format (float16 rows halve the bytes on the link). */
 int mate_b200_step_host(MateSim* sim, const float* cam_act, const float* tgt_act,
                         float* cam_obs, float* tgt_obs, float* rewards, uint8_t* done,
                         uint32_t flags);
@@ -217,7 +231,8 @@ int mate_b200_episode_stats(MateSim* sim, float* out16, int32_t reset_after, voi
  *   MATE_OBS_RESCALED                   normalize_observation, mate/agents/utils.py:97-127 (RescaledObservation)
  * `ops` is a HOST array of num_ops <= MATE_MAX_OBS_OPS codes.  cam_affine [Dc][2] / tgt_affine [Dt][2] are dev
  * arrays of (scale, shift) per observation column, needed (non-NULL) only with MATE_OBS_RESCALED.  cam_obs /
- * tgt_obs must hold the observations the last step/reset/observe call wrote for this handle. */
+ * tgt_obs must hold the observations the last step/reset/observe call wrote for this handle.  float32 handles only
+ * (MATE_EINVAL after MATE_OBS_FORMAT_F16). */
 #define MATE_OBS_ENHANCED_CAMERA 1
 #define MATE_OBS_ENHANCED_TARGET 2
 #define MATE_OBS_SHARED_CAMERA 3

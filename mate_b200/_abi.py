@@ -20,6 +20,8 @@ c_int8_p = ctypes.POINTER(ctypes.c_int8)
 
 MATE_STEP_AUTO_RESET = 1
 MATE_STEP_HOST_ROWS_KEPT = 2
+MATE_OBS_FORMAT_F32 = 0
+MATE_OBS_FORMAT_F16 = 1
 
 
 class MateConfig(ctypes.Structure):
@@ -174,6 +176,7 @@ def load_library():
     lib.mate_b200_create.argtypes = [ctypes.POINTER(MateConfig), ctypes.c_int32, ctypes.c_int32, ctypes.c_int64, ctypes.POINTER(void_p)]
     lib.mate_b200_destroy.argtypes = [void_p]
     lib.mate_b200_obs_dims.argtypes = [void_p, c_int32_p, c_int32_p]
+    lib.mate_b200_set_observation_format.argtypes = [void_p, ctypes.c_int32]
     lib.mate_b200_reset.argtypes = [void_p, void_p, ctypes.c_uint64, void_p, void_p, void_p]
     lib.mate_b200_seed.argtypes = [void_p, void_p, ctypes.c_uint64, void_p]
     lib.mate_b200_step.argtypes = [void_p, void_p, void_p, void_p, void_p, void_p, void_p,
@@ -197,7 +200,7 @@ def load_library():
     lib.mate_b200_greedy_camera_actions.argtypes = [void_p, void_p, void_p, void_p, ctypes.c_uint64, ctypes.c_uint64,
                                                     ctypes.POINTER(MateCameraAgentReplay), void_p, void_p]
     lib.mate_b200_soft_coverage.argtypes = [void_p, void_p, void_p, void_p, void_p]
-    for name in ('create', 'destroy', 'obs_dims', 'reset', 'seed', 'step', 'observe', 'step_host',
+    for name in ('create', 'destroy', 'obs_dims', 'set_observation_format', 'reset', 'seed', 'step', 'observe', 'step_host',
                  'get_state', 'set_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions'):
         getattr(lib, 'mate_b200_' + name).restype = ctypes.c_int
     _LIB = lib
@@ -206,7 +209,7 @@ def load_library():
 
 EXPORTED_SYMBOLS = [
     'mate_b200_last_error', 'mate_b200_abi_version', 'mate_b200_create', 'mate_b200_destroy',
-    'mate_b200_obs_dims', 'mate_b200_reset', 'mate_b200_seed', 'mate_b200_step', 'mate_b200_observe',
+    'mate_b200_obs_dims', 'mate_b200_set_observation_format', 'mate_b200_reset', 'mate_b200_seed', 'mate_b200_step', 'mate_b200_observe',
     'mate_b200_step_host', 'mate_b200_get_state', 'mate_b200_set_state',
     'mate_b200_episode_stats', 'mate_b200_launch_count', 'mate_b200_host_leg_info', 'mate_b200_transform_observations', 'mate_b200_set_observation_ops',
     'mate_b200_decode_actions', 'mate_b200_auxiliary_terms', 'mate_b200_fov_range', 'mate_b200_soft_coverage', 'mate_b200_greedy_target_actions', 'mate_b200_greedy_camera_actions',

@@ -195,6 +195,8 @@ struct MateSim {
     int refill_mode = 0;      // 0 = off, 1 = side stream every refill_period steps, 2 = same stream after every step (tests)
     int refill_period = 512;
     int tile_envs = 32;       // environments per warp tile (Params::tile_envs), chosen from the batch size at creation
+    int obs_format = MATE_OBS_FORMAT_F32;   // element type of the observation rows (mate_b200_set_observation_format)
+    bool rows_written = false;              // a reset / step / step_host / observe has run: the format is fixed
     long long steps_since_refill = 0;
     // host-path (step_host) resources
     static constexpr int kHostStreams = 4;
@@ -423,6 +425,23 @@ extern "C" int mate_b200_obs_dims(const MateSim* sim, int32_t* cam_dim, int32_t*
     return MATE_OK;
 }
 
+// bytes of one value of the observation rows in the handle's format
+static size_t obs_elem_bytes(const MateSim* sim) { return sim->obs_format == MATE_OBS_FORMAT_F16 ? 2 : 4; }
+// `base` advanced by `values` values of the observation rows (the row pointers are typed float* in the ABI)
+static float* obs_advance(const MateSim* sim, float* base, size_t values) {
+    return reinterpret_cast<float*>(reinterpret_cast<char*>(base) + values * obs_elem_bytes(sim));
+}
+
+extern "C" int mate_b200_set_observation_format(MateSim* sim, int32_t format) {
+    if (!sim) return fail(MATE_EINVAL, "null handle");
+    if (format != MATE_OBS_FORMAT_F32 && format != MATE_OBS_FORMAT_F16) return fail(MATE_EINVAL, "unknown observation format code");
+    if (sim->rows_written)
+        return fail(MATE_ESTATE, "the observation format can only be set before the handle's first reset, step, step_host or observe");
+    sim->obs_format = format;
+    sim->base.obs_format = format;
+    return MATE_OK;
+}
+
 extern "C" int mate_b200_fov_range(MateSim* sim, const int32_t* env, const int32_t* camera, const double* angle_deg,
                                    double* out, int64_t n, void* stream) {
     if (!sim || !env || !camera || !angle_deg || !out || n < 0) return fail(MATE_EINVAL, "bad argument");
@@ -449,6 +468,8 @@ extern "C" int mate_b200_transform_observations(MateSim* sim, float* cam_obs, fl
                                                 void* stream) {
     if (!sim || !tgt_obs || (sim->cfg.num_cameras > 0 && !cam_obs) || (num_ops > 0 && !ops)) return fail(MATE_EINVAL, "null argument");
     if (num_ops < 0 || num_ops > MATE_MAX_OBS_OPS) return fail(MATE_EINVAL, "too many observation wrappers (MATE_MAX_OBS_OPS)");
+    if (sim->obs_format != MATE_OBS_FORMAT_F32)
+        return fail(MATE_EINVAL, "transform_observations works on float32 rows; register the wrappers (set_observation_ops) on a float16 handle");
     if (num_ops == 0) return MATE_OK;
     if (((uintptr_t)cam_obs & 15) || ((uintptr_t)tgt_obs & 15)) return fail(MATE_EINVAL, "observation buffers must be 16-byte aligned");
     ObsOps o{};
@@ -617,8 +638,8 @@ static int launch_range(MateSim* sim, Params p, int begin, int count, cudaStream
     p.tgt_pack += begin; p.cargo += begin; p.env_a += begin; p.env_b += begin; p.cc_clear += begin;
     if (p.cam_act) p.cam_act += (size_t)begin * nc * 2;
     if (p.tgt_act) p.tgt_act += (size_t)begin * nt * 2;
-    if (p.cam_obs) p.cam_obs += (size_t)begin * nc * dc;
-    if (p.tgt_obs) p.tgt_obs += (size_t)begin * nt * dt;
+    if (p.cam_obs) p.cam_obs = obs_advance(sim, p.cam_obs, (size_t)begin * nc * dc);
+    if (p.tgt_obs) p.tgt_obs = obs_advance(sim, p.tgt_obs, (size_t)begin * nt * dt);
     if (p.rewards) p.rewards += (size_t)begin * 2;
     if (p.done) p.done += begin;
     if (p.env_mask) p.env_mask += begin;
@@ -719,6 +740,7 @@ extern "C" int mate_b200_reset(MateSim* sim, const uint8_t* env_mask, uint64_t s
     if (int rc = check_obs_alignment(cam_obs, tgt_obs)) return rc;
     CUDA_TRY(cudaSetDevice(sim->device));
     sim->seed = seed;
+    sim->rows_written = true;
     Params p = sim->base;
     p.mode = MODE_RESET; p.flags = 0; p.seed = seed;
     p.cam_obs = cam_obs; p.tgt_obs = tgt_obs; p.env_mask = env_mask;
@@ -737,6 +759,7 @@ extern "C" int mate_b200_step(MateSim* sim, const float* cam_act, const float* t
     if (((uintptr_t)cam_act & 7) || ((uintptr_t)tgt_act & 7) || ((uintptr_t)rewards & 7)) return fail(MATE_EINVAL, "action/reward buffers must be 8-byte aligned");
     if (int rc = check_aux_alignment(aux)) return rc;
     CUDA_TRY(cudaSetDevice(sim->device));
+    sim->rows_written = true;
     Params p = sim->base;
     p.mode = MODE_STEP; p.flags = flags; p.seed = sim->seed;
     p.cam_act = cam_act; p.tgt_act = tgt_act; p.cam_obs = cam_obs; p.tgt_obs = tgt_obs; p.rewards = rewards; p.done = done;
@@ -754,6 +777,7 @@ extern "C" int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs, c
     if (int rc = check_obs_alignment(cam_obs, tgt_obs)) return rc;
     if (int rc = check_aux_alignment(aux)) return rc;
     CUDA_TRY(cudaSetDevice(sim->device));
+    sim->rows_written = true;
     Params p = sim->base;
     p.mode = MODE_OBSERVE; p.flags = 0; p.seed = sim->seed;
     p.cam_obs = cam_obs; p.tgt_obs = tgt_obs;
@@ -797,9 +821,10 @@ static int ensure_host_path(MateSim* sim) {
     // copy densely
     sim->compact_mode = threads >= 14 ? 1 : ((threads >= 5 || (threads >= 3 && sharers >= 4)) ? 2 : 0);
     if (const char* v = getenv("MATE_B200_HOST_COMPACT")) sim->compact_mode = v[0] == '1' ? 1 : (v[0] == '2' ? 2 : 0);
-    if ((sizeof(float) * nc * sim->kernel.dc) % 16 || (sizeof(float) * nt * sim->kernel.dt) % 16) sim->compact_mode = 0;
+    const size_t esz = obs_elem_bytes(sim);
+    if ((esz * nc * sim->kernel.dc) % 16 || (esz * nt * sim->kernel.dt) % 16) sim->compact_mode = 0;
     if (sim->compact_mode) {
-        const size_t region_bytes[2] = {sizeof(float) * B * nc * sim->kernel.dc, sizeof(float) * B * nt * sim->kernel.dt};
+        const size_t region_bytes[2] = {esz * B * nc * sim->kernel.dc, esz * B * nt * sim->kernel.dt};
         bool ok = true;
         for (int r = 0; r < 2 && ok; ++r) {
             if (region_bytes[r] == 0) continue;
@@ -833,6 +858,7 @@ extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const flo
     const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets;
     if (nc > 0 && (!cam_act || !cam_obs)) return fail(MATE_EINVAL, "null camera buffers");
     CUDA_TRY(cudaSetDevice(sim->device));
+    sim->rows_written = true;
     if (int rc = ensure_host_path(sim)) return rc;
     const int dc = sim->kernel.dc, dt = sim->kernel.dt;
     const int B = sim->num_envs;
@@ -868,7 +894,7 @@ extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const flo
         const auto t_start = std::chrono::steady_clock::now();
         auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count(); };
         double t_enq = 0, t_counts = 0, t_last_stream = 0;
-        const size_t per_env[2] = {(size_t)nc * dc * 4, (size_t)nt * dt * 4};   // bytes of rows per environment and region
+        const size_t per_env[2] = {(size_t)nc * dc * obs_elem_bytes(sim), (size_t)nt * dt * obs_elem_bytes(sim)};   // bytes of rows per environment and region
         float* const host_rows[2] = {cam_obs, tgt_obs};
         float* const dev_rows[2] = {rows_now[0], rows_now[1]};
         std::vector<long long> table_base(2 * (num_chunks + 1), 0);
@@ -970,13 +996,14 @@ extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const flo
         if (nc) CUDA_TRY(cudaMemcpyAsync(sim->h_cam_act + (size_t)begin * nc * 2, cam_act + (size_t)begin * nc * 2, sizeof(float) * count * nc * 2, cudaMemcpyHostToDevice, s));
         CUDA_TRY(cudaMemcpyAsync(sim->h_tgt_act + (size_t)begin * nt * 2, tgt_act + (size_t)begin * nt * 2, sizeof(float) * count * nt * 2, cudaMemcpyHostToDevice, s));
         if (int rc = launch_range(sim, p, begin, count, s)) return rc;
-        if (nc) CUDA_TRY(cudaMemcpyAsync(cam_obs + (size_t)begin * nc * dc, rows_now[0] + (size_t)begin * nc * dc, sizeof(float) * count * nc * dc, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaMemcpyAsync(tgt_obs + (size_t)begin * nt * dt, rows_now[1] + (size_t)begin * nt * dt, sizeof(float) * count * nt * dt, cudaMemcpyDeviceToHost, s));
+        const size_t esz = obs_elem_bytes(sim);
+        if (nc) CUDA_TRY(cudaMemcpyAsync(obs_advance(sim, cam_obs, (size_t)begin * nc * dc), obs_advance(sim, rows_now[0], (size_t)begin * nc * dc), esz * count * nc * dc, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaMemcpyAsync(obs_advance(sim, tgt_obs, (size_t)begin * nt * dt), obs_advance(sim, rows_now[1], (size_t)begin * nt * dt), esz * count * nt * dt, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(cudaMemcpyAsync(rewards + (size_t)begin * 2, sim->h_rewards + (size_t)begin * 2, sizeof(float) * count * 2, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(cudaMemcpyAsync(done + begin, sim->h_done + begin, count, cudaMemcpyDeviceToHost, s));
     }
     for (int i = 0; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamSynchronize(sim->hstreams[i]));
-    sim->last_leg = 0; sim->last_link_bytes = (unsigned long long)B * ((size_t)nc * dc + (size_t)nt * dt) * sizeof(float);
+    sim->last_leg = 0; sim->last_link_bytes = (unsigned long long)B * ((size_t)nc * dc + (size_t)nt * dt) * obs_elem_bytes(sim);
     if (two_buffers) {   // the caller's buffers and the device hold this call's rows: the next call may send changes only
         sim->kept_rows[0] = cam_obs; sim->kept_rows[1] = tgt_obs; sim->kept_valid = true; sim->row_parity ^= 1;
     }

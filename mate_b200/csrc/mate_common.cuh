@@ -98,6 +98,7 @@ struct Params {
     double tgt_step_size, tgt_sight_range, transmittance;
     double obs_r_low, obs_r_high;
     const double* cam_ranges; const double* tgt_ranges; const double* obs_ranges;  // device [N][4]
+    int obs_format;    // element type of cam_obs / tgt_obs: MATE_OBS_FORMAT_F32 or _F16 (mate_b200_set_observation_format)
 };
 
 // ---- small math helpers --------------------------------------------------------------------

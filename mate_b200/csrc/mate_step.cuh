@@ -30,6 +30,10 @@
 //     are handed from the simulation phase to this phase through shared memory.
 #pragma once
 
+#include <cuda_fp16.h>
+
+#include <type_traits>
+
 #include "mate_common.cuh"
 #include "mate_wrappers.cuh"
 
@@ -630,12 +634,23 @@ __device__ __noinline__ void fold_obs_ops(const Params& p, const int env, float*
     apply_obs_ops<NC, NT, NO>(p, p.obs_ops, env, stage, stage + S::STAGE_CAM, scratch, p.cam_affine, p.tgt_affine);
 }
 
+// two fp32 values rounded to float16 (nearest even), `lo` at the lower address
+__device__ __forceinline__ uint32_t half2_bits(const float lo, const float hi) {
+    const __half2 h = __float22half2_rn(make_float2(lo, hi));
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
+
 // FOLD = the instantiation that also applies the registered observation wrappers (FoldOps, mate_common.cuh) while
 // the rows are composed; the common case (no wrappers) runs the FOLD = false instantiation, which has none of it.
-template <int NC, int NT, int NO, bool FOLD>
+// OutT = element type of the rows in HBM (Params::obs_format): float, or __half rounded once from the staged fp32 rows
+// while they leave the SM.  Everything before the copy-out is the same for both.
+template <int NC, int NT, int NO, bool FOLD, class OutT>
 __device__ __noinline__ void pack_observations(const Params& p, const int env0, const int nvalid, float* stage,
                                                const uint32_t* mk, const float* val, float* ops_scratch) {
     using S = Shape2<NC, NT, NO>;
+    constexpr bool F16 = std::is_same<OutT, __half>::value;
+    static_assert(F16 || std::is_same<OutT, float>::value, "observation rows are float or __half");
+    static_assert(!(F16 && MATE2_COPYOUT == 0), "the bulk copy (MATE2_COPYOUT=0) moves bytes unchanged: float16 rows need MATE2_COPYOUT=1");
     constexpr int R = S::R, MW = S::MW, DC = S::DC, DT = S::DT, CV = S::CV;
     constexpr int NCX = NC > 0 ? NC : 1;
     constexpr uint32_t FULLMASK = 0xffffffffu;
@@ -654,8 +669,8 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     // launch parameters used inside the loop, read once (a reference to the parameter block is a generic
     // pointer: the compiler would re-load through it after every store)
     const size_t bp = p.bpad;
-    float* const cam_obs0 = p.cam_obs + (size_t)env0 * S::CAM_ROW;
-    float* const tgt_obs0 = p.tgt_obs + (size_t)env0 * S::TGT_ROW;
+    OutT* const cam_obs0 = reinterpret_cast<OutT*>(p.cam_obs) + (size_t)env0 * S::CAM_ROW;
+    OutT* const tgt_obs0 = reinterpret_cast<OutT*>(p.tgt_obs) + (size_t)env0 * S::TGT_ROW;
     const float4* const obs_f4 = p.obs_f4;
     // The warp walks over its environments and assembles the 6 KB block of observation rows of one
     // environment in shared memory, every float written exactly once and without branches:
@@ -1047,7 +1062,47 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
         }
         // ---- staged rows -> HBM
         static_assert(!(S::BULK && S::CAM_SKEW != 0), "the 16-byte copy of the whole block expects dense camera rows");
-        if (S::BULK && MATE2_COPYOUT == 1) {
+        if constexpr (F16) {
+            // float16 rows: the lanes read the staged fp32 values, round them in pairs (__float22half2_rn, nearest even)
+            // and store each team's part with the widest store its size allows -- 16, 8, 4 or 2 bytes (part i starts at a
+            // multiple of gcd(16, part bytes) of the 16-byte aligned buffers); camera rows staged `skew` floats apart
+            __syncwarp();
+            auto copy_part_f16 = [&](__half* dst, const float* src, auto n_c, auto row_c, auto skew_c) {
+                constexpr int n = decltype(n_c)::value, row = decltype(row_c)::value, skew = decltype(skew_c)::value;
+                constexpr int W = n % 8 == 0 ? 8 : (n % 4 == 0 ? 4 : (n % 2 == 0 ? 2 : 1));   // values per store
+                static_assert(skew == 0 || (row % W == 0 && skew % 4 == 0), "a store must not straddle two skewed rows");
+                auto at = [](const int f) { return skew ? f + (f / row) * skew : f; };       // staged index of value f
+#pragma unroll
+                for (int it = 0; it < (n / W + 31) / 32; ++it) {
+                    const int k = it * 32 + lane;
+                    if (k < n / W) {
+                        if constexpr (W == 8) {
+                            // lanes 4-7 of every quarter-warp read their two 16-byte halves in the other order: each of the
+                            // two loads then covers eight distinct 16-byte bank groups per quarter-warp
+                            const int sw = (lane >> 2) & 1;
+                            const float4 a = *reinterpret_cast<const float4*>(src + at(8 * k + 4 * sw));
+                            const float4 b = *reinterpret_cast<const float4*>(src + at(8 * k + 4 - 4 * sw));
+                            const float4 lo = sw ? b : a, hi = sw ? a : b;
+                            __stcs(reinterpret_cast<uint4*>(dst) + k, make_uint4(half2_bits(lo.x, lo.y), half2_bits(lo.z, lo.w),
+                                                                                 half2_bits(hi.x, hi.y), half2_bits(hi.z, hi.w)));
+                        } else if constexpr (W == 4) {
+                            const float4 a = *reinterpret_cast<const float4*>(src + at(4 * k));
+                            __stcs(reinterpret_cast<uint2*>(dst) + k, make_uint2(half2_bits(a.x, a.y), half2_bits(a.z, a.w)));
+                        } else if constexpr (W == 2) {
+                            const float2 a = *reinterpret_cast<const float2*>(src + at(2 * k));
+                            __stcs(reinterpret_cast<unsigned int*>(dst) + k, half2_bits(a.x, a.y));
+                        } else {
+                            __stcs(reinterpret_cast<unsigned short*>(dst) + k, __half_as_ushort(__float2half_rn(src[at(k)])));
+                        }
+                    }
+                }
+            };
+            if (NC > 0) copy_part_f16(cam_obs0 + (size_t)i * S::CAM_ROW, stage, std::integral_constant<int, S::CAM_ROW>{},
+                                      std::integral_constant<int, (DC > 0 ? DC : 1)>{}, std::integral_constant<int, DCS - DC>{});
+            copy_part_f16(tgt_obs0 + (size_t)i * S::TGT_ROW, stage + S::STAGE_CAM, std::integral_constant<int, S::TGT_ROW>{},
+                          std::integral_constant<int, 1>{}, std::integral_constant<int, 0>{});
+            __syncwarp();
+        } else if (S::BULK && MATE2_COPYOUT == 1) {
             // plain 16-byte copies: every warp store covers 512 contiguous bytes; unlike the bulk copy there
             // is nothing to wait for before the block is reused (MATE2_COPYOUT, see DESIGN.md)
             __syncwarp();
@@ -1836,8 +1891,13 @@ mate_step_kernel2(const __grid_constant__ Params p) {
 
     // ------------------------------------------------------------------ joint_observation (environment.py:908-983)
     TL_MARK(5);
-    if (p.obs_ops.n > 0) pack_observations<NC, NT, NO, true>(p, env0, nvalid, stage, mk, val, reinterpret_cast<float*>(wbase + S::WARP_BYTES));
-    else pack_observations<NC, NT, NO, false>(p, env0, nvalid, stage, mk, val, nullptr);
+    if (p.obs_format == MATE_OBS_FORMAT_F16) {
+        if (p.obs_ops.n > 0) pack_observations<NC, NT, NO, true, __half>(p, env0, nvalid, stage, mk, val, reinterpret_cast<float*>(wbase + S::WARP_BYTES));
+        else pack_observations<NC, NT, NO, false, __half>(p, env0, nvalid, stage, mk, val, nullptr);
+    } else {
+        if (p.obs_ops.n > 0) pack_observations<NC, NT, NO, true, float>(p, env0, nvalid, stage, mk, val, reinterpret_cast<float*>(wbase + S::WARP_BYTES));
+        else pack_observations<NC, NT, NO, false, float>(p, env0, nvalid, stage, mk, val, nullptr);
+    }
     TL_MARK(6);
 }
 

@@ -46,10 +46,23 @@ def rescale_tables(nc, nt, no):
     return tuple(tables)
 
 
-class BatchedSim:
-    """One batch of MultiAgentTracking environments resident on one GPU."""
+OBSERVATION_FORMATS = {torch.float32: _abi.MATE_OBS_FORMAT_F32, torch.float16: _abi.MATE_OBS_FORMAT_F16}
 
-    def __init__(self, flat_config, num_envs, device=0, env_index_base=0):
+
+def check_observation_dtype(dtype):
+    """The element type of the observation rows: ``torch.float32`` or ``torch.float16`` (rounded once, to nearest even,
+    from the float32 rows), else ``ValueError``."""
+    if dtype not in OBSERVATION_FORMATS:
+        raise ValueError(f'observation_dtype must be torch.float32 or torch.float16, got {dtype!r}')
+    return dtype
+
+
+class BatchedSim:
+    """One batch of MultiAgentTracking environments resident on one GPU.  ``observation_dtype`` is the element type of
+    the observation rows (``cam_obs`` / ``tgt_obs``); everything else stays float32."""
+
+    def __init__(self, flat_config, num_envs, device=0, env_index_base=0, observation_dtype=torch.float32):
+        self.observation_dtype = check_observation_dtype(observation_dtype)
         if not torch.cuda.is_available():
             raise RuntimeError('mate_b200 needs a CUDA device (there is no CPU fallback)')
         self.lib = _abi.load_library()
@@ -64,12 +77,13 @@ class BatchedSim:
         self.handle = ctypes.c_void_p()
         _check(self.lib, self.lib.mate_b200_create(ctypes.byref(self._cfg_struct), self.B, self.device.index,
                                                    int(env_index_base), ctypes.byref(self.handle)))
+        _check(self.lib, self.lib.mate_b200_set_observation_format(self.handle, OBSERVATION_FORMATS[self.observation_dtype]))
         dc, dt = ctypes.c_int32(), ctypes.c_int32()
         _check(self.lib, self.lib.mate_b200_obs_dims(self.handle, ctypes.byref(dc), ctypes.byref(dt)))
         self.dc, self.dt = dc.value, dt.value
         dev = self.device
-        self.cam_obs = torch.zeros((self.B, self.nc, self.dc), dtype=torch.float32, device=dev)
-        self.tgt_obs = torch.zeros((self.B, self.nt, self.dt), dtype=torch.float32, device=dev)
+        self.cam_obs = torch.zeros((self.B, self.nc, self.dc), dtype=self.observation_dtype, device=dev)
+        self.tgt_obs = torch.zeros((self.B, self.nt, self.dt), dtype=self.observation_dtype, device=dev)
         self.rewards = torch.zeros((self.B, 2), dtype=torch.float32, device=dev)
         self.done = torch.zeros((self.B,), dtype=torch.uint8, device=dev)
         self._stats = torch.zeros(16, dtype=torch.float32, device=dev)
@@ -276,8 +290,12 @@ class BatchedSim:
         """Host-buffer step: `cam_act`/`tgt_act` and the tensors in `out` (cam_obs, tgt_obs,
         rewards, done) are CPU tensors (pinned for full PCIe speed).  `rows_kept=True` promises that
         `out` is the tuple of the previous `step_host` call and has not been written to since
-        (MATE_STEP_HOST_ROWS_KEPT, include/mate_b200.h): parts of the rows that stay zero are then not rewritten."""
+        (MATE_STEP_HOST_ROWS_KEPT, include/mate_b200.h): parts of the rows that stay zero are then not rewritten.
+        cam_obs / tgt_obs have the simulator's ``observation_dtype``."""
         cam_obs, tgt_obs, rewards, done = out
+        for name, rows in (('cam_obs', cam_obs if self.nc else None), ('tgt_obs', tgt_obs)):
+            if rows is not None and rows.dtype != self.observation_dtype:   # the C call sees only a pointer
+                raise ValueError(f'step_host: {name} is {rows.dtype}, the simulator writes {self.observation_dtype} rows')
         flags = (_abi.MATE_STEP_AUTO_RESET if auto_reset else 0) | (_abi.MATE_STEP_HOST_ROWS_KEPT if rows_kept else 0)
         _check(self.lib, self.lib.mate_b200_step_host(
             self.handle, _dptr(cam_act) if self.nc else None, _dptr(tgt_act),
