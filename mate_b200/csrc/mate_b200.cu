@@ -13,6 +13,7 @@
 #include <sched.h>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "mate_step.cuh"
@@ -204,7 +205,7 @@ struct MateSim {
     cudaEvent_t hevents[kHostStreams] = {};
     float *h_cam_act = nullptr, *h_tgt_act = nullptr, *h_cam_obs = nullptr, *h_tgt_obs = nullptr, *h_rewards = nullptr;
     uint8_t* h_done = nullptr;
-    bool host_ready = false;
+    bool host_ready = false;                  // ensure_host_path has run to the end
     size_t l2_window = 0;                     // bytes of obs_f4 the step launches keep in the L2 (0: none), see l2_keep_acquire
     // compacted device -> host leg (mate_hostpath.cuh): region 0 = camera rows, 1 = target rows
     static constexpr int kMaxHostChunks = 64;
@@ -227,12 +228,69 @@ struct MateSim {
     cudaEvent_t e_counts[kMaxHostChunks] = {}, e_stream[kMaxHostChunks] = {}, e_tables[kMaxHostChunks] = {};
     unsigned int* p_count_dev = nullptr;      // device address of the pinned p_count (the sizes are stored there by a kernel, not copied)
     std::unique_ptr<ExpandPool> pool;
+
+    // Releases whatever mate_b200_create and ensure_host_path have made, also when either stopped part-way.
+    ~MateSim() {
+        for (int i = 0; i < kHostStreams; ++i) { if (hstreams[i]) cudaStreamDestroy(hstreams[i]); if (hevents[i]) cudaEventDestroy(hevents[i]); }
+        cudaFree(h_cam_act); cudaFree(h_tgt_act); cudaFree(h_cam_obs); cudaFree(h_tgt_obs);
+        cudaFree(h_rewards); cudaFree(h_done);
+        pool.reset();   // before the events its threads wait on and the pinned buffers they read
+        for (int r = 0; r < 2; ++r) { cudaFree(d_compact[r]); cudaFree(d_table[r]); cudaFreeHost(p_compact[r]); cudaFreeHost(p_table[r]); cudaFree(h_rows2[r]); }
+        cudaFree(d_count); cudaFreeHost(p_count);
+        if (copy_stream) cudaStreamDestroy(copy_stream);
+        for (int i = 0; i < kMaxHostChunks; ++i) {
+            if (e_counts[i]) cudaEventDestroy(e_counts[i]);
+            if (e_stream[i]) cudaEventDestroy(e_stream[i]);
+            if (e_tables[i]) cudaEventDestroy(e_tables[i]);
+        }
+        if (side) { cudaStreamSynchronize(side); cudaStreamDestroy(side); }
+        if (side_event) cudaEventDestroy(side_event);
+        cudaFree(soft_edges);
+        cudaFree(next_block);
+        cudaFree(d_next);
+        cudaFree(state_block);
+        cudaFree(d_ranges);
+        if (l2_window) l2_keep_release(device);
+    }
 };
 
 extern "C" const char* mate_b200_last_error(void) { return g_error.c_str(); }
 extern "C" int mate_b200_abi_version(void) { return MATE_B200_ABI_VERSION; }
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// The per-environment struct-of-arrays members of a state block, in carve order, each with its rows per environment
+// (a row is bpad elements, indexed [row * bpad + env]).  `stats` is not per environment; masks, vals and ready exist
+// in the second block only.
+template <typename F>
+static void for_each_state_array(Params& p, int nc, int nt, int no, F&& f) {
+    f(p.cam_x, nc); f(p.cam_y, nc); f(p.cam_phi, nc); f(p.cam_theta, nc);
+    f(p.tgt_x, nt); f(p.tgt_y, nt);
+    f(p.obs_x, no); f(p.obs_y, no); f(p.obs_r, no);
+    f(p.obs_f4, no);
+    f(p.tgt_pack, nt);
+    f(p.cargo, 2); f(p.env_a, 1); f(p.env_b, 1);
+    f(p.cc_clear, 1);
+}
+
+// Points the state arrays of `p` into `block`, each 256-byte aligned: the per-environment arrays, then `stats`, then
+// (`prepared`: the second block of prepared resets) the first-view masks, the entity values and the ready tags.
+// Returns the bytes of the block; with block == nullptr the pointers are left alone and only the size is computed.
+static size_t carve_state(Params& p, char* block, int nc, int nt, int no, size_t bpad, bool prepared) {
+    size_t off = 0;
+    auto carve = [&](auto*& ptr, size_t count) {
+        if (block) ptr = reinterpret_cast<std::remove_reference_t<decltype(ptr)>>(block + off);
+        off = align_up(off + sizeof(*ptr) * count, 256);
+    };
+    for_each_state_array(p, nc, nt, no, [&](auto*& ptr, int rows) { carve(ptr, (size_t)rows * bpad); });
+    carve(p.stats, 16);
+    if (prepared) {
+        carve(p.masks, (size_t)(nc + nt) * (no <= 16 ? 1 : 2) * bpad);
+        carve(p.vals, (size_t)(3 * nt + 5 * nc) * bpad);
+        carve(p.ready, bpad);
+    }
+    return off;
+}
 
 extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t device,
                                 int64_t env_index_base, MateSim** out) {
@@ -264,7 +322,7 @@ extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t
     CUDA_TRY(cudaSetDevice(device));
     CUDA_TRY(kernel.prepare());
     CUDA_TRY(kernel.prepare_wrappers());
-    MateSim* sim = new MateSim();
+    std::unique_ptr<MateSim> sim(new MateSim());   // frees what is made so far on every early return
     sim->cfg = *cfg;
     sim->cfg.camera_location_ranges = sim->cfg.target_location_ranges = sim->cfg.obstacle_location_ranges = nullptr;
     sim->num_envs = num_envs;
@@ -274,31 +332,12 @@ extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t
     const int bpad = (int)align_up((size_t)num_envs, 256);
     sim->bpad = bpad;
 
-    // one allocation, carved into the SoA arrays (each 256-byte aligned)
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-    const size_t o_cam_x = carve(sizeof(double) * nc * bpad), o_cam_y = carve(sizeof(double) * nc * bpad);
-    const size_t o_cam_phi = carve(sizeof(double) * nc * bpad), o_cam_theta = carve(sizeof(double) * nc * bpad);
-    const size_t o_tgt_x = carve(sizeof(double) * nt * bpad), o_tgt_y = carve(sizeof(double) * nt * bpad);
-    const size_t o_obs_x = carve(sizeof(double) * no * bpad), o_obs_y = carve(sizeof(double) * no * bpad), o_obs_r = carve(sizeof(double) * no * bpad);
-    const size_t o_obs_f4 = carve(sizeof(float4) * no * bpad);
-    const size_t o_pack = carve(sizeof(uint32_t) * nt * bpad);
-    const size_t o_cargo = carve(sizeof(uint4) * 2 * bpad), o_env_a = carve(sizeof(uint4) * bpad), o_env_b = carve(sizeof(int4) * bpad);
-    const size_t o_cc = carve(sizeof(unsigned long long) * bpad);
-    const size_t o_stats = carve(sizeof(float) * 16);
-    sim->state_bytes = off;
-    if (cudaMalloc(&sim->state_block, off) != cudaSuccess) { delete sim; return fail(MATE_ENOMEM, "cudaMalloc(state) failed"); }
-    CUDA_TRY(cudaMemset(sim->state_block, 0, off));
-    char* b = (char*)sim->state_block;
+    // one allocation, carved into the SoA arrays
     Params& p = sim->base;
-    p.cam_x = (double*)(b + o_cam_x); p.cam_y = (double*)(b + o_cam_y); p.cam_phi = (double*)(b + o_cam_phi); p.cam_theta = (double*)(b + o_cam_theta);
-    p.tgt_x = (double*)(b + o_tgt_x); p.tgt_y = (double*)(b + o_tgt_y);
-    p.obs_x = (double*)(b + o_obs_x); p.obs_y = (double*)(b + o_obs_y); p.obs_r = (double*)(b + o_obs_r);
-    p.obs_f4 = (float4*)(b + o_obs_f4);
-    p.tgt_pack = (uint32_t*)(b + o_pack);
-    p.cargo = (uint4*)(b + o_cargo); p.env_a = (uint4*)(b + o_env_a); p.env_b = (int4*)(b + o_env_b);
-    p.cc_clear = (unsigned long long*)(b + o_cc);
-    p.stats = (float*)(b + o_stats);
+    sim->state_bytes = carve_state(p, nullptr, nc, nt, no, bpad, false);
+    if (cudaMalloc(&sim->state_block, sim->state_bytes) != cudaSuccess) return fail(MATE_ENOMEM, "cudaMalloc(state) failed");
+    CUDA_TRY(cudaMemset(sim->state_block, 0, sim->state_bytes));
+    carve_state(p, (char*)sim->state_block, nc, nt, no, bpad, false);
 
     // Warp tiles: 32 environments per warp for the batches that give every SM several of those; smaller batches are cut
     // into tiles of 16 or 8 so that the latency-bound launch still has warps to overlap (measured, MATE-4v8-9: 16 384
@@ -307,41 +346,6 @@ extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t
     sim->tile_envs = num_envs >= 24576 ? 32 : (num_envs >= 8192 ? 16 : 8);
     if (const char* v = getenv("MATE_B200_TILE")) { const int t = atoi(v); if (t == 8 || t == 16 || t == 32) sim->tile_envs = t; }
     p.tile_envs = sim->tile_envs;
-
-    // prepared resets: a second state block of the same layout + first-view masks + the ready tags
-    sim->refill_mode = 1;
-    if (const char* v = getenv("MATE_B200_REFILL")) {
-        if (!strcmp(v, "0") || !strcmp(v, "off")) sim->refill_mode = 0;
-        else if (!strcmp(v, "sync")) sim->refill_mode = sim->refill_mode ? 2 : 0;
-        else if (atoi(v) > 0) sim->refill_period = atoi(v);
-    }
-    if (sim->refill_mode) {
-        const int mask_words = (nc + nt) * (no <= 16 ? 1 : 2);
-        const size_t o_masks = carve(sizeof(uint32_t) * mask_words * bpad);
-        const size_t o_vals = carve(sizeof(float) * (3 * nt + 5 * nc) * bpad);
-        const size_t o_ready = carve(sizeof(uint32_t) * bpad);
-        const size_t block2 = off;
-        if (cudaMalloc(&sim->next_block, block2) != cudaSuccess) { cudaFree(sim->state_block); delete sim; return fail(MATE_ENOMEM, "cudaMalloc(prepared state) failed"); }
-        CUDA_TRY(cudaMemset(sim->next_block, 0, block2));
-        char* b2 = (char*)sim->next_block;
-        Params& n = sim->next_base;
-        n = p;   // scalars are copied again below, once they are set
-        n.cam_x = (double*)(b2 + o_cam_x); n.cam_y = (double*)(b2 + o_cam_y); n.cam_phi = (double*)(b2 + o_cam_phi); n.cam_theta = (double*)(b2 + o_cam_theta);
-        n.tgt_x = (double*)(b2 + o_tgt_x); n.tgt_y = (double*)(b2 + o_tgt_y);
-        n.obs_x = (double*)(b2 + o_obs_x); n.obs_y = (double*)(b2 + o_obs_y); n.obs_r = (double*)(b2 + o_obs_r);
-        n.obs_f4 = (float4*)(b2 + o_obs_f4);
-        n.tgt_pack = (uint32_t*)(b2 + o_pack);
-        n.cargo = (uint4*)(b2 + o_cargo); n.env_a = (uint4*)(b2 + o_env_a); n.env_b = (int4*)(b2 + o_env_b);
-        n.cc_clear = (unsigned long long*)(b2 + o_cc);
-        n.stats = (float*)(b2 + o_stats);
-        n.masks = (uint32_t*)(b2 + o_masks);
-        n.vals = (float*)(b2 + o_vals);
-        n.ready = (uint32_t*)(b2 + o_ready);
-        p.ready = n.ready;
-        CUDA_TRY(cudaMalloc(&sim->d_next, sizeof(Params)));
-        CUDA_TRY(cudaStreamCreateWithFlags(&sim->side, cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&sim->side_event, cudaEventDisableTiming));
-    }
 
     // location ranges on device (reset)
     std::vector<double> ranges((size_t)4 * (nc + nt + no) + 4, 0.0);
@@ -368,14 +372,26 @@ extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t
     p.tgt_step_size = cfg->target_step_size; p.tgt_sight_range = cfg->target_sight_range;
     p.obs_r_low = cfg->obstacle_radius_low; p.obs_r_high = cfg->obstacle_radius_high;
 
+    // prepared resets: a second state block of the same layout + first-view masks + the ready tags, addressed by
+    // next_base: the scalars and range pointers of the live block with the state pointers of the second block
+    sim->refill_mode = 1;
+    if (const char* v = getenv("MATE_B200_REFILL")) {
+        if (!strcmp(v, "0") || !strcmp(v, "off")) sim->refill_mode = 0;
+        else if (!strcmp(v, "sync")) sim->refill_mode = sim->refill_mode ? 2 : 0;
+        else if (atoi(v) > 0) sim->refill_period = atoi(v);
+    }
     if (sim->refill_mode) {
-        Params n = p;   // all scalars / range pointers of the live block ...
-        const Params& o = sim->next_base;   // ... with the state pointers of the second block
-        n.cam_x = o.cam_x; n.cam_y = o.cam_y; n.cam_phi = o.cam_phi; n.cam_theta = o.cam_theta; n.tgt_x = o.tgt_x; n.tgt_y = o.tgt_y;
-        n.obs_x = o.obs_x; n.obs_y = o.obs_y; n.obs_r = o.obs_r; n.obs_f4 = o.obs_f4; n.tgt_pack = o.tgt_pack;
-        n.cargo = o.cargo; n.env_a = o.env_a; n.env_b = o.env_b; n.cc_clear = o.cc_clear; n.stats = o.stats;
-        n.masks = o.masks; n.vals = o.vals; n.ready = o.ready; n.live_env_b = p.env_b; n.next = nullptr;
-        sim->next_base = n;
+        Params& n = sim->next_base;
+        n = p;
+        const size_t block2 = carve_state(n, nullptr, nc, nt, no, bpad, true);
+        if (cudaMalloc(&sim->next_block, block2) != cudaSuccess) return fail(MATE_ENOMEM, "cudaMalloc(prepared state) failed");
+        CUDA_TRY(cudaMemset(sim->next_block, 0, block2));
+        carve_state(n, (char*)sim->next_block, nc, nt, no, bpad, true);
+        n.live_env_b = p.env_b;
+        p.ready = n.ready;   // the live tags are the second block's
+        CUDA_TRY(cudaMalloc(&sim->d_next, sizeof(Params)));
+        CUDA_TRY(cudaStreamCreateWithFlags(&sim->side, cudaStreamNonBlocking));
+        CUDA_TRY(cudaEventCreateWithFlags(&sim->side_event, cudaEventDisableTiming));
         CUDA_TRY(cudaMemcpy(sim->d_next, &sim->next_base, sizeof(Params), cudaMemcpyHostToDevice));
         p.next = sim->d_next;
     }
@@ -387,33 +403,13 @@ extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t
         std::vector<uint32_t> pack((size_t)nt * bpad, pack_target(0, -1, 0, 1, 0, 0));
         CUDA_TRY(cudaMemcpy(p.tgt_pack, pack.data(), pack.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
     }
-    *out = sim;
+    *out = sim.release();
     return MATE_OK;
 }
 
 extern "C" int mate_b200_destroy(MateSim* sim) {
     if (!sim) return MATE_OK;
     cudaSetDevice(sim->device);
-    if (sim->host_ready) {
-        for (int i = 0; i < MateSim::kHostStreams; ++i) { cudaStreamDestroy(sim->hstreams[i]); cudaEventDestroy(sim->hevents[i]); }
-        cudaFree(sim->h_cam_act); cudaFree(sim->h_tgt_act); cudaFree(sim->h_cam_obs); cudaFree(sim->h_tgt_obs);
-        cudaFree(sim->h_rewards); cudaFree(sim->h_done);
-        sim->pool.reset();
-        for (int r = 0; r < 2; ++r) { cudaFree(sim->d_compact[r]); cudaFree(sim->d_table[r]); cudaFreeHost(sim->p_compact[r]); cudaFreeHost(sim->p_table[r]); cudaFree(sim->h_rows2[r]); }
-        cudaFree(sim->d_count); cudaFreeHost(sim->p_count);
-        if (sim->copy_stream) {
-            cudaStreamDestroy(sim->copy_stream);
-            for (int i = 0; i < MateSim::kMaxHostChunks; ++i) { cudaEventDestroy(sim->e_counts[i]); cudaEventDestroy(sim->e_stream[i]); cudaEventDestroy(sim->e_tables[i]); }
-        }
-    }
-    if (sim->side) { cudaStreamSynchronize(sim->side); cudaStreamDestroy(sim->side); }
-    if (sim->side_event) cudaEventDestroy(sim->side_event);
-    cudaFree(sim->soft_edges);
-    cudaFree(sim->next_block);
-    cudaFree(sim->d_next);
-    cudaFree(sim->state_block);
-    cudaFree(sim->d_ranges);
-    if (sim->l2_window) l2_keep_release(sim->device);
     delete sim;
     return MATE_OK;
 }
@@ -425,11 +421,35 @@ extern "C" int mate_b200_obs_dims(const MateSim* sim, int32_t* cam_dim, int32_t*
     return MATE_OK;
 }
 
-// bytes of one value of the observation rows in the handle's format
-static size_t obs_elem_bytes(const MateSim* sim) { return sim->obs_format == MATE_OBS_FORMAT_F16 ? 2 : 4; }
-// `base` advanced by `values` values of the observation rows (the row pointers are typed float* in the ABI)
-static float* obs_advance(const MateSim* sim, float* base, size_t values) {
-    return reinterpret_cast<float*>(reinterpret_cast<char*>(base) + values * obs_elem_bytes(sim));
+// bytes of observation rows per environment in the handle's format: region 0 = camera rows, 1 = target rows
+static size_t env_row_bytes(const MateSim* sim, int region) {
+    const size_t elem = sim->obs_format == MATE_OBS_FORMAT_F16 ? 2 : 4;
+    return region == 0 ? elem * sim->cfg.num_cameras * sim->kernel.dc : elem * sim->cfg.num_targets * sim->kernel.dt;
+}
+// the rows of environment `env` in a buffer of one region's rows (the row pointers are typed float* in the ABI)
+static float* env_rows(const MateSim* sim, float* rows, int region, size_t env) {
+    return reinterpret_cast<float*>(reinterpret_cast<char*>(rows) + env * env_row_bytes(sim, region));
+}
+
+// the kernel launch just enqueued was accepted
+static int check_launch(const char* what) {
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string(what) + " launch: " + cudaGetErrorString(err));
+    return MATE_OK;
+}
+
+// the observation wrapper codes as an ObsOps (the count has been checked)
+static int parse_obs_ops(const MateSim* sim, const int32_t* ops, int32_t num_ops, const float* cam_affine, const float* tgt_affine,
+                         ObsOps* o) {
+    *o = ObsOps{};
+    o->n = num_ops;
+    for (int i = 0; i < num_ops; ++i) {
+        if (ops[i] < MATE_OBS_ENHANCED_CAMERA || ops[i] > MATE_OBS_RESCALED) return fail(MATE_EINVAL, "unknown observation wrapper code");
+        if (ops[i] == MATE_OBS_RESCALED && (!tgt_affine || (sim->cfg.num_cameras > 0 && !cam_affine)))
+            return fail(MATE_EINVAL, "MATE_OBS_RESCALED needs the affine tables");
+        o->op[i] = ops[i];
+    }
+    return MATE_OK;
 }
 
 extern "C" int mate_b200_set_observation_format(MateSim* sim, int32_t format) {
@@ -450,9 +470,7 @@ extern "C" int mate_b200_fov_range(MateSim* sim, const int32_t* env, const int32
     CUDA_TRY(cudaSetDevice(sim->device));
     sim->kernel.launch_fov(sim->base, env, camera, angle_deg, out, n, (cudaStream_t)stream);
     sim->launches += 1;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("fov_range launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("fov_range");
 }
 
 extern "C" int64_t mate_b200_launch_count(const MateSim* sim) { return sim ? sim->launches : 0; }
@@ -472,36 +490,22 @@ extern "C" int mate_b200_transform_observations(MateSim* sim, float* cam_obs, fl
         return fail(MATE_EINVAL, "transform_observations works on float32 rows; register the wrappers (set_observation_ops) on a float16 handle");
     if (num_ops == 0) return MATE_OK;
     if (((uintptr_t)cam_obs & 15) || ((uintptr_t)tgt_obs & 15)) return fail(MATE_EINVAL, "observation buffers must be 16-byte aligned");
-    ObsOps o{};
-    o.n = num_ops;
-    for (int i = 0; i < num_ops; ++i) {
-        if (ops[i] < MATE_OBS_ENHANCED_CAMERA || ops[i] > MATE_OBS_RESCALED) return fail(MATE_EINVAL, "unknown observation wrapper code");
-        if (ops[i] == MATE_OBS_RESCALED && (!tgt_affine || (sim->cfg.num_cameras > 0 && !cam_affine)))
-            return fail(MATE_EINVAL, "MATE_OBS_RESCALED needs the affine tables");
-        o.op[i] = ops[i];
-    }
+    ObsOps o;
+    if (int rc = parse_obs_ops(sim, ops, num_ops, cam_affine, tgt_affine, &o)) return rc;
     CUDA_TRY(cudaSetDevice(sim->device));
     Params p = sim->base;
     p.cam_obs = cam_obs; p.tgt_obs = tgt_obs;
     sim->kernel.launch_wrappers(p, o, cam_affine, tgt_affine, sim->num_envs, (cudaStream_t)stream);
     sim->launches += 1;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("wrapper kernel launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("wrapper kernel");
 }
 
 extern "C" int mate_b200_set_observation_ops(MateSim* sim, const int32_t* ops, int32_t num_ops, const float* cam_affine,
                                              const float* tgt_affine) {
     if (!sim || (num_ops > 0 && !ops)) return fail(MATE_EINVAL, "null argument");
     if (num_ops < 0 || num_ops > MATE_MAX_OBS_OPS) return fail(MATE_EINVAL, "too many observation wrappers (MATE_MAX_OBS_OPS)");
-    ObsOps o{};
-    o.n = num_ops;
-    for (int i = 0; i < num_ops; ++i) {
-        if (ops[i] < MATE_OBS_ENHANCED_CAMERA || ops[i] > MATE_OBS_RESCALED) return fail(MATE_EINVAL, "unknown observation wrapper code");
-        if (ops[i] == MATE_OBS_RESCALED && (!tgt_affine || (sim->cfg.num_cameras > 0 && !cam_affine)))
-            return fail(MATE_EINVAL, "MATE_OBS_RESCALED needs the affine tables");
-        o.op[i] = ops[i];
-    }
+    ObsOps o;
+    if (int rc = parse_obs_ops(sim, ops, num_ops, cam_affine, tgt_affine, &o)) return rc;
     // canonical stacks -- (Enhanced | Shared)* Relative? Rescaled? -- are applied while the rows are composed (FoldOps)
     FoldOps f{};
     int k = 0;
@@ -555,9 +559,7 @@ extern "C" int mate_b200_soft_coverage(MateSim* sim, const uint8_t* mask_ct, con
         CUDA_TRY(cudaMalloc(&sim->soft_edges, sizeof(double) * 2 * (size_t)sim->num_envs * sim->cfg.num_cameras));
     sim->kernel.launch_soft(sim->base, mask_ct, done, sim->soft_edges, soft_matrix, (cudaStream_t)stream);
     sim->launches += 2;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("soft coverage launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("soft coverage");
 }
 
 extern "C" int mate_b200_auxiliary_terms(MateSim* sim, const MateStepAux* aux, const float* rewards, const float* soft_matrix,
@@ -574,9 +576,7 @@ extern "C" int mate_b200_auxiliary_terms(MateSim* sim, const MateStepAux* aux, c
     aux_terms_kernel<<<(unsigned)((agents + threads - 1) / threads), threads, 0, (cudaStream_t)stream>>>(
         *aux, rewards, soft_matrix, cam_terms, tgt_terms, sim->num_envs, sim->cfg.num_cameras, sim->cfg.num_targets);
     sim->launches += 1;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("auxiliary terms launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("auxiliary terms");
 }
 
 extern "C" int mate_b200_greedy_target_actions(MateSim* sim, double* memory, const uint8_t* reset_mask, double noise_scale,
@@ -591,9 +591,7 @@ extern "C" int mate_b200_greedy_target_actions(MateSim* sim, double* memory, con
     greedy_target_kernel<<<(sim->num_envs + threads - 1) / threads, threads, 0, (cudaStream_t)stream>>>(
         sim->base, sim->cfg.num_targets, memory, reset_mask, noise_scale, seed, serial, r, tgt_act);
     sim->launches += 1;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("greedy target launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("greedy target");
 }
 
 extern "C" int mate_b200_greedy_camera_actions(MateSim* sim, double* memory, const uint8_t* tracked, const uint8_t* reset_mask,
@@ -612,9 +610,7 @@ extern "C" int mate_b200_greedy_camera_actions(MateSim* sim, double* memory, con
     greedy_camera_kernel<<<(unsigned)((agents + kCameraAgentThreads - 1) / kCameraAgentThreads), kCameraAgentThreads, 0, (cudaStream_t)stream>>>(
         sim->base, nc, nt, memory, tracked, reset_mask, seed, serial, r, cam_act);
     sim->launches += 1;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("greedy camera launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("greedy camera");
 }
 
 extern "C" int mate_b200_decode_actions(const int64_t* index, const float* table, int32_t table_size, float* out,
@@ -623,39 +619,36 @@ extern "C" int mate_b200_decode_actions(const int64_t* index, const float* table
     if (count == 0) return MATE_OK;
     if (((uintptr_t)out & 7) || ((uintptr_t)table & 7)) return fail(MATE_EINVAL, "action buffers must be 8-byte aligned");
     decode_actions_kernel<<<(unsigned)((count + 255) / 256), 256, 0, (cudaStream_t)stream>>>(index, table, table_size, out, count);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("decode launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("decode");
+}
+
+// CTAs of a step-kernel launch over `count` environments
+static int step_grid(const MateSim* sim, int count) {
+    const int per_cta = sim->kernel.envs_per_cta / 32 * sim->tile_envs;
+    return (count + per_cta - 1) / per_cta;
 }
 
 // Launch the fused kernel over envs [begin, begin + count); I/O pointers are for env 0.
 static int launch_range(MateSim* sim, Params p, int begin, int count, cudaStream_t stream) {
     const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets;
-    const int dc = sim->kernel.dc, dt = sim->kernel.dt;
     // SoA rows are indexed [row * bpad + env]: shifting the base pointers selects the sub-range
-    p.cam_x += begin; p.cam_y += begin; p.cam_phi += begin; p.cam_theta += begin;
-    p.tgt_x += begin; p.tgt_y += begin; p.obs_x += begin; p.obs_y += begin; p.obs_r += begin; p.obs_f4 += begin;
-    p.tgt_pack += begin; p.cargo += begin; p.env_a += begin; p.env_b += begin; p.cc_clear += begin;
+    for_each_state_array(p, nc, nt, sim->cfg.num_obstacles, [&](auto*& ptr, int) { ptr += begin; });
     if (p.cam_act) p.cam_act += (size_t)begin * nc * 2;
     if (p.tgt_act) p.tgt_act += (size_t)begin * nt * 2;
-    if (p.cam_obs) p.cam_obs = obs_advance(sim, p.cam_obs, (size_t)begin * nc * dc);
-    if (p.tgt_obs) p.tgt_obs = obs_advance(sim, p.tgt_obs, (size_t)begin * nt * dt);
+    if (p.cam_obs) p.cam_obs = env_rows(sim, p.cam_obs, 0, begin);
+    if (p.tgt_obs) p.tgt_obs = env_rows(sim, p.tgt_obs, 1, begin);
     if (p.rewards) p.rewards += (size_t)begin * 2;
     if (p.done) p.done += begin;
     if (p.env_mask) p.env_mask += begin;
     if (p.replay_transmit) p.replay_transmit += (size_t)begin * nc * nt;
     if (p.replay_choice) p.replay_choice += (size_t)begin * nt;
-    if (p.ready) p.ready += begin;
+    if (p.ready) p.ready += begin;   // the live tags, an array of the second block
     p.next_offset = begin;   // `next` addresses whole-batch arrays
     p.env_index_base += begin;
     p.num_envs = count;
-    const int per_cta = sim->kernel.envs_per_cta / 32 * sim->tile_envs;
-    const int grid = (count + per_cta - 1) / per_cta;
-    sim->kernel.launch(p, grid, stream);
+    sim->kernel.launch(p, step_grid(sim, count), stream);
     sim->launches += 1;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("kernel launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("kernel");
 }
 
 static int check_obs_alignment(const void* cam_obs, const void* tgt_obs) {
@@ -700,13 +693,17 @@ static int launch_prepare(MateSim* sim, cudaStream_t stream) {
     n.mode = MODE_PREPARE; n.flags = 0; n.seed = sim->seed; n.l2_window_bytes = 0;
     n.cam_act = n.tgt_act = nullptr; n.cam_obs = n.tgt_obs = n.rewards = nullptr; n.done = nullptr; n.env_mask = nullptr;
     fill_aux(n, nullptr, nullptr);
-    const int per_cta = sim->kernel.envs_per_cta / 32 * sim->tile_envs;
-    const int grid = (sim->num_envs + per_cta - 1) / per_cta;
-    sim->kernel.launch(n, grid, target);
+    sim->kernel.launch(n, step_grid(sim, sim->num_envs), target);
     sim->launches += 1;
     sim->steps_since_refill = 0;
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("prepare launch: ") + cudaGetErrorString(err));
+    return check_launch("prepare");
+}
+
+// after a step with auto-resets: refill the prepared episodes every refill_period steps (refill_mode 2: every step)
+static int refill_after_step(MateSim* sim, uint32_t flags, cudaStream_t stream) {
+    if ((flags & MATE_STEP_AUTO_RESET) && sim->refill_mode &&
+        (sim->refill_mode == 2 || ++sim->steps_since_refill >= sim->refill_period))
+        return launch_prepare(sim, stream);
     return MATE_OK;
 }
 
@@ -729,9 +726,7 @@ extern "C" int mate_b200_seed(MateSim* sim, const uint8_t* env_mask, uint64_t se
     sim->seed = seed;
     if (int rc = invalidate_prepared(sim, (cudaStream_t)stream)) return rc;
     rewind_episode_kernel<<<(sim->num_envs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(sim->base.env_b, env_mask, sim->num_envs);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(MATE_ECUDA, std::string("seed launch: ") + cudaGetErrorString(err));
-    return MATE_OK;
+    return check_launch("seed");
 }
 
 extern "C" int mate_b200_reset(MateSim* sim, const uint8_t* env_mask, uint64_t seed, float* cam_obs,
@@ -765,10 +760,7 @@ extern "C" int mate_b200_step(MateSim* sim, const float* cam_act, const float* t
     p.cam_act = cam_act; p.tgt_act = tgt_act; p.cam_obs = cam_obs; p.tgt_obs = tgt_obs; p.rewards = rewards; p.done = done;
     fill_aux(p, aux, replay);
     if (int rc = launch_range(sim, p, 0, sim->num_envs, (cudaStream_t)stream)) return rc;
-    if ((flags & MATE_STEP_AUTO_RESET) && sim->refill_mode &&
-        (sim->refill_mode == 2 || ++sim->steps_since_refill >= sim->refill_period))
-        return launch_prepare(sim, (cudaStream_t)stream);
-    return MATE_OK;
+    return refill_after_step(sim, flags, (cudaStream_t)stream);
 }
 
 extern "C" int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs, const MateStepAux* aux,
@@ -786,20 +778,21 @@ extern "C" int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs, c
 }
 
 // ---- host-buffer path: chunked H2D -> kernel -> D2H over a few streams ------------------------
+// Makes only what is still missing, so that a call after a failed one does not make anything twice.
 static int ensure_host_path(MateSim* sim) {
     if (sim->host_ready) return MATE_OK;
     const size_t B = sim->num_envs;
     const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets;
     for (int i = 0; i < MateSim::kHostStreams; ++i) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&sim->hstreams[i], cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&sim->hevents[i], cudaEventDisableTiming));
+        if (!sim->hstreams[i]) CUDA_TRY(cudaStreamCreateWithFlags(&sim->hstreams[i], cudaStreamNonBlocking));
+        if (!sim->hevents[i]) CUDA_TRY(cudaEventCreateWithFlags(&sim->hevents[i], cudaEventDisableTiming));
     }
-    CUDA_TRY(cudaMalloc(&sim->h_cam_act, sizeof(float) * (B * nc * 2 + 4)));
-    CUDA_TRY(cudaMalloc(&sim->h_tgt_act, sizeof(float) * B * nt * 2));
-    CUDA_TRY(cudaMalloc(&sim->h_cam_obs, sizeof(float) * (B * nc * sim->kernel.dc + 4)));
-    CUDA_TRY(cudaMalloc(&sim->h_tgt_obs, sizeof(float) * B * nt * sim->kernel.dt));
-    CUDA_TRY(cudaMalloc(&sim->h_rewards, sizeof(float) * B * 2));
-    CUDA_TRY(cudaMalloc(&sim->h_done, B));
+    if (!sim->h_cam_act) CUDA_TRY(cudaMalloc(&sim->h_cam_act, sizeof(float) * (B * nc * 2 + 4)));
+    if (!sim->h_tgt_act) CUDA_TRY(cudaMalloc(&sim->h_tgt_act, sizeof(float) * B * nt * 2));
+    if (!sim->h_cam_obs) CUDA_TRY(cudaMalloc(&sim->h_cam_obs, sizeof(float) * (B * nc * sim->kernel.dc + 4)));
+    if (!sim->h_tgt_obs) CUDA_TRY(cudaMalloc(&sim->h_tgt_obs, sizeof(float) * B * nt * sim->kernel.dt));
+    if (!sim->h_rewards) CUDA_TRY(cudaMalloc(&sim->h_rewards, sizeof(float) * B * 2));
+    if (!sim->h_done) CUDA_TRY(cudaMalloc(&sim->h_done, B));
     // Compacted device -> host leg (mate_hostpath.cuh): what bounds it is the number of host threads that rebuild the dense
     // rows (measured with 15: 9.3 - 9.6e6 env-steps/s against 8.6 - 8.7e6 for the dense copy, with 10: 8.3e6, with 6: 6.4e6,
     // profiles/r2v_hostpath.md), so it is used when this process has at least 14 of them to itself -- all host threads the
@@ -821,10 +814,9 @@ static int ensure_host_path(MateSim* sim) {
     // copy densely
     sim->compact_mode = threads >= 14 ? 1 : ((threads >= 5 || (threads >= 3 && sharers >= 4)) ? 2 : 0);
     if (const char* v = getenv("MATE_B200_HOST_COMPACT")) sim->compact_mode = v[0] == '1' ? 1 : (v[0] == '2' ? 2 : 0);
-    const size_t esz = obs_elem_bytes(sim);
-    if ((esz * nc * sim->kernel.dc) % 16 || (esz * nt * sim->kernel.dt) % 16) sim->compact_mode = 0;
+    if (env_row_bytes(sim, 0) % 16 || env_row_bytes(sim, 1) % 16) sim->compact_mode = 0;
     if (sim->compact_mode) {
-        const size_t region_bytes[2] = {esz * B * nc * sim->kernel.dc, esz * B * nt * sim->kernel.dt};
+        const size_t region_bytes[2] = {B * env_row_bytes(sim, 0), B * env_row_bytes(sim, 1)};
         bool ok = true;
         for (int r = 0; r < 2 && ok; ++r) {
             if (region_bytes[r] == 0) continue;
@@ -852,15 +844,145 @@ static int ensure_host_path(MateSim* sim) {
     return MATE_OK;
 }
 
+// one launch chunk of a step_host call, enqueued on `s`: its actions to the device, then the step over its environments
+static int step_chunk(MateSim* sim, const Params& p, const float* cam_act, const float* tgt_act, int begin, int count, cudaStream_t s) {
+    const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets;
+    if (nc) CUDA_TRY(cudaMemcpyAsync(sim->h_cam_act + (size_t)begin * nc * 2, cam_act + (size_t)begin * nc * 2, sizeof(float) * count * nc * 2, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(sim->h_tgt_act + (size_t)begin * nt * 2, tgt_act + (size_t)begin * nt * 2, sizeof(float) * count * nt * 2, cudaMemcpyHostToDevice, s));
+    return launch_range(sim, p, begin, count, s);
+}
+
+// the rewards and done flags of a launch chunk to the caller's buffers, enqueued on `s`
+static int copy_rewards_done(MateSim* sim, float* rewards, uint8_t* done, int begin, int count, cudaStream_t s) {
+    CUDA_TRY(cudaMemcpyAsync(rewards + (size_t)begin * 2, sim->h_rewards + (size_t)begin * 2, sizeof(float) * count * 2, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(done + begin, sim->h_done + begin, count, cudaMemcpyDeviceToHost, s));
+    return MATE_OK;
+}
+
+// ---- dense device -> host leg: every chunk's rows are copied as they are
+static int dense_leg(MateSim* sim, const Params& p, int chunk, const float* cam_act, const float* tgt_act, float* cam_obs,
+                     float* tgt_obs, float* rewards, uint8_t* done) {
+    const int B = sim->num_envs;
+    int k = 0;
+    for (int begin = 0; begin < B; begin += chunk, ++k) {
+        const int count = std::min(chunk, B - begin);
+        cudaStream_t s = sim->hstreams[k % MateSim::kHostStreams];
+        if (int rc = step_chunk(sim, p, cam_act, tgt_act, begin, count, s)) return rc;
+        if (sim->cfg.num_cameras) CUDA_TRY(cudaMemcpyAsync(env_rows(sim, cam_obs, 0, begin), env_rows(sim, p.cam_obs, 0, begin), count * env_row_bytes(sim, 0), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaMemcpyAsync(env_rows(sim, tgt_obs, 1, begin), env_rows(sim, p.tgt_obs, 1, begin), count * env_row_bytes(sim, 1), cudaMemcpyDeviceToHost, s));
+        if (int rc = copy_rewards_done(sim, rewards, done, begin, count, s)) return rc;
+    }
+    for (int i = 0; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamSynchronize(sim->hstreams[i]));
+    sim->last_leg = 0; sim->last_link_bytes = (unsigned long long)B * (env_row_bytes(sim, 0) + env_row_bytes(sim, 1));
+    return MATE_OK;
+}
+
+// ---- compacted device -> host leg (mate_hostpath.cuh): every launch chunk's rows are compacted on the device, the
+//      compact streams cross the link one after the other, host threads expand them into the caller's buffers
+//      (`delta`: the changes against `rows_before` are patched into the rows the caller's buffers still hold)
+static int compact_leg(MateSim* sim, const Params& p, int chunk, bool delta, const float* const rows_before[2],
+                       const float* cam_act, const float* tgt_act, float* cam_obs, float* tgt_obs, float* rewards, uint8_t* done) {
+    static const bool trace = getenv("MATE_B200_HOST_TRACE") != nullptr;
+    const auto t_start = std::chrono::steady_clock::now();
+    auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count(); };
+    double t_enq = 0, t_counts = 0, t_last_stream = 0;
+    const int B = sim->num_envs;
+    const int num_chunks = (B + chunk - 1) / chunk;
+    const size_t per_env[2] = {env_row_bytes(sim, 0), env_row_bytes(sim, 1)};
+    float* const host_rows[2] = {cam_obs, tgt_obs};
+    const float* const dev_rows[2] = {p.cam_obs, p.tgt_obs};
+    std::vector<long long> table_base(2 * (num_chunks + 1), 0);
+    CUDA_TRY(cudaMemsetAsync(sim->d_count, 0, sizeof(unsigned int) * MateSim::kMaxHostChunks * 2, sim->hstreams[0]));
+    CUDA_TRY(cudaEventRecord(sim->hevents[1], sim->hstreams[0]));
+    for (int i = 1; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamWaitEvent(sim->hstreams[i], sim->hevents[1], 0));
+    int kc = 0;
+    for (int begin = 0; begin < B; begin += chunk, ++kc) {
+        const int count = std::min(chunk, B - begin);
+        cudaStream_t s = sim->hstreams[kc % MateSim::kHostStreams];
+        if (int rc = step_chunk(sim, p, cam_act, tgt_act, begin, count, s)) return rc;
+        for (int r = 0; r < 2; ++r) {
+            table_base[2 * (kc + 1) + r] = table_base[2 * kc + r];
+            if (per_env[r] == 0) continue;
+            const size_t first = (size_t)begin * per_env[r] / 16;            // B % 4 == 0 and chunk % 4 == 0: whole chunks
+            const long long nchunks = (long long)((size_t)count * per_env[r] / 16);
+            const long long nblocks = (nchunks + kCompactBlock - 1) / kCompactBlock;
+            CompactEntry* table = sim->d_table[r] + table_base[2 * kc + r];
+            table_base[2 * (kc + 1) + r] += nblocks;
+            if (delta) compact_changes_kernel<<<1184, 128, 0, s>>>(reinterpret_cast<const uint4*>(dev_rows[r]) + first, reinterpret_cast<const uint4*>(rows_before[r]) + first,
+                                                                   nchunks, sim->d_compact[r] + first, table, sim->d_count + 2 * kc + r);
+            else compact_chunks_kernel<<<1184, 128, 0, s>>>(reinterpret_cast<const uint4*>(dev_rows[r]) + first, nchunks,
+                                                            sim->d_compact[r] + first, table, sim->d_count + 2 * kc + r);
+        }
+        sim->launches += (sim->cfg.num_cameras ? 2 : 1);
+        // The sizes of the chunk's compact streams go to the host by a store into pinned memory, not by a copy: a copy
+        // would queue behind the compact streams of earlier chunks on the copy engine, and the next stream could only be
+        // enqueued after the previous one had crossed the link (a bubble per chunk).
+        publish_counts_kernel<<<1, 32, 0, s>>>(sim->d_count + 2 * kc, sim->p_count_dev + 2 * kc);
+        CUDA_TRY(cudaEventRecord(sim->e_counts[kc], s));
+        for (int r = 0; r < 2; ++r) {
+            const long long nblocks = table_base[2 * (kc + 1) + r] - table_base[2 * kc + r];
+            if (nblocks > 0) CUDA_TRY(cudaMemcpyAsync(sim->p_table[r] + table_base[2 * kc + r], sim->d_table[r] + table_base[2 * kc + r], sizeof(CompactEntry) * nblocks, cudaMemcpyDeviceToHost, s));
+        }
+        if (int rc = copy_rewards_done(sim, rewards, done, begin, count, s)) return rc;
+        CUDA_TRY(cudaEventRecord(sim->e_tables[kc], s));
+    }
+    t_enq = since();
+    // the sizes are known once a chunk's kernels have run: its compact streams go on the copy stream in chunk order
+    const int pieces = std::max(1, sim->pool->size());
+    kc = 0;
+    for (int begin = 0; begin < B; begin += chunk, ++kc) {
+        CUDA_TRY(cudaEventSynchronize(sim->e_counts[kc]));
+        CUDA_TRY(cudaStreamWaitEvent(sim->copy_stream, sim->e_tables[kc], 0));   // a chunk's stream event then covers its tables too
+        for (int r = 0; r < 2; ++r) {
+            if (per_env[r] == 0 || sim->p_count[2 * kc + r] == 0) continue;
+            const size_t first = (size_t)begin * per_env[r] / 16;
+            CUDA_TRY(cudaMemcpyAsync(sim->p_compact[r] + first, sim->d_compact[r] + first, (size_t)sim->p_count[2 * kc + r] * 16,
+                                     cudaMemcpyDeviceToHost, sim->copy_stream));
+        }
+        CUDA_TRY(cudaEventRecord(sim->e_stream[kc], sim->copy_stream));
+        // expansion: the pool's threads wait for the chunk's stream themselves, so the caller's thread goes on to the next sizes
+        const int count = std::min(chunk, B - begin);
+        for (int r = 0; r < 2; ++r) {
+            if (per_env[r] == 0) continue;
+            const size_t first = (size_t)begin * per_env[r] / 16;
+            const long long nchunks = (long long)((size_t)count * per_env[r] / 16);
+            const long long nblocks = (nchunks + kCompactBlock - 1) / kCompactBlock;
+            const long long per_piece = (nblocks + pieces - 1) / pieces;
+            __m128i* dst = reinterpret_cast<__m128i*>(host_rows[r]) + first;
+            const bool aligned = (((uintptr_t)dst) & 15) == 0;
+            for (long long b0 = 0; b0 < nblocks; b0 += per_piece)
+                sim->pool->submit(ExpandPool::Work{sim->p_table[r] + table_base[2 * kc + r], delta, reinterpret_cast<const __m128i*>(sim->p_compact[r] + first),
+                                                   dst, nchunks, b0, std::min(nblocks, b0 + per_piece), aligned, sim->e_stream[kc]});
+        }
+    }
+    t_counts = since();
+    CUDA_TRY(cudaStreamSynchronize(sim->copy_stream));
+    t_last_stream = since();
+    sim->pool->wait();
+    for (int i = 0; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamSynchronize(sim->hstreams[i]));
+    {
+        unsigned long long link = 0;
+        for (int i = 0; i < 2 * num_chunks; ++i) link += (unsigned long long)sim->p_count[i] * 16ull;
+        link += (unsigned long long)(table_base[2 * num_chunks] + table_base[2 * num_chunks + 1]) * sizeof(CompactEntry);
+        sim->last_leg = delta ? 2 : 1; sim->last_link_bytes = link;
+    }
+    if (trace) {
+        unsigned long long kept = 0;
+        for (int i = 0; i < 2 * num_chunks; ++i) kept += sim->p_count[i];
+        fprintf(stderr, "step_host compact: enqueued %.2f ms, sizes known + copies enqueued %.2f, last stream arrived %.2f, expanded %.2f; kept %.1f MB of %.1f MB, %d threads, changes only %d\n",
+                t_enq, t_counts, t_last_stream, since(), kept * 16 / 1e6, (per_env[0] + per_env[1]) * (double)B / 1e6, sim->pool->size(), (int)delta);
+    }
+    return MATE_OK;
+}
+
 extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const float* tgt_act, float* cam_obs,
                                    float* tgt_obs, float* rewards, uint8_t* done, uint32_t flags) {
     if (!sim || !tgt_act || !tgt_obs || !rewards || !done) return fail(MATE_EINVAL, "null argument");
-    const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets;
+    const int nc = sim->cfg.num_cameras;
     if (nc > 0 && (!cam_act || !cam_obs)) return fail(MATE_EINVAL, "null camera buffers");
     CUDA_TRY(cudaSetDevice(sim->device));
     sim->rows_written = true;
     if (int rc = ensure_host_path(sim)) return rc;
-    const int dc = sim->kernel.dc, dt = sim->kernel.dt;
     const int B = sim->num_envs;
     // chunk size: a multiple of the CTA tile, ~16 chunks so copies and kernels overlap
     int chunk = (B + 15) / 16;
@@ -879,8 +1001,6 @@ extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const flo
     // callers that use non-blocking streams of their own synchronise them before this call (include/mate_b200.h)
     CUDA_TRY(cudaEventRecord(sim->hevents[0], nullptr));
     for (int i = 0; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamWaitEvent(sim->hstreams[i], sim->hevents[0], 0));
-    // ---- compacted device -> host leg (mate_hostpath.cuh): every launch chunk's rows are compacted on the device, the
-    //      compact streams cross the link one after the other, host threads expand them into the caller's buffers
     const int num_chunks = (B + chunk - 1) / chunk;
     // MATE_STEP_HOST_ROWS_KEPT: the caller's row buffers still hold the rows of the previous call (same buffers, not
     // modified since) and the device still holds them too: only the 64-byte groups that differ cross the link and are
@@ -889,129 +1009,15 @@ extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const flo
     const bool compact = (sim->compact_mode == 1 || (sim->compact_mode == 2 && delta)) && num_chunks <= MateSim::kMaxHostChunks && B % 4 == 0 &&
                          !((uintptr_t)cam_obs & 3) && !((uintptr_t)tgt_obs & 3);
     sim->kept_valid = false;
-    if (compact) {
-        static const bool trace = getenv("MATE_B200_HOST_TRACE") != nullptr;
-        const auto t_start = std::chrono::steady_clock::now();
-        auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count(); };
-        double t_enq = 0, t_counts = 0, t_last_stream = 0;
-        const size_t per_env[2] = {(size_t)nc * dc * obs_elem_bytes(sim), (size_t)nt * dt * obs_elem_bytes(sim)};   // bytes of rows per environment and region
-        float* const host_rows[2] = {cam_obs, tgt_obs};
-        float* const dev_rows[2] = {rows_now[0], rows_now[1]};
-        std::vector<long long> table_base(2 * (num_chunks + 1), 0);
-        CUDA_TRY(cudaMemsetAsync(sim->d_count, 0, sizeof(unsigned int) * MateSim::kMaxHostChunks * 2, sim->hstreams[0]));
-        CUDA_TRY(cudaEventRecord(sim->hevents[1], sim->hstreams[0]));
-        for (int i = 1; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamWaitEvent(sim->hstreams[i], sim->hevents[1], 0));
-        int kc = 0;
-        for (int begin = 0; begin < B; begin += chunk, ++kc) {
-            const int count = std::min(chunk, B - begin);
-            cudaStream_t s = sim->hstreams[kc % MateSim::kHostStreams];
-            if (nc) CUDA_TRY(cudaMemcpyAsync(sim->h_cam_act + (size_t)begin * nc * 2, cam_act + (size_t)begin * nc * 2, sizeof(float) * count * nc * 2, cudaMemcpyHostToDevice, s));
-            CUDA_TRY(cudaMemcpyAsync(sim->h_tgt_act + (size_t)begin * nt * 2, tgt_act + (size_t)begin * nt * 2, sizeof(float) * count * nt * 2, cudaMemcpyHostToDevice, s));
-            if (int rc = launch_range(sim, p, begin, count, s)) return rc;
-            for (int r = 0; r < 2; ++r) {
-                table_base[2 * (kc + 1) + r] = table_base[2 * kc + r];
-                if (per_env[r] == 0) continue;
-                const size_t first = (size_t)begin * per_env[r] / 16;            // B % 4 == 0 and chunk % 4 == 0: whole chunks
-                const long long nchunks = (long long)((size_t)count * per_env[r] / 16);
-                const long long nblocks = (nchunks + kCompactBlock - 1) / kCompactBlock;
-                CompactEntry* table = sim->d_table[r] + table_base[2 * kc + r];
-                table_base[2 * (kc + 1) + r] += nblocks;
-                if (delta) compact_changes_kernel<<<1184, 128, 0, s>>>(reinterpret_cast<const uint4*>(dev_rows[r]) + first, reinterpret_cast<const uint4*>(rows_before[r]) + first,
-                                                                       nchunks, sim->d_compact[r] + first, table, sim->d_count + 2 * kc + r);
-                else compact_chunks_kernel<<<1184, 128, 0, s>>>(reinterpret_cast<const uint4*>(dev_rows[r]) + first, nchunks,
-                                                                sim->d_compact[r] + first, table, sim->d_count + 2 * kc + r);
-            }
-            sim->launches += (nc ? 2 : 1);
-            // The sizes of the chunk's compact streams go to the host by a store into pinned memory, not by a copy: a copy
-            // would queue behind the compact streams of earlier chunks on the copy engine, and the next stream could only be
-            // enqueued after the previous one had crossed the link (a bubble per chunk).
-            publish_counts_kernel<<<1, 32, 0, s>>>(sim->d_count + 2 * kc, sim->p_count_dev + 2 * kc);
-            CUDA_TRY(cudaEventRecord(sim->e_counts[kc], s));
-            for (int r = 0; r < 2; ++r) {
-                const long long nblocks = table_base[2 * (kc + 1) + r] - table_base[2 * kc + r];
-                if (nblocks > 0) CUDA_TRY(cudaMemcpyAsync(sim->p_table[r] + table_base[2 * kc + r], sim->d_table[r] + table_base[2 * kc + r], sizeof(CompactEntry) * nblocks, cudaMemcpyDeviceToHost, s));
-            }
-            CUDA_TRY(cudaMemcpyAsync(rewards + (size_t)begin * 2, sim->h_rewards + (size_t)begin * 2, sizeof(float) * count * 2, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(cudaMemcpyAsync(done + begin, sim->h_done + begin, count, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(cudaEventRecord(sim->e_tables[kc], s));
-        }
-        t_enq = since();
-        // the sizes are known once a chunk's kernels have run: its compact streams go on the copy stream in chunk order
-        const int pieces = std::max(1, sim->pool->size());
-        kc = 0;
-        for (int begin = 0; begin < B; begin += chunk, ++kc) {
-            CUDA_TRY(cudaEventSynchronize(sim->e_counts[kc]));
-            CUDA_TRY(cudaStreamWaitEvent(sim->copy_stream, sim->e_tables[kc], 0));   // a chunk's stream event then covers its tables too
-            for (int r = 0; r < 2; ++r) {
-                if (per_env[r] == 0 || sim->p_count[2 * kc + r] == 0) continue;
-                const size_t first = (size_t)begin * per_env[r] / 16;
-                CUDA_TRY(cudaMemcpyAsync(sim->p_compact[r] + first, sim->d_compact[r] + first, (size_t)sim->p_count[2 * kc + r] * 16,
-                                         cudaMemcpyDeviceToHost, sim->copy_stream));
-            }
-            CUDA_TRY(cudaEventRecord(sim->e_stream[kc], sim->copy_stream));
-            // expansion: the pool's threads wait for the chunk's stream themselves, so the caller's thread goes on to the next sizes
-            const int count = std::min(chunk, B - begin);
-            for (int r = 0; r < 2; ++r) {
-                if (per_env[r] == 0) continue;
-                const size_t first = (size_t)begin * per_env[r] / 16;
-                const long long nchunks = (long long)((size_t)count * per_env[r] / 16);
-                const long long nblocks = (nchunks + kCompactBlock - 1) / kCompactBlock;
-                const long long per_piece = (nblocks + pieces - 1) / pieces;
-                __m128i* dst = reinterpret_cast<__m128i*>(host_rows[r]) + first;
-                const bool aligned = (((uintptr_t)dst) & 15) == 0;
-                for (long long b0 = 0; b0 < nblocks; b0 += per_piece)
-                    sim->pool->submit(ExpandPool::Work{sim->p_table[r] + table_base[2 * kc + r], delta, reinterpret_cast<const __m128i*>(sim->p_compact[r] + first),
-                                                       dst, nchunks, b0, std::min(nblocks, b0 + per_piece), aligned, sim->e_stream[kc]});
-            }
-        }
-        t_counts = since();
-        CUDA_TRY(cudaStreamSynchronize(sim->copy_stream));
-        t_last_stream = since();
-        sim->pool->wait();
-        for (int i = 0; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamSynchronize(sim->hstreams[i]));
-        {
-            unsigned long long link = 0;
-            for (int i = 0; i < 2 * num_chunks; ++i) link += (unsigned long long)sim->p_count[i] * 16ull;
-            link += (unsigned long long)(table_base[2 * num_chunks] + table_base[2 * num_chunks + 1]) * sizeof(CompactEntry);
-            sim->last_leg = delta ? 2 : 1; sim->last_link_bytes = link;
-        }
-        // the caller's buffers and the device now hold this call's rows
+    if (int rc = compact ? compact_leg(sim, p, chunk, delta, rows_before, cam_act, tgt_act, cam_obs, tgt_obs, rewards, done)
+                         : dense_leg(sim, p, chunk, cam_act, tgt_act, cam_obs, tgt_obs, rewards, done))
+        return rc;
+    if (compact || two_buffers) {   // the caller's buffers and the device hold this call's rows: the next call may send changes only
         sim->kept_rows[0] = cam_obs; sim->kept_rows[1] = tgt_obs; sim->kept_valid = true;
-        if (two_buffers) sim->row_parity ^= 1;
-        if (trace) {
-            unsigned long long kept = 0;
-            for (int i = 0; i < 2 * num_chunks; ++i) kept += sim->p_count[i];
-            fprintf(stderr, "step_host compact: enqueued %.2f ms, sizes known + copies enqueued %.2f, last stream arrived %.2f, expanded %.2f; kept %.1f MB of %.1f MB, %d threads, changes only %d\n",
-                    t_enq, t_counts, t_last_stream, since(), kept * 16 / 1e6, (per_env[0] + per_env[1]) * (double)B / 1e6, sim->pool->size(), (int)delta);
-        }
-        if ((flags & MATE_STEP_AUTO_RESET) && sim->refill_mode &&
-            (sim->refill_mode == 2 || ++sim->steps_since_refill >= sim->refill_period))
-            return launch_prepare(sim, nullptr);
-        return MATE_OK;
     }
-    int k = 0;
-    for (int begin = 0; begin < B; begin += chunk, ++k) {
-        const int count = std::min(chunk, B - begin);
-        cudaStream_t s = sim->hstreams[k % MateSim::kHostStreams];
-        if (nc) CUDA_TRY(cudaMemcpyAsync(sim->h_cam_act + (size_t)begin * nc * 2, cam_act + (size_t)begin * nc * 2, sizeof(float) * count * nc * 2, cudaMemcpyHostToDevice, s));
-        CUDA_TRY(cudaMemcpyAsync(sim->h_tgt_act + (size_t)begin * nt * 2, tgt_act + (size_t)begin * nt * 2, sizeof(float) * count * nt * 2, cudaMemcpyHostToDevice, s));
-        if (int rc = launch_range(sim, p, begin, count, s)) return rc;
-        const size_t esz = obs_elem_bytes(sim);
-        if (nc) CUDA_TRY(cudaMemcpyAsync(obs_advance(sim, cam_obs, (size_t)begin * nc * dc), obs_advance(sim, rows_now[0], (size_t)begin * nc * dc), esz * count * nc * dc, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaMemcpyAsync(obs_advance(sim, tgt_obs, (size_t)begin * nt * dt), obs_advance(sim, rows_now[1], (size_t)begin * nt * dt), esz * count * nt * dt, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaMemcpyAsync(rewards + (size_t)begin * 2, sim->h_rewards + (size_t)begin * 2, sizeof(float) * count * 2, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaMemcpyAsync(done + begin, sim->h_done + begin, count, cudaMemcpyDeviceToHost, s));
-    }
-    for (int i = 0; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamSynchronize(sim->hstreams[i]));
-    sim->last_leg = 0; sim->last_link_bytes = (unsigned long long)B * ((size_t)nc * dc + (size_t)nt * dt) * obs_elem_bytes(sim);
-    if (two_buffers) {   // the caller's buffers and the device hold this call's rows: the next call may send changes only
-        sim->kept_rows[0] = cam_obs; sim->kept_rows[1] = tgt_obs; sim->kept_valid = true; sim->row_parity ^= 1;
-    }
+    if (two_buffers) sim->row_parity ^= 1;
     // the prepared episodes are refilled on the side stream like on the device path
-    if ((flags & MATE_STEP_AUTO_RESET) && sim->refill_mode &&
-        (sim->refill_mode == 2 || ++sim->steps_since_refill >= sim->refill_period))
-        return launch_prepare(sim, nullptr);
-    return MATE_OK;
+    return refill_after_step(sim, flags, nullptr);
 }
 
 // ---- state get / set (host arrays, synchronous) --------------------------------------------------
@@ -1026,6 +1032,18 @@ static int upload(const std::vector<T>& host, T* dev) {
     CUDA_TRY(cudaMemcpy(dev, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice));
     return MATE_OK;
 }
+// struct-of-arrays values [rows][bpad] -> component k of the batched rows [B][rows][comps] of a MateStateView field
+template <typename T>
+static void gather_rows(const MateSim* sim, const std::vector<T>& soa, int rows, T* out, int comps, int k) {
+    for (size_t e = 0; e < (size_t)sim->num_envs; ++e)
+        for (int r = 0; r < rows; ++r) out[(e * rows + r) * comps + k] = soa[r * (size_t)sim->bpad + e];
+}
+// component k of the batched rows [B][rows][comps] of a MateStateView field -> struct-of-arrays values [rows][bpad]
+template <typename T>
+static void scatter_rows(const MateSim* sim, const T* in, int rows, int comps, int k, std::vector<T>& soa) {
+    for (size_t e = 0; e < (size_t)sim->num_envs; ++e)
+        for (int r = 0; r < rows; ++r) soa[r * (size_t)sim->bpad + e] = in[(e * rows + r) * comps + k];
+}
 
 extern "C" int mate_b200_get_state(MateSim* sim, MateStateView* v) {
     if (!sim || !v) return fail(MATE_EINVAL, "null argument");
@@ -1037,22 +1055,20 @@ extern "C" int mate_b200_get_state(MateSim* sim, MateStateView* v) {
     std::vector<double> a, b2, c, d;
     if (nc && (v->cam_xy || v->cam_phi || v->cam_theta)) {
         if (download(a, p.cam_x, nc * bp) || download(b2, p.cam_y, nc * bp) || download(c, p.cam_phi, nc * bp) || download(d, p.cam_theta, nc * bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < nc; ++k) {
-                if (v->cam_xy) { v->cam_xy[(e * nc + k) * 2] = a[k * bp + e]; v->cam_xy[(e * nc + k) * 2 + 1] = b2[k * bp + e]; }
-                if (v->cam_phi) v->cam_phi[e * nc + k] = c[k * bp + e];
-                if (v->cam_theta) v->cam_theta[e * nc + k] = d[k * bp + e];
-            }
+        if (v->cam_xy) { gather_rows(sim, a, nc, v->cam_xy, 2, 0); gather_rows(sim, b2, nc, v->cam_xy, 2, 1); }
+        if (v->cam_phi) gather_rows(sim, c, nc, v->cam_phi, 1, 0);
+        if (v->cam_theta) gather_rows(sim, d, nc, v->cam_theta, 1, 0);
     }
     if (v->tgt_xy) {
         if (download(a, p.tgt_x, nt * bp) || download(b2, p.tgt_y, nt * bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < nt; ++k) { v->tgt_xy[(e * nt + k) * 2] = a[k * bp + e]; v->tgt_xy[(e * nt + k) * 2 + 1] = b2[k * bp + e]; }
+        gather_rows(sim, a, nt, v->tgt_xy, 2, 0);
+        gather_rows(sim, b2, nt, v->tgt_xy, 2, 1);
     }
     if (no && v->obs_xyr) {
         if (download(a, p.obs_x, no * bp) || download(b2, p.obs_y, no * bp) || download(c, p.obs_r, no * bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < no; ++k) { v->obs_xyr[(e * no + k) * 3] = a[k * bp + e]; v->obs_xyr[(e * no + k) * 3 + 1] = b2[k * bp + e]; v->obs_xyr[(e * no + k) * 3 + 2] = c[k * bp + e]; }
+        gather_rows(sim, a, no, v->obs_xyr, 3, 0);
+        gather_rows(sim, b2, no, v->obs_xyr, 3, 1);
+        gather_rows(sim, c, no, v->obs_xyr, 3, 2);
     }
     {
         std::vector<uint32_t> pack;
@@ -1095,30 +1111,27 @@ extern "C" int mate_b200_set_state(MateSim* sim, const MateStateView* v) {
     std::vector<double> a, b2, c, d;
     if (nc) {
         if (download(a, p.cam_x, nc * bp) || download(b2, p.cam_y, nc * bp) || download(c, p.cam_phi, nc * bp) || download(d, p.cam_theta, nc * bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < nc; ++k) {
-                if (v->cam_xy) { a[k * bp + e] = v->cam_xy[(e * nc + k) * 2]; b2[k * bp + e] = v->cam_xy[(e * nc + k) * 2 + 1]; }
-                if (v->cam_phi) c[k * bp + e] = v->cam_phi[e * nc + k];
-                if (v->cam_theta) {
-                    const double th = v->cam_theta[e * nc + k];
-                    if (!(th > 0.0) || th > 180.0) return fail(MATE_EINVAL, "cam_theta out of (0, 180]");
-                    d[k * bp + e] = th;
-                }
-            }
+        if (v->cam_theta)
+            for (size_t i = 0; i < B * nc; ++i)
+                if (!(v->cam_theta[i] > 0.0) || v->cam_theta[i] > 180.0) return fail(MATE_EINVAL, "cam_theta out of (0, 180]");
+        if (v->cam_xy) { scatter_rows(sim, v->cam_xy, nc, 2, 0, a); scatter_rows(sim, v->cam_xy, nc, 2, 1, b2); }
+        if (v->cam_phi) scatter_rows(sim, v->cam_phi, nc, 1, 0, c);
+        if (v->cam_theta) scatter_rows(sim, v->cam_theta, nc, 1, 0, d);
         if (upload(a, p.cam_x) || upload(b2, p.cam_y) || upload(c, p.cam_phi) || upload(d, p.cam_theta)) return MATE_ECUDA;
     }
     if (v->cam_xy || v->obs_xyr)   // geometry changed: invalidate the per-episode camera line-of-sight cache
         CUDA_TRY(cudaMemset(p.cc_clear, 0, sizeof(unsigned long long) * bp));
     if (v->tgt_xy) {
         a.assign(nt * bp, 0.0); b2.assign(nt * bp, 0.0);
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < nt; ++k) { a[k * bp + e] = v->tgt_xy[(e * nt + k) * 2]; b2[k * bp + e] = v->tgt_xy[(e * nt + k) * 2 + 1]; }
+        scatter_rows(sim, v->tgt_xy, nt, 2, 0, a);
+        scatter_rows(sim, v->tgt_xy, nt, 2, 1, b2);
         if (upload(a, p.tgt_x) || upload(b2, p.tgt_y)) return MATE_ECUDA;
     }
     if (no && v->obs_xyr) {
         a.assign(no * bp, 0.0); b2.assign(no * bp, 0.0); c.assign(no * bp, 0.0);
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < no; ++k) { a[k * bp + e] = v->obs_xyr[(e * no + k) * 3]; b2[k * bp + e] = v->obs_xyr[(e * no + k) * 3 + 1]; c[k * bp + e] = v->obs_xyr[(e * no + k) * 3 + 2]; }
+        scatter_rows(sim, v->obs_xyr, no, 3, 0, a);
+        scatter_rows(sim, v->obs_xyr, no, 3, 1, b2);
+        scatter_rows(sim, v->obs_xyr, no, 3, 2, c);
         if (upload(a, p.obs_x) || upload(b2, p.obs_y) || upload(c, p.obs_r)) return MATE_ECUDA;
         std::vector<float4> f4(no * bp);   // fp32 shadow read by the prefilters and the observation packer
         for (size_t i = 0; i < f4.size(); ++i) f4[i] = make_float4((float)a[i], (float)b2[i], (float)c[i], 0.f);
