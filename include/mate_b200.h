@@ -21,7 +21,7 @@
  *     (the ``float* cam_obs / tgt_obs`` arguments) may instead be float16 per handle, see
  *     mate_b200_set_observation_format: the arguments then address buffers of that type;
  *   - a handle is not re-entrant; different handles are independent (one per GPU);
- *   - step/reset/observe enqueue work on the given stream and never synchronise the host.
+ *   - step/reset/observe/save_state/load_state enqueue work on the given stream and never synchronise the host.
  */
 #ifndef MATE_B200_H_
 #define MATE_B200_H_
@@ -211,9 +211,62 @@ int mate_b200_step_host(MateSim* sim, const float* cam_act, const float* tgt_act
                         float* cam_obs, float* tgt_obs, float* rewards, uint8_t* done,
                         uint32_t flags);
 
-/* State checkpoint / injection (host arrays; synchronises the device). */
+/* State view / injection (host arrays; synchronises the device).  A view, not a complete checkpoint: it leaves out the
+ * running coverage sum, the line-of-sight cache, the Philox seed and the episode statistics; use mate_b200_save_state
+ * to save and restore a batch exactly. */
 int mate_b200_get_state(MateSim* sim, MateStateView* view);
 int mate_b200_set_state(MateSim* sim, const MateStateView* view);
+
+/* Device-side state snapshots: the complete per-environment state of a batch, saved to and loaded from a device buffer
+ * without leaving the device, for exact resume (checkpoints) and for branching (environment d takes the state of
+ * environment s).  The payload is a caller-owned device buffer on the handle's device, 16-byte aligned, of
+ * mate_b200_snapshot_bytes(count) bytes; its layout is private to the library and tagged with MATE_SNAPSHOT_VERSION.
+ * The library allocates nothing for snapshots.  Both calls only enqueue work on `stream`, like mate_b200_step.
+ *
+ * What a snapshot holds: every live state array of the environments (entities, target and cargo integers, episode
+ * step / id / rewards / coverage sum, the per-episode line-of-sight cache), copied verbatim, plus the handle's 16
+ * episode-statistics accumulators.  Observation rows and MateStepAux outputs are not saved: mate_b200_observe
+ * recomputes them.
+ *
+ * Random draws after a load: a reset is a function of (seed, global environment index, episode id) and the step's
+ * draws (transmission, goal choice) of (seed, global environment index, episode id, episode step).  An environment
+ * restored at its own global index under the saving handle's seed therefore replays exactly.  A clone at another index
+ * shares the state but draws its own outcomes from its next step on, unless the step is given a MateReplay. */
+#define MATE_SNAPSHOT_VERSION 1
+typedef struct MateSnapshotInfo {      /* host-side header of a device payload */
+    int32_t version;                   /* MATE_SNAPSHOT_VERSION */
+    int32_t num_cameras, num_targets, num_obstacles;
+    int32_t count;                     /* environments in the payload */
+    int32_t reserved;
+    uint64_t config_hash;              /* fingerprint of the MateConfig the saving handle was created with: 64-bit FNV-1a
+                                          over its scalar fields (reserved0 excepted) and the values of its three range
+                                          arrays, in declaration order */
+    uint64_t seed;                     /* the saving handle's Philox key */
+    uint64_t payload_bytes;
+} MateSnapshotInfo;
+
+/* Bytes of the payload of a snapshot of `count` (> 0) environments of this handle's shape. */
+int mate_b200_snapshot_bytes(const MateSim* sim, int32_t count, uint64_t* bytes);
+
+/* Save: payload entry i gets the state of environment env[i] (dev int32 [count]; NULL = every environment, which
+ * requires count == num_envs).  An entry of env outside [0, num_envs) leaves payload entry i unwritten.  Fills *info
+ * on the host without reading device memory (it never synchronises). */
+int mate_b200_save_state(MateSim* sim, const int32_t* env, int32_t count, void* payload,
+                         MateSnapshotInfo* info, void* stream);
+
+/* Load: environment d takes payload entry src[d] (dev int32 [num_envs]; NULL = entry d for every d, which requires
+ * info->count == num_envs); a negative or out-of-range entry keeps environment d as it is.  Only the mapped environments
+ * change; the handle's seed and statistics stay.  With MATE_LOAD_STATE_RESUME (requires src == NULL) the handle also
+ * takes the saving handle's seed (info->seed) and statistics, so that the batch continues bit for bit.
+ * The saving and the loading handle need the same (Nc, Nt, No) and configuration (config_hash); their observation
+ * format, env_index_base and num_envs may differ.  A load is allowed before the first reset and does not fix the
+ * observation format.  The prepared next episodes of the loaded environments are discarded and prepared again (on
+ * the side stream, ordered after the load); the load waits for a prepare still running with an event, not by
+ * synchronising the host.  MATE_EINVAL, with the handle unchanged, for another version, shape or configuration, a
+ * count <= 0, a NULL map with a count other than num_envs, RESUME with a map, or a misaligned payload. */
+#define MATE_LOAD_STATE_RESUME 1u
+int mate_b200_load_state(MateSim* sim, const void* payload, const MateSnapshotInfo* info,
+                         const int32_t* src, uint32_t flags, void* stream);
 
 /* Episode statistics accumulated on device since the last call with reset_after != 0:
  * out[0]=episodes finished, [1]=sum return (target team), [2]=sum length,

@@ -22,6 +22,8 @@ MATE_STEP_AUTO_RESET = 1
 MATE_STEP_HOST_ROWS_KEPT = 2
 MATE_OBS_FORMAT_F32 = 0
 MATE_OBS_FORMAT_F16 = 1
+MATE_SNAPSHOT_VERSION = 1
+MATE_LOAD_STATE_RESUME = 1
 
 
 class MateConfig(ctypes.Structure):
@@ -115,6 +117,23 @@ class MateReplay(ctypes.Structure):
     _fields_ = [('transmit', c_uint8_p), ('goal_choice', c_int8_p)]
 
 
+SNAPSHOT_INFO_FIELDS = ('version', 'num_cameras', 'num_targets', 'num_obstacles', 'count', 'config_hash', 'seed', 'payload_bytes')
+
+
+class MateSnapshotInfo(ctypes.Structure):
+    _fields_ = [
+        ('version', ctypes.c_int32),
+        ('num_cameras', ctypes.c_int32),
+        ('num_targets', ctypes.c_int32),
+        ('num_obstacles', ctypes.c_int32),
+        ('count', ctypes.c_int32),
+        ('reserved', ctypes.c_int32),
+        ('config_hash', ctypes.c_uint64),
+        ('seed', ctypes.c_uint64),
+        ('payload_bytes', ctypes.c_uint64),
+    ]
+
+
 def alloc_state_arrays(B, nc, nt, no):
     """Fresh host arrays for every MateStateView field."""
     return {name: np.zeros(shape(B, nc, nt, no), dtype=dtype) for name, _, dtype, shape in STATE_FIELDS}
@@ -186,6 +205,9 @@ def load_library():
     lib.mate_b200_get_state.argtypes = [void_p, ctypes.POINTER(MateStateView)]
     lib.mate_b200_set_state.argtypes = [void_p, ctypes.POINTER(MateStateView)]
     lib.mate_b200_episode_stats.argtypes = [void_p, void_p, ctypes.c_int32, void_p]
+    lib.mate_b200_snapshot_bytes.argtypes = [void_p, ctypes.c_int32, ctypes.POINTER(ctypes.c_uint64)]
+    lib.mate_b200_save_state.argtypes = [void_p, void_p, ctypes.c_int32, void_p, ctypes.POINTER(MateSnapshotInfo), void_p]
+    lib.mate_b200_load_state.argtypes = [void_p, void_p, ctypes.POINTER(MateSnapshotInfo), void_p, ctypes.c_uint32, void_p]
     lib.mate_b200_launch_count.argtypes = [void_p]
     lib.mate_b200_launch_count.restype = ctypes.c_int64
     lib.mate_b200_host_leg_info.argtypes = [void_p, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_uint64)]
@@ -201,7 +223,7 @@ def load_library():
                                                     ctypes.POINTER(MateCameraAgentReplay), void_p, void_p]
     lib.mate_b200_soft_coverage.argtypes = [void_p, void_p, void_p, void_p, void_p]
     for name in ('create', 'destroy', 'obs_dims', 'set_observation_format', 'reset', 'seed', 'step', 'observe', 'step_host',
-                 'get_state', 'set_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions'):
+                 'get_state', 'set_state', 'snapshot_bytes', 'save_state', 'load_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions'):
         getattr(lib, 'mate_b200_' + name).restype = ctypes.c_int
     _LIB = lib
     return lib
@@ -210,7 +232,8 @@ def load_library():
 EXPORTED_SYMBOLS = [
     'mate_b200_last_error', 'mate_b200_abi_version', 'mate_b200_create', 'mate_b200_destroy',
     'mate_b200_obs_dims', 'mate_b200_set_observation_format', 'mate_b200_reset', 'mate_b200_seed', 'mate_b200_step', 'mate_b200_observe',
-    'mate_b200_step_host', 'mate_b200_get_state', 'mate_b200_set_state',
+    'mate_b200_step_host', 'mate_b200_get_state', 'mate_b200_set_state', 'mate_b200_snapshot_bytes', 'mate_b200_save_state',
+    'mate_b200_load_state',
     'mate_b200_episode_stats', 'mate_b200_launch_count', 'mate_b200_host_leg_info', 'mate_b200_transform_observations', 'mate_b200_set_observation_ops',
     'mate_b200_decode_actions', 'mate_b200_auxiliary_terms', 'mate_b200_fov_range', 'mate_b200_soft_coverage', 'mate_b200_greedy_target_actions', 'mate_b200_greedy_camera_actions',
 ]

@@ -20,6 +20,7 @@
 #include "mate_wrappers.cuh"
 #include "mate_agents.cuh"
 #include "mate_hostpath.cuh"
+#include "mate_snapshot.cuh"
 
 using namespace mate;
 
@@ -185,6 +186,7 @@ struct MateSim {
     size_t state_bytes = 0;
     double* d_ranges = nullptr;
     unsigned long long seed = 0;
+    uint64_t config_hash = 0; // fingerprint of cfg (config_fingerprint): snapshots load only into handles of the same configuration
     long long launches = 0;
     // prepared resets (mate_step.cuh): second state block, parameter block that addresses it, side stream
     void* next_block = nullptr;
@@ -292,6 +294,26 @@ static size_t carve_state(Params& p, char* block, int nc, int nt, int no, size_t
     return off;
 }
 
+// 64-bit FNV-1a over the scalar fields of a MateConfig (reserved0 excepted) and the values of its three range arrays,
+// in declaration order (MateSnapshotInfo::config_hash)
+static uint64_t config_fingerprint(const MateConfig& c) {
+    uint64_t h = 14695981039346656037ull;
+    auto mix = [&](const void* data, size_t bytes) {
+        for (size_t i = 0; i < bytes; ++i) { h ^= static_cast<const unsigned char*>(data)[i]; h *= 1099511628211ull; }
+    };
+    for (const int32_t v : {c.num_cameras, c.num_targets, c.num_obstacles, c.max_episode_steps, c.num_cargoes_per_target,
+                            c.num_high_capacity_targets, c.targets_start_with_cargoes, c.shuffle_entities, c.reward_sparse})
+        mix(&v, sizeof(v));
+    for (const double v : {c.bounty_factor, c.camera_radius, c.camera_min_viewing_angle, c.camera_max_sight_range,
+                           c.camera_rotation_step, c.camera_zooming_step, c.target_step_size, c.target_sight_range,
+                           c.obstacle_transmittance, c.obstacle_radius_low, c.obstacle_radius_high})
+        mix(&v, sizeof(v));
+    if (c.num_cameras > 0) mix(c.camera_location_ranges, sizeof(double) * 4 * c.num_cameras);
+    mix(c.target_location_ranges, sizeof(double) * 4 * c.num_targets);
+    if (c.num_obstacles > 0) mix(c.obstacle_location_ranges, sizeof(double) * 4 * c.num_obstacles);
+    return h;
+}
+
 extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t device,
                                 int64_t env_index_base, MateSim** out) {
     if (!cfg || !out) return fail(MATE_EINVAL, "null argument");
@@ -324,6 +346,7 @@ extern "C" int mate_b200_create(const MateConfig* cfg, int32_t num_envs, int32_t
     CUDA_TRY(kernel.prepare_wrappers());
     std::unique_ptr<MateSim> sim(new MateSim());   // frees what is made so far on every early return
     sim->cfg = *cfg;
+    sim->config_hash = config_fingerprint(*cfg);
     sim->cfg.camera_location_ranges = sim->cfg.target_location_ranges = sim->cfg.obstacle_location_ranges = nullptr;
     sim->num_envs = num_envs;
     sim->device = device;
@@ -1177,6 +1200,90 @@ extern "C" int mate_b200_set_state(MateSim* sim, const MateStateView* v) {
         if (upload(cargo, p.cargo) || upload(ea, p.env_a) || upload(eb, p.env_b)) return MATE_ECUDA;
     }
     return launch_prepare(sim, nullptr);   // prepare the next episodes of the new state right away
+}
+
+// ---- device-side snapshots (mate_snapshot.cuh) ----------------------------------------------------------------------
+// The payload of `count` environments: every array of for_each_state_array as rows x count elements ([row * count + i]),
+// each section 256-byte aligned, then the 16 floats of `stats`.  With a table the sections are bound to the handle's live
+// arrays and to `payload`; table->n counts the arrays even past kSnapMaxArrays.  Returns the payload bytes.
+static size_t snapshot_layout(const MateSim* sim, size_t count, char* payload, SnapTable* table) {
+    Params p = sim->base;
+    size_t off = 0;
+    if (table) { *table = SnapTable{}; table->bpad = sim->bpad; table->num_envs = sim->num_envs; table->count = (int)count; table->stats = p.stats; }
+    for_each_state_array(p, sim->cfg.num_cameras, sim->cfg.num_targets, sim->cfg.num_obstacles, [&](auto*& ptr, int rows) {
+        const size_t elem = sizeof(*ptr);
+        if (table && rows > 0) {
+            if (table->n < kSnapMaxArrays)
+                table->a[table->n] = SnapArray{reinterpret_cast<char*>(ptr), payload + off, rows, (int)elem};
+            table->n += 1;
+            table->rows += rows;
+        }
+        off = align_up(off + elem * rows * count, 256);
+    });
+    if (table) table->payload_stats = reinterpret_cast<float*>(payload + off);
+    return off + sizeof(float) * 16;
+}
+
+extern "C" int mate_b200_snapshot_bytes(const MateSim* sim, int32_t count, uint64_t* bytes) {
+    if (!sim || !bytes) return fail(MATE_EINVAL, "null argument");
+    if (count <= 0) return fail(MATE_EINVAL, "count must be positive");
+    *bytes = snapshot_layout(sim, (size_t)count, nullptr, nullptr);
+    return MATE_OK;
+}
+
+extern "C" int mate_b200_save_state(MateSim* sim, const int32_t* env, int32_t count, void* payload, MateSnapshotInfo* info,
+                                    void* stream) {
+    if (!sim || !payload || !info) return fail(MATE_EINVAL, "null argument");
+    if (count <= 0) return fail(MATE_EINVAL, "count must be positive");
+    if (!env && count != sim->num_envs) return fail(MATE_EINVAL, "without an environment list the snapshot holds every environment: count must be num_envs");
+    if ((uintptr_t)payload & 15) return fail(MATE_EINVAL, "the snapshot payload must be 16-byte aligned");
+    SnapTable t;
+    const size_t bytes = snapshot_layout(sim, (size_t)count, static_cast<char*>(payload), &t);
+    if (t.n > kSnapMaxArrays) return fail(MATE_EINVAL, "more state arrays than the snapshot table holds (kSnapMaxArrays)");
+    CUDA_TRY(cudaSetDevice(sim->device));
+    snapshot_gather_kernel<<<snapshot_grid(t, count), kSnapThreads, 0, (cudaStream_t)stream>>>(t, env);
+    sim->launches += 1;
+    if (int rc = check_launch("snapshot gather")) return rc;
+    *info = MateSnapshotInfo{};
+    info->version = MATE_SNAPSHOT_VERSION;
+    info->num_cameras = sim->cfg.num_cameras; info->num_targets = sim->cfg.num_targets; info->num_obstacles = sim->cfg.num_obstacles;
+    info->count = count;
+    info->config_hash = sim->config_hash;
+    info->seed = sim->seed;
+    info->payload_bytes = bytes;
+    return MATE_OK;
+}
+
+extern "C" int mate_b200_load_state(MateSim* sim, const void* payload, const MateSnapshotInfo* info, const int32_t* src,
+                                    uint32_t flags, void* stream) {
+    if (!sim || !payload || !info) return fail(MATE_EINVAL, "null argument");
+    if (info->version != MATE_SNAPSHOT_VERSION) return fail(MATE_EINVAL, "snapshot version " + std::to_string(info->version) + ", this library reads version " + std::to_string(MATE_SNAPSHOT_VERSION));
+    if (info->num_cameras != sim->cfg.num_cameras || info->num_targets != sim->cfg.num_targets || info->num_obstacles != sim->cfg.num_obstacles)
+        return fail(MATE_EINVAL, "the snapshot is of another shape (cameras, targets, obstacles)");
+    if (info->config_hash != sim->config_hash) return fail(MATE_EINVAL, "the snapshot was saved by a handle with another configuration");
+    if (info->count <= 0) return fail(MATE_EINVAL, "the snapshot's count must be positive");
+    if (flags & ~MATE_LOAD_STATE_RESUME) return fail(MATE_EINVAL, "unknown load flags");
+    const bool resume = (flags & MATE_LOAD_STATE_RESUME) != 0;
+    if (resume && src) return fail(MATE_EINVAL, "MATE_LOAD_STATE_RESUME restores the whole batch: it takes no map");
+    if (!src && info->count != sim->num_envs) return fail(MATE_EINVAL, "without a map the snapshot must hold num_envs environments");
+    if ((uintptr_t)payload & 15) return fail(MATE_EINVAL, "the snapshot payload must be 16-byte aligned");
+    SnapTable t;
+    const size_t bytes = snapshot_layout(sim, (size_t)info->count, static_cast<char*>(const_cast<void*>(payload)), &t);
+    if (info->payload_bytes != bytes) return fail(MATE_EINVAL, "the snapshot's payload_bytes do not match its count");
+    if (t.n > kSnapMaxArrays) return fail(MATE_EINVAL, "more state arrays than the snapshot table holds (kSnapMaxArrays)");
+    t.copy_stats = resume;
+    t.ready = sim->refill_mode ? sim->base.ready : nullptr;
+    CUDA_TRY(cudaSetDevice(sim->device));
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (sim->refill_mode == 1) {   // a prepare still running on the side stream writes the tags this load clears
+        CUDA_TRY(cudaEventRecord(sim->side_event, sim->side));
+        CUDA_TRY(cudaStreamWaitEvent(s, sim->side_event, 0));
+    }
+    snapshot_scatter_kernel<<<snapshot_grid(t, sim->num_envs), kSnapThreads, 0, s>>>(t, src);
+    sim->launches += 1;
+    if (int rc = check_launch("snapshot scatter")) return rc;
+    if (resume) sim->seed = info->seed;
+    return launch_prepare(sim, s);   // fresh prepared episodes for the loaded environments
 }
 
 extern "C" int mate_b200_episode_stats(MateSim* sim, float* out16, int32_t reset_after, void* stream) {

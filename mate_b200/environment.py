@@ -359,12 +359,40 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
 
     # ------------------------------------------------------------------ state access
     def get_state(self) -> Dict[str, np.ndarray]:
-        """Checkpoint of the full simulator state as host arrays (fields of ``MateStateView``)."""
+        """A view of the simulator state as host arrays (fields of ``MateStateView``).  It is not a complete checkpoint
+        (the running coverage sum, the line-of-sight cache, the seed and the episode statistics are left out):
+        ``save_state`` / ``load_state`` save and restore a batch exactly."""
         return self.sim.get_state()
 
+    def save_state(self, envs=None):
+        """Snapshot of the environments ``envs`` (``None`` = all; entry i = environment ``envs[i]``) on the device, with
+        this object's seed and NumPy RNG state (a :class:`mate_b200.sim.StateSnapshot`; ``torch.save`` keeps it)."""
+        snapshot = self.sim.save_state(envs)
+        kind, key, pos, has_gauss, cached = self._np_random.get_state()
+        snapshot.extras['environment'] = {'seed': self._seed,
+                                          'np_random': (kind, torch.from_numpy(key.astype(np.int64)), pos, has_gauss, cached)}
+        return snapshot
+
+    def load_state(self, snapshot, src=None, resume: bool = False):
+        """Load a snapshot and return the joint observation of the loaded state, like ``reset``.  ``src=None``: every
+        environment takes its own entry; otherwise environment d takes entry ``src[d]`` (a negative entry keeps d), e.g.
+        ``env.load_state(env.save_state(), src=idx)`` branches the batch from the environments ``idx``.  ``resume=True``
+        continues exactly where the snapshot was saved: it also restores the seed, the episode statistics and the NumPy
+        RNG state."""
+        self.sim.load_state(snapshot, src=src, resume=resume)
+        saved = snapshot.extras.get('environment')
+        if resume and saved is not None:
+            kind, key, pos, has_gauss, cached = saved['np_random']
+            self._seed = saved['seed']
+            self._np_random.set_state((kind, key.numpy().astype(np.uint32), pos, has_gauss, cached))
+        cam_obs, tgt_obs = self.sim.observe(aux=True)   # the mask attributes of the loaded state
+        self._needs_reset = False
+        self._state_serial += 1
+        return self._format_obs(cam_obs, tgt_obs)
+
     def set_state(self, arrays: Dict[str, np.ndarray]) -> None:
-        """Inject a state (the reference has no equivalent; used by the parity harness and for
-        checkpoint/resume)."""
+        """Inject a state (the reference has no equivalent; used by the parity harness).  For checkpoint / resume use
+        ``save_state`` / ``load_state``."""
         self.sim.set_state(arrays)
         self.sim.observe(aux=True)
         self._needs_reset = False

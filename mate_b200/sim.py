@@ -57,6 +57,34 @@ def check_observation_dtype(dtype):
     return dtype
 
 
+class StateSnapshot:
+    """The complete state of some environments of a batch, saved on the device (:meth:`BatchedSim.save_state`).
+
+    ``payload`` is a ``uint8`` tensor in the library's private layout; the header fields are those of
+    ``MateSnapshotInfo`` (``include/mate_b200.h``); ``py_seed`` is the saving simulator's Python-side seed, and
+    ``extras`` holds the per-snapshot state of the Python layers above the simulator (environment RNG, opponent
+    agents).  ``torch.save`` / ``torch.load`` keep it as it is; a payload on the CPU or on another GPU is copied to the
+    loading simulator's device."""
+
+    def __init__(self, payload, py_seed=0, extras=None, **header):
+        self.payload = payload
+        for name in _abi.SNAPSHOT_INFO_FIELDS:
+            setattr(self, name, int(header[name]))
+        self.py_seed = int(py_seed)
+        self.extras = {} if extras is None else extras
+
+    def info(self):
+        """The header as a ``MateSnapshotInfo``."""
+        return _abi.MateSnapshotInfo(**{name: getattr(self, name) for name in _abi.SNAPSHOT_INFO_FIELDS})
+
+    def __repr__(self):
+        return (f'StateSnapshot(count={self.count}, shape=({self.num_cameras}, {self.num_targets}, {self.num_obstacles}), '
+                f'{self.payload_bytes} bytes on {self.payload.device})')
+
+
+torch.serialization.add_safe_globals([StateSnapshot])   # torch.load(weights_only=True), the default, accepts it
+
+
 class BatchedSim:
     """One batch of MultiAgentTracking environments resident on one GPU.  ``observation_dtype`` is the element type of
     the observation rows (``cam_obs`` / ``tgt_obs``); everything else stays float32."""
@@ -312,6 +340,65 @@ class BatchedSim:
         arrays = dict(arrays)
         view = _abi.state_view_from_arrays(arrays)
         _check(self.lib, self.lib.mate_b200_set_state(self.handle, ctypes.byref(view)))
+
+    def _index_map(self, index, name, length, low, high):
+        """Environment / snapshot indices as an int32 tensor on the simulator's device (``None`` stays ``None``).  A host
+        sequence (or CPU tensor) is checked here: 1-D integers, ``length`` of them if given, each in ``[low, high)``,
+        else ``ValueError`` before any library call.  A device tensor is passed on without a synchronisation: the
+        library's kernels skip entries that are out of range."""
+        if index is None:
+            return None
+        if torch.is_tensor(index) and index.is_cuda:
+            if index.dtype.is_floating_point or index.dtype.is_complex or index.dtype == torch.bool:
+                raise ValueError(f'{name} must hold integers, got {index.dtype}')
+            host = None
+        else:
+            host = index.numpy() if torch.is_tensor(index) else np.asarray(index)
+            if host.dtype.kind not in 'iu':
+                raise ValueError(f'{name} must hold integers, got {host.dtype}')
+        size = tuple(index.shape) if host is None else host.shape
+        if len(size) != 1 or size[0] == 0 or (length is not None and size[0] != length):
+            raise ValueError(f'{name} must be a 1-D sequence of {length if length is not None else "one or more"} indices, got shape {size}')
+        if host is None:
+            return index.to(self.device, torch.int32).contiguous()
+        if host.min() < low or host.max() >= high:
+            raise ValueError(f'{name} has entries outside [{low}, {high})')
+        return torch.from_numpy(host.astype(np.int32)).to(self.device)
+
+    def snapshot_bytes(self, count):
+        """Bytes of the payload of a snapshot of ``count`` environments (mate_b200_snapshot_bytes)."""
+        out = ctypes.c_uint64(0)
+        _check(self.lib, self.lib.mate_b200_snapshot_bytes(self.handle, int(count), ctypes.byref(out)))
+        return int(out.value)
+
+    def save_state(self, envs=None):
+        """Snapshot of the environments ``envs`` (``None`` = the whole batch, entry i = environment ``envs[i]``), saved on
+        the device on the current stream (mate_b200_save_state): no synchronisation, no host copy of the state."""
+        index = self._index_map(envs, 'envs', None, 0, self.B)
+        with torch.cuda.device(self.device):
+            count = self.B if index is None else int(index.numel())
+            payload = torch.empty(self.snapshot_bytes(count), dtype=torch.uint8, device=self.device)
+            info = _abi.MateSnapshotInfo()
+            _check(self.lib, self.lib.mate_b200_save_state(self.handle, _dptr(index), count, _dptr(payload), ctypes.byref(info),
+                                                           self._stream()))
+        return StateSnapshot(payload, py_seed=self._seed, **{name: getattr(info, name) for name in _abi.SNAPSHOT_INFO_FIELDS})
+
+    def load_state(self, snapshot, src=None, resume=False):
+        """Load a snapshot on the current stream (mate_b200_load_state).  ``src=None``: environment d takes entry d (the
+        snapshot holds the whole batch); otherwise environment d takes entry ``src[d]`` (``B`` indices) and a negative
+        entry keeps environment d.  ``resume=True`` also takes the snapshot's seed and episode statistics, so the batch
+        continues bit for bit where it was saved (whole-batch snapshots only)."""
+        index = self._index_map(src, 'src', self.B, -(1 << 31), snapshot.count)
+        with torch.cuda.device(self.device):
+            payload = snapshot.payload
+            if payload.device != self.device:
+                payload = payload.to(self.device)
+            payload = payload.contiguous()
+            info = snapshot.info()
+            _check(self.lib, self.lib.mate_b200_load_state(self.handle, _dptr(payload), ctypes.byref(info), _dptr(index),
+                                                           _abi.MATE_LOAD_STATE_RESUME if resume else 0, self._stream()))
+        if resume:
+            self._seed = snapshot.py_seed
 
     def episode_stats(self, reset_after=False):
         with torch.cuda.device(self.device):

@@ -471,11 +471,67 @@ class AuxiliaryTargetRewards(_AuxiliaryRewards):
 # SURVEY.md section 8f, N4: single-team wrapper with a batched built-in opponent.
 # ------------------------------------------------------------------------------------------------------------
 
-class MultiCamera(Wrapper):
+class _SingleTeamSnapshot:
+    """``save_state`` / ``load_state`` of the single-team wrappers: besides the environment they carry the per-environment
+    state of the opponent agent (its memory, gathered / scattered along the memory's environment axis with the
+    snapshot's index map) and the pending reset mask; the agent's step serial is restored on resume only."""
+
+    _MEMORY_AXIS = None   # environment axis of the agent's field-major memory tensor
+    _TEAM = None          # index of this wrapper's team in the joint (camera, target) tuples
+
+    def _pending_resets(self):
+        base = self.unwrapped
+        if self._reset_mask is True:
+            return torch.ones(base.num_envs, dtype=torch.uint8, device=base.device)
+        if self._reset_mask is None:
+            return torch.zeros(base.num_envs, dtype=torch.uint8, device=base.device)
+        return torch.as_tensor(self._reset_mask, device=base.device).to(torch.uint8).clone()
+
+    def save_state(self, envs=None):
+        base = self.unwrapped
+        snapshot = self.env.save_state(envs)
+        agent = self.opponent_agent
+        memory, pending = agent._memory, self._pending_resets()   # pylint: disable=protected-access
+        if envs is not None:   # out-of-range device indices: the kernel leaves those entries unwritten, here they are clamped
+            index = base.sim._index_map(envs, 'envs', None, 0, base.num_envs).long().clamp_(0, base.num_envs - 1)  # pylint: disable=protected-access
+            memory, pending = memory.index_select(self._MEMORY_AXIS, index), pending.index_select(0, index)
+        snapshot.extras['opponent'] = {'memory': memory.clone(), 'reset_mask': pending.clone(), 'serial': agent._serial}  # pylint: disable=protected-access
+        return snapshot
+
+    def load_state(self, snapshot, src=None, resume=False):
+        base = self.unwrapped
+        joint_observation = self.env.load_state(snapshot, src=src, resume=resume)
+        saved = snapshot.extras['opponent']
+        agent = self.opponent_agent
+        memory, pending = agent._memory, self._pending_resets()   # pylint: disable=protected-access
+        saved_memory, saved_pending = saved['memory'].to(memory.device), saved['reset_mask'].to(pending.device)
+        if src is None:
+            memory.copy_(saved_memory)
+            pending = saved_pending.clone()
+        else:
+            index = base.sim._index_map(src, 'src', base.num_envs, -(1 << 31), snapshot.count).long()  # pylint: disable=protected-access
+            keep = (index < 0) | (index >= snapshot.count)
+            index = index.clamp(0, snapshot.count - 1)
+            shape = [1] * memory.dim()
+            shape[self._MEMORY_AXIS] = -1
+            memory.copy_(torch.where(keep.view(shape), memory, saved_memory.index_select(self._MEMORY_AXIS, index)))
+            pending = torch.where(keep, pending, saved_pending.index_select(0, index))
+        self._reset_mask = pending
+        if resume:
+            agent._serial = saved['serial']   # pylint: disable=protected-access
+        self.opponent_infos = None
+        self.opponent_joint_observation = joint_observation[1 - self._TEAM]
+        return joint_observation[self._TEAM]
+
+
+class MultiCamera(_SingleTeamSnapshot, Wrapper):
     """mate/wrappers/single_team.py:281-292: a single-team multi-agent environment for the camera team; the targets
     are played by ``target_agent`` (``mate_b200.agents.GreedyTargetAgent``), whose whole team acts in one kernel per
     step on the GPU.  ``reset`` returns the camera joint observation, ``step(camera_joint_action)`` returns
     ``(camera_joint_observation, camera_reward, done, camera_infos)``."""
+
+    _MEMORY_AXIS = 2   # GreedyTargetAgent memory [6, Nt, B]
+    _TEAM = 0
 
     def __init__(self, env, target_agent):
         from mate_b200 import agents  # pylint: disable=import-outside-toplevel
@@ -518,11 +574,14 @@ class MultiCamera(Wrapper):
         return f'<{type(self).__name__}(opponent={type(self.opponent_agent).__module__}.{type(self.opponent_agent).__name__}){self.env}>'
 
 
-class MultiTarget(Wrapper):
+class MultiTarget(_SingleTeamSnapshot, Wrapper):
     """mate/wrappers/single_team.py:295-306: a single-team multi-agent environment for the target team; the cameras
     are played by ``camera_agent`` (``mate_b200.agents.GreedyCameraAgent``), whose whole team acts in one kernel per
     step on the GPU.  ``reset`` returns the target joint observation, ``step(target_joint_action)`` returns
     ``(target_joint_observation, target_reward, done, target_infos)``."""
+
+    _MEMORY_AXIS = 1   # GreedyCameraAgent memory [M, B, Nc]
+    _TEAM = 1
 
     def __init__(self, env, camera_agent):
         from mate_b200 import agents  # pylint: disable=import-outside-toplevel
