@@ -312,11 +312,7 @@ __device__ __noinline__ double sight_range_at(const ObsRef ob, double cx, double
     // Both bracketing samples lie within 1 degree of the bearing, so a disc that cuts one of those two rays
     // is at an angular distance <= half + 1 degree from the bearing: it is in `passing` (discs outside the
     // camera's obstacle set are farther than rmax + R and cannot shorten a ray of length <= rmax).
-#ifdef MATE2_NO_CASTMASK
-    const unsigned long long near_discs = NO >= 64 ? ~0ull : ((1ull << NO) - 1ull);
-#else
     const unsigned long long near_discs = passing;
-#endif
     // phase 2: the sample angles of those obstacles, one obstacle per iteration (lanes of a warp that
     // evaluate different obstacles stay converged)
     while (passing != 0ull) {

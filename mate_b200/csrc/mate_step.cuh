@@ -25,9 +25,9 @@
 //   * OBSERVATIONS: the warp walks over its 32 environments; for each, the lanes are (observer row,
 //     entity) PAIRS: a pair writes the entity's public state + flag into the staged row if the observer's
 //     mask bit is set and zeros otherwise, every float of the block exactly once, and the finished block
-//     leaves the SM with 16-byte streaming stores (bulk copies are kept behind MATE2_COPYOUT=0; they were
-//     slower here, see DESIGN.md).  Masks (one or two words per observer row) and the fp32 entity values
-//     are handed from the simulation phase to this phase through shared memory.
+//     leaves the SM with 16-byte streaming stores (bulk copies were slower here, see DESIGN.md).  Masks (one or
+//     two words per observer row) and the fp32 entity values are handed from the simulation phase to this phase
+//     through shared memory.
 #pragma once
 
 #include <cuda_fp16.h>
@@ -37,29 +37,10 @@
 #include "mate_common.cuh"
 #include "mate_wrappers.cuh"
 
-#ifndef MATE2_ROLL_C
-#define MATE2_ROLL_C 5        // from this many cameras on, the loop over the observing camera of Camera.perceive stays rolled (instruction cache)
-#endif
-#ifndef MATE2_WARPS
-#define MATE2_WARPS 2          // warps per CTA (warps are independent; this only sets the CTA granularity)
-#endif
-#ifndef MATE2_COPYOUT
-#define MATE2_COPYOUT 1        // staged observation block -> HBM: 0 = bulk copy (TMA), 1 = 16-byte vector stores
-#endif
-#ifndef MATE2_STREAMING
-#define MATE2_STREAMING 1       // evict-first stores for the observation rows (written once, read by another kernel)
-#endif
-#ifndef MATE2_PF_OBS
-#define MATE2_PF_OBS 1         // fp64 obstacle discs -> L2 ahead of the exact paths: 0 = off, 1 = envs that will need them, 2 = all envs
-#endif
-#ifndef MATE2_PF_CARGO
-#define MATE2_PF_CARGO 1       // cargo tables -> L2 at the start of the step (read by _assign_goals, late in the chain)
-#endif
-#ifndef MATE2_MIN_CTAS
-#define MATE2_MIN_CTAS 8       // caps registers at 128 (4 warps per SM sub-partition); 65 536 envs = 2048 warp tiles = 13.8 per SM -> one wave
-#endif
-
 namespace mate {
+
+constexpr int kRollCamerasFrom = 5;   // from this many cameras on, the loop over the observing camera of Camera.perceive stays rolled (instruction cache)
+constexpr int kStepMinCtas = 8;       // caps registers at 128 (4 warps per SM sub-partition); 65 536 envs = 2048 warp tiles = 13.8 per SM -> one wave
 
 #ifdef MATE_DEV_TIMELINE   // development builds only: per-tile phase time stamps (profiles/tools/timeline.py)
 __device__ unsigned long long g_timeline[4096 * 8];
@@ -95,7 +76,7 @@ struct Shape2 {
     static constexpr int CAM_SKEW = (NC > 1 && DC % 32 == 0) ? 4 : 0;
     static constexpr int STAGE_CAM = ((NC * (DC + CAM_SKEW) + 3) / 4) * 4;
     static constexpr int STAGE_FLOATS = STAGE_CAM + ((TGT_ROW + 3) / 4) * 4;
-    static constexpr bool BULK = (CAM_ROW % 4 == 0) && (TGT_ROW % 4 == 0);   // 16-byte aligned blocks per env
+    static constexpr bool DENSE16 = (CAM_ROW % 4 == 0) && (TGT_ROW % 4 == 0);   // both teams' float32 rows of an env are 16-byte multiples
     static constexpr int E = NT + NO + NC;                     // entity slots (lanes of the scatter)
     // Obstacle slots of the packer: a slot is 4 floats, a row's slots are contiguous, and scalar stores of lanes 16 bytes
     // apart are 4-way bank conflicts.  Observer rows are therefore grouped by the ALIGNMENT of their obstacle block
@@ -127,7 +108,7 @@ struct Shape2 {
         r.n = plain;
         return r;
     }
-    static constexpr int WARPS = MATE2_WARPS;
+    static constexpr int WARPS = 2;   // warps per CTA (warps are independent; this only sets the CTA granularity)
     static constexpr int ENVS_PER_CTA = WARPS * 32;
     static constexpr int QCAP = 64;
     static constexpr int OFF_STAGE = 0;
@@ -640,6 +621,59 @@ __device__ __forceinline__ uint32_t half2_bits(const float lo, const float hi) {
     return *reinterpret_cast<const uint32_t*>(&h);
 }
 
+// One team's rows of an environment -> HBM: N values, staged in shared memory as float32 with rows of ROW values SKEW
+// floats apart (camera rows, Shape2::CAM_SKEW).  Each lane stores with the widest type whose size divides the part: 16, 8
+// or 4 bytes for float32, 16, 8, 4 or 2 bytes for float16 (the caller's buffers are 16-byte aligned, so the part of
+// environment i starts at a multiple of gcd(16, part bytes); MATE-4v2-9: 2 x 101 floats of target rows leave with 8-byte
+// stores).  float16 values are rounded from the staged ones in pairs (__float22half2_rn, nearest even).
+template <class OutT, int N, int ROW, int SKEW>
+__device__ __forceinline__ void store_team_rows(OutT* dst, const float* src) {
+    constexpr bool F16 = std::is_same<OutT, __half>::value;
+    constexpr int W = (F16 && N % 8 == 0) ? 8 : (N % 4 == 0 ? 4 : (N % 2 == 0 ? 2 : 1));   // values per store
+    static_assert(SKEW == 0 || (ROW % W == 0 && SKEW % 4 == 0), "a store must not straddle two skewed rows");
+    // staged index of chunk c of the part, in chunks of v floats.  The float32 loads index whole 16- / 8-byte chunks, the
+    // float16 loads single floats: the same addresses, but each form gives its format's packers the code they were
+    // measured with (ptxas allocates registers across all packers of a kernel, so one form for both changes the others)
+    auto at = [](const int c, const int v) { return SKEW ? c + (c / (ROW / v)) * (SKEW / v) : c; };
+    const float4* const src4 = reinterpret_cast<const float4*>(src);
+    const float2* const src2 = reinterpret_cast<const float2*>(src);
+    const int lane = threadIdx.x & 31;
+#pragma unroll
+    for (int it = 0; it < (N / W + 31) / 32; ++it) {
+        const int k = it * 32 + lane;
+        if (k < N / W) {
+            if constexpr (W == 8) {
+                // lanes 4-7 of every quarter-warp read their two 16-byte halves in the other order: each of the
+                // two loads then covers eight distinct 16-byte bank groups per quarter-warp
+                const int sw = (lane >> 2) & 1;
+                const float4 a = *reinterpret_cast<const float4*>(src + at(8 * k + 4 * sw, 1));
+                const float4 b = *reinterpret_cast<const float4*>(src + at(8 * k + 4 - 4 * sw, 1));
+                const float4 lo = sw ? b : a, hi = sw ? a : b;
+                __stcs(reinterpret_cast<uint4*>(dst) + k, make_uint4(half2_bits(lo.x, lo.y), half2_bits(lo.z, lo.w),
+                                                                     half2_bits(hi.x, hi.y), half2_bits(hi.z, hi.w)));
+            } else if constexpr (W == 4) {
+                if constexpr (F16) {
+                    const float4 a = *reinterpret_cast<const float4*>(src + at(4 * k, 1));
+                    __stcs(reinterpret_cast<uint2*>(dst) + k, make_uint2(half2_bits(a.x, a.y), half2_bits(a.z, a.w)));
+                } else {
+                    __stcs(reinterpret_cast<float4*>(dst) + k, src4[at(k, 4)]);
+                }
+            } else if constexpr (W == 2) {
+                if constexpr (F16) {
+                    const float2 a = *reinterpret_cast<const float2*>(src + at(2 * k, 1));
+                    __stcs(reinterpret_cast<unsigned int*>(dst) + k, half2_bits(a.x, a.y));
+                } else {
+                    __stcs(reinterpret_cast<float2*>(dst) + k, src2[at(k, 2)]);
+                }
+            } else if constexpr (F16) {
+                __stcs(reinterpret_cast<unsigned short*>(dst) + k, __half_as_ushort(__float2half_rn(src[at(k, 1)])));
+            } else {
+                dst[k] = src[at(k, 1)];   // odd float32 parts (MATE-1v1-x, 1v2-x): plain stores, the streaming hint is not measured there
+            }
+        }
+    }
+}
+
 // FOLD = the instantiation that also applies the registered observation wrappers (FoldOps, mate_common.cuh) while
 // the rows are composed; the common case (no wrappers) runs the FOLD = false instantiation, which has none of it.
 // OutT = element type of the rows in HBM (Params::obs_format): float, or __half rounded once from the staged fp32 rows
@@ -650,7 +684,6 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     using S = Shape2<NC, NT, NO>;
     constexpr bool F16 = std::is_same<OutT, __half>::value;
     static_assert(F16 || std::is_same<OutT, float>::value, "observation rows are float or __half");
-    static_assert(!(F16 && MATE2_COPYOUT == 0), "the bulk copy (MATE2_COPYOUT=0) moves bytes unchanged: float16 rows need MATE2_COPYOUT=1");
     constexpr int R = S::R, MW = S::MW, DC = S::DC, DT = S::DT, CV = S::CV;
     constexpr int NCX = NC > 0 ? NC : 1;
     constexpr uint32_t FULLMASK = 0xffffffffu;
@@ -842,8 +875,6 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
             }
             __syncwarp();
         }
-        // ---- everything is computed into registers first: the previous environment's bulk copy is
-        //      still reading the staged block, only the stores have to wait for it
         // Target.state public part (entities.py:631-637), Camera.state public part (entities.py:313-324)
         const uint32_t tpk = __float_as_uint(v[S::V_T + 3 * t_idx + 2]);
         const float t0 = v[S::V_T + 3 * t_idx], t1 = v[S::V_T + 3 * t_idx + 1];
@@ -862,10 +893,6 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
         for (int w = 0; w < NW; ++w) { sg[w] = (goal == w) ? (float)weight : 0.f; se[w] = (float)((empty >> w) & 1); }
         const float s_step = capacity == 1 ? f_step1 : f_step2, s_cap = (float)capacity;
 
-        if (i > 0 && MATE2_COPYOUT == 0) {   // the previous environment's bulk copy must have read the staged block
-            if (S::BULK) { if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-            __syncwarp();
-        }
         if constexpr (FOLD) {
             if (fast) {
                 // one entity kind at a time (values -> wrappers -> staged rows): fewer live registers than the plain path
@@ -1061,51 +1088,11 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
             __syncwarp();
         }
         // ---- staged rows -> HBM
-        static_assert(!(S::BULK && S::CAM_SKEW != 0), "the 16-byte copy of the whole block expects dense camera rows");
-        if constexpr (F16) {
-            // float16 rows: the lanes read the staged fp32 values, round them in pairs (__float22half2_rn, nearest even)
-            // and store each team's part with the widest store its size allows -- 16, 8, 4 or 2 bytes (part i starts at a
-            // multiple of gcd(16, part bytes) of the 16-byte aligned buffers); camera rows staged `skew` floats apart
-            __syncwarp();
-            auto copy_part_f16 = [&](__half* dst, const float* src, auto n_c, auto row_c, auto skew_c) {
-                constexpr int n = decltype(n_c)::value, row = decltype(row_c)::value, skew = decltype(skew_c)::value;
-                constexpr int W = n % 8 == 0 ? 8 : (n % 4 == 0 ? 4 : (n % 2 == 0 ? 2 : 1));   // values per store
-                static_assert(skew == 0 || (row % W == 0 && skew % 4 == 0), "a store must not straddle two skewed rows");
-                auto at = [](const int f) { return skew ? f + (f / row) * skew : f; };       // staged index of value f
-#pragma unroll
-                for (int it = 0; it < (n / W + 31) / 32; ++it) {
-                    const int k = it * 32 + lane;
-                    if (k < n / W) {
-                        if constexpr (W == 8) {
-                            // lanes 4-7 of every quarter-warp read their two 16-byte halves in the other order: each of the
-                            // two loads then covers eight distinct 16-byte bank groups per quarter-warp
-                            const int sw = (lane >> 2) & 1;
-                            const float4 a = *reinterpret_cast<const float4*>(src + at(8 * k + 4 * sw));
-                            const float4 b = *reinterpret_cast<const float4*>(src + at(8 * k + 4 - 4 * sw));
-                            const float4 lo = sw ? b : a, hi = sw ? a : b;
-                            __stcs(reinterpret_cast<uint4*>(dst) + k, make_uint4(half2_bits(lo.x, lo.y), half2_bits(lo.z, lo.w),
-                                                                                 half2_bits(hi.x, hi.y), half2_bits(hi.z, hi.w)));
-                        } else if constexpr (W == 4) {
-                            const float4 a = *reinterpret_cast<const float4*>(src + at(4 * k));
-                            __stcs(reinterpret_cast<uint2*>(dst) + k, make_uint2(half2_bits(a.x, a.y), half2_bits(a.z, a.w)));
-                        } else if constexpr (W == 2) {
-                            const float2 a = *reinterpret_cast<const float2*>(src + at(2 * k));
-                            __stcs(reinterpret_cast<unsigned int*>(dst) + k, half2_bits(a.x, a.y));
-                        } else {
-                            __stcs(reinterpret_cast<unsigned short*>(dst) + k, __half_as_ushort(__float2half_rn(src[at(k)])));
-                        }
-                    }
-                }
-            };
-            if (NC > 0) copy_part_f16(cam_obs0 + (size_t)i * S::CAM_ROW, stage, std::integral_constant<int, S::CAM_ROW>{},
-                                      std::integral_constant<int, (DC > 0 ? DC : 1)>{}, std::integral_constant<int, DCS - DC>{});
-            copy_part_f16(tgt_obs0 + (size_t)i * S::TGT_ROW, stage + S::STAGE_CAM, std::integral_constant<int, S::TGT_ROW>{},
-                          std::integral_constant<int, 1>{}, std::integral_constant<int, 0>{});
-            __syncwarp();
-        } else if (S::BULK && MATE2_COPYOUT == 1) {
-            // plain 16-byte copies: every warp store covers 512 contiguous bytes; unlike the bulk copy there
-            // is nothing to wait for before the block is reused (MATE2_COPYOUT, see DESIGN.md)
-            __syncwarp();
+        static_assert(!(S::DENSE16 && S::CAM_SKEW != 0), "the 16-byte copy of the whole block expects dense camera rows");
+        __syncwarp();
+        if constexpr (!F16 && S::DENSE16) {
+            // plain 16-byte copies of the whole block: every warp store covers 512 contiguous bytes; unlike a bulk copy
+            // there is nothing to wait for before the block is reused (see DESIGN.md)
             const float4* src4 = reinterpret_cast<const float4*>(stage);
             float4* cam4 = reinterpret_cast<float4*>(cam_obs0 + (size_t)i * S::CAM_ROW);
             float4* tgt4 = reinterpret_cast<float4*>(tgt_obs0 + (size_t)i * S::TGT_ROW) - S::CAM_ROW / 4;
@@ -1116,59 +1103,15 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
                 if (it * 32 + 32 <= NZ || k < NZ) {
                     const float4 x = src4[k];
                     float4* dst = (k < S::CAM_ROW / 4 ? cam4 : tgt4) + k;
-                    if (MATE2_STREAMING == 1) __stcs(dst, x); else if (MATE2_STREAMING == 2) __stcg(dst, x); else if (MATE2_STREAMING == 3) __stwt(dst, x); else *dst = x;
+                    __stcs(dst, x);
                 }
-            }
-            __syncwarp();
-        } else if (S::BULK) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) {
-                if (NC > 0) {
-                    const uint32_t src = (uint32_t)__cvta_generic_to_shared(stage);
-                    float* dst = cam_obs0 + (size_t)i * S::CAM_ROW;
-                    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                                 :: "l"(dst), "r"(src), "r"((uint32_t)(S::CAM_ROW * 4)) : "memory");
-                }
-                const uint32_t src = (uint32_t)__cvta_generic_to_shared(stage + S::STAGE_CAM);
-                float* dst = tgt_obs0 + (size_t)i * S::TGT_ROW;
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                             :: "l"(dst), "r"(src), "r"((uint32_t)(S::TGT_ROW * 4)) : "memory");
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             }
         } else {
-            // an environment's rows of one team are not a multiple of 16 bytes (MATE-4v2-9: 2 x 101 floats): each team's part
-            // leaves with the widest store its size allows (the caller's buffers are 16-byte aligned, so part i starts at
-            // a multiple of gcd(16, part bytes))
-            __syncwarp();
-            auto copy_part = [&](float* dst, const float* src, auto nfloats_c, auto row4_c, auto skew4_c) {
-                constexpr int n = decltype(nfloats_c)::value;
-                constexpr int row4 = decltype(row4_c)::value, skew4 = decltype(skew4_c)::value;   // staged rows `skew4` chunks apart
-                if constexpr (n % 4 == 0) {
-#pragma unroll
-                    for (int it = 0; it < (n / 4 + 31) / 32; ++it) {
-                        const int k = it * 32 + lane;
-                        if (k < n / 4) __stcs(reinterpret_cast<float4*>(dst) + k, reinterpret_cast<const float4*>(src)[skew4 ? k + (k / row4) * skew4 : k]);
-                    }
-                } else if constexpr (n % 2 == 0) {
-#pragma unroll
-                    for (int it = 0; it < (n / 2 + 31) / 32; ++it) {
-                        const int k = it * 32 + lane;
-                        if (k < n / 2) __stcs(reinterpret_cast<float2*>(dst) + k, reinterpret_cast<const float2*>(src)[k]);
-                    }
-                } else {
-                    for (int k = lane; k < n; k += 32) dst[k] = src[k];
-                }
-            };
-            static_assert(S::CAM_SKEW == 0 || DC % 4 == 0, "skewed camera rows are copied in 16-byte chunks");
-            if (NC > 0) copy_part(cam_obs0 + (size_t)i * S::CAM_ROW, stage, std::integral_constant<int, S::CAM_ROW>{},
-                                  std::integral_constant<int, (DC / 4 > 0 ? DC / 4 : 1)>{}, std::integral_constant<int, (DCS - DC) / 4>{});
-            copy_part(tgt_obs0 + (size_t)i * S::TGT_ROW, stage + S::STAGE_CAM, std::integral_constant<int, S::TGT_ROW>{},
-                      std::integral_constant<int, 1>{}, std::integral_constant<int, 0>{});
-            __syncwarp();
+            store_team_rows<OutT, S::CAM_ROW, DC, DCS - DC>(cam_obs0 + (size_t)i * S::CAM_ROW, stage);
+            store_team_rows<OutT, S::TGT_ROW, DT, 0>(tgt_obs0 + (size_t)i * S::TGT_ROW, stage + S::STAGE_CAM);
         }
+        __syncwarp();
     }
-    if (S::BULK && MATE2_COPYOUT == 0 && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
 }
 
 // Camera.sight_range_at (entities.py:507-511) for a list of (environment, camera, bearing) queries: the same
@@ -1195,7 +1138,7 @@ __global__ void fov_range_kernel(const Params p, const int32_t* __restrict__ env
 // The fused kernel
 // =============================================================================================
 template <int NC, int NT, int NO>
-__global__ void __launch_bounds__(Shape2<NC, NT, NO>::WARPS * 32, MATE2_MIN_CTAS)
+__global__ void __launch_bounds__(Shape2<NC, NT, NO>::WARPS * 32, kStepMinCtas)
 mate_step_kernel2(const __grid_constant__ Params p) {
     using S = Shape2<NC, NT, NO>;
     static_assert(NC <= 8 && NT <= 8 && NO <= 32, "mask layout: 8 cameras, 8 targets, 32 obstacles");
@@ -1248,8 +1191,7 @@ mate_step_kernel2(const __grid_constant__ Params p) {
         if (!__any_sync(FULL, need)) return;
     }
 
-    if (MATE2_PF_OBS == 2 && NO > 0 && mode == MODE_STEP) prefetch_discs64<NO>(p, er);
-    if (MATE2_PF_CARGO && mode == MODE_STEP) {   // _assign_goals reads them ~50 us from now, when every other warp is storing rows
+    if (mode == MODE_STEP) {   // cargo tables -> L2: _assign_goals reads them ~50 us from now, when every other warp is storing rows
         asm volatile("prefetch.global.L2 [%0];" :: "l"(p.cargo + er));
         asm volatile("prefetch.global.L2 [%0];" :: "l"(p.cargo + bp + er));
     }
@@ -1324,7 +1266,7 @@ mate_step_kernel2(const __grid_constant__ Params p) {
             }
         }
         if (!env_ok) slow = 0u;
-        if (MATE2_PF_OBS == 1 && NO > 0 && slow != 0) prefetch_discs64<NO>(p, er);
+        if (NO > 0 && slow != 0) prefetch_discs64<NO>(p, er);
         double ntx_ = p.tgt_x[er], nty_ = p.tgt_y[er];
         uint32_t npk_ = p.tgt_pack[er];
         float2 nta_ = make_float2(0.f, 0.f);
@@ -1544,7 +1486,7 @@ mate_step_kernel2(const __grid_constant__ Params p) {
             // With 8 cameras the fully unrolled loop nest (8 x 16 inlined range + sector tests, 50 KB of code) does not fit the
             // 32 KB instruction cache and a fifth of the warps' stalls are instruction fetches: the loop over the observing
             // camera stays rolled there (its own entries come from shared memory, its camera -> camera bits go through `cc_bits`)
-            constexpr bool ROLL_C = NC >= MATE2_ROLL_C;
+            constexpr bool ROLL_C = NC >= kRollCamerasFrom;
             unsigned long long cc_bits = 0ull;
 #pragma unroll (ROLL_C ? 1 : (NC > 0 ? NC : 1))
             for (int c = 0; c < NC; ++c) {
@@ -1640,7 +1582,7 @@ mate_step_kernel2(const __grid_constant__ Params p) {
                                 const int fast = occlusion_fast<NO>(p.obs_f4 + envr, bp, cx, cy, v[S::V_T + 3 * t] - cx, v[S::V_T + 3 * t + 1] - cy, (float)p.cam_rmax);
                                 sees = fast == 1;
                                 need_exact = fast == 2;
-                                if (MATE2_PF_OBS == 1 && need_exact) prefetch_discs64<NO>(p, envr);
+                                if (need_exact) prefetch_discs64<NO>(p, envr);
                             }
                         }
                         if (sees) atomicOr(&mk[src * S::MSTRIDE + c * MW], bit_tgt(t));
