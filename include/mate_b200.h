@@ -375,6 +375,33 @@ int mate_b200_greedy_camera_actions(MateSim* sim, double* memory, const uint8_t*
                                     uint64_t seed, uint64_t serial, const MateCameraAgentReplay* replay, float* cam_act,
                                     void* stream);
 
+/* The reference's communication wrappers (RestrictedCommunicationRange, RandomMessageDropout, NoCommunication,
+ * mate/wrappers/message_filter.py) applied to the messages the batched greedy teams exchange inside
+ * mate_b200_greedy_target_actions / _camera_actions (DESIGN.md section 7h).  A message is one routed copy (sender,
+ * recipient) of a team: a target's broadcast of its non-empty warehouse set is one copy per teammate, its own
+ * included; a camera sends at most one message (state bit and target byte) to each other camera per call.  A
+ * message is delivered iff
+ *   - the Euclidean distance of sender and recipient, taken in fp64 without fused multiply-add from the state the
+ *     agents act on, is <= range_limit[team], and
+ *   - its dropout draw keeps it: a 32-bit Philox word keyed on (the handle's seed, see mate_b200_seed, the global
+ *     environment index) with counter (the call's serial, team, sender, recipient) below
+ *     floor(keep_probability[team] * 2^32).  Several dropout wrappers compose into the product of their keep
+ *     probabilities: equal in distribution to the reference, not draw for draw.
+ * A dropped message changes only what the recipient receives; the sender's communication delay is drawn as before.
+ * Every call also writes, when the pointers are given, the team's delivered set (delivered[team][b], bit 8 s + r:
+ * s's message reached r) and adds it to total_edges[team] [B, N, N] (sender-major, int32); an environment's totals
+ * restart from this call's set when its agents are reset (reset_mask).  Edges are counted with or without a
+ * restriction.  The handle copies the struct; NULL = deliver everything, count nothing (the default).  MATE_EINVAL,
+ * with the handle unchanged, for a range_limit that is negative or NaN, a keep_probability outside [0, 1], misaligned
+ * pointers, or a restriction or edge pointer for a team of more than 8 agents. */
+typedef struct MateMessageFilter {
+    double range_limit[2];         /* per team, 0 = cameras, 1 = targets; INFINITY = unrestricted                     */
+    double keep_probability[2];    /* per team; 1 = no dropout, 0 = no communication                                  */
+    uint64_t* delivered[2];        /* dev [B]: bit 8 s + r = s's message reached r in the team's last call; nullable   */
+    int32_t* total_edges[2];       /* dev [B, N, N]: delivered since the environment's agents were reset; nullable    */
+} MateMessageFilter;
+int mate_b200_set_message_filter(MateSim* sim, const MateMessageFilter* filter);
+
 /* DiscreteCamera / DiscreteTarget.action (mate/wrappers/discrete_action_spaces.py:98-117, 204-228): grid
  * indices (dev int64 [count]) -> continuous actions (dev float32 [count][2]) through the wrapper's table
  * (dev float32 [table_size][2]). */

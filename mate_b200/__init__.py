@@ -67,7 +67,8 @@ del _nc, _nt, _no
 
 _WRAPPERS = ('EnhancedObservation', 'SharedFieldOfView', 'RelativeCoordinates', 'RescaledObservation',
              'DiscreteCamera', 'DiscreteTarget', 'RepeatedRewardIndividualDone', 'MoreTrainingInformation',
-             'AuxiliaryCameraRewards', 'AuxiliaryTargetRewards', 'MultiCamera', 'MultiTarget')
+             'AuxiliaryCameraRewards', 'AuxiliaryTargetRewards', 'MultiCamera', 'MultiTarget',
+             'RestrictedCommunicationRange', 'RandomMessageDropout', 'NoCommunication')
 _AGENTS = ('GreedyTargetAgent', 'GreedyCameraAgent', 'TargetAgentBase', 'CameraAgentBase')
 
 

@@ -113,6 +113,11 @@ class MateCameraAgentReplay(ctypes.Structure):
 AGENT_MEMORY = 6   # MATE_AGENT_MEMORY
 
 
+class MateMessageFilter(ctypes.Structure):
+    _fields_ = [('range_limit', ctypes.c_double * 2), ('keep_probability', ctypes.c_double * 2),
+                ('delivered', ctypes.c_void_p * 2), ('total_edges', ctypes.c_void_p * 2)]
+
+
 class MateReplay(ctypes.Structure):
     _fields_ = [('transmit', c_uint8_p), ('goal_choice', c_int8_p)]
 
@@ -222,8 +227,9 @@ def load_library():
     lib.mate_b200_greedy_camera_actions.argtypes = [void_p, void_p, void_p, void_p, ctypes.c_uint64, ctypes.c_uint64,
                                                     ctypes.POINTER(MateCameraAgentReplay), void_p, void_p]
     lib.mate_b200_soft_coverage.argtypes = [void_p, void_p, void_p, void_p, void_p]
+    lib.mate_b200_set_message_filter.argtypes = [void_p, ctypes.POINTER(MateMessageFilter)]
     for name in ('create', 'destroy', 'obs_dims', 'set_observation_format', 'reset', 'seed', 'step', 'observe', 'step_host',
-                 'get_state', 'set_state', 'snapshot_bytes', 'save_state', 'load_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions'):
+                 'get_state', 'set_state', 'snapshot_bytes', 'save_state', 'load_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions', 'set_message_filter'):
         getattr(lib, 'mate_b200_' + name).restype = ctypes.c_int
     _LIB = lib
     return lib
@@ -236,6 +242,7 @@ EXPORTED_SYMBOLS = [
     'mate_b200_load_state',
     'mate_b200_episode_stats', 'mate_b200_launch_count', 'mate_b200_host_leg_info', 'mate_b200_transform_observations', 'mate_b200_set_observation_ops',
     'mate_b200_decode_actions', 'mate_b200_auxiliary_terms', 'mate_b200_fov_range', 'mate_b200_soft_coverage', 'mate_b200_greedy_target_actions', 'mate_b200_greedy_camera_actions',
+    'mate_b200_set_message_filter',
 ]
 
 # observation wrapper codes (include/mate_b200.h)

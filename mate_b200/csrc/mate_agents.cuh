@@ -4,7 +4,8 @@
 // (mate/wrappers/single_team.py:79-92, 261-279: observe -> communicate -> act), for all targets of all
 // environments in one launch.  One thread = one environment: the team's message exchange (broadcast of the
 // remembered non-empty warehouses, greedy.py:338-365, routed to every teammate, environment.py:1249-1269) is an
-// AND over at most 8 four-bit sets and stays in registers.  The agents read their private state from the
+// AND over at most 8 four-bit sets and stays in registers; with communication wrappers registered (DESIGN.md section 7h)
+// it is one AND per recipient over the copies that reached it.  The agents read their private state from the
 // simulator's state arrays (not from the observation tensors, which observation wrappers may have transformed).
 #pragma once
 
@@ -13,7 +14,52 @@
 namespace mate {
 
 constexpr uint32_t STREAM_AGENT_BINOMIAL = 16, STREAM_AGENT_SAMPLE = 17, STREAM_AGENT_CHOICE = 18, STREAM_AGENT_RESET = 19, STREAM_AGENT_DELAY = 20;
+constexpr uint32_t STREAM_AGENT_COMM = 21;
 constexpr int kAgentMemory = 6;   // per target: goal, non-empty warehouse set, previous x, y, previous noise x, y; stored FIELD-MAJOR [6][Nt][B]
+
+// The communication wrappers of one team as its agent kernel applies them (mate_b200_set_message_filter, DESIGN.md
+// section 7h).  A message is delivered iff it passes the range rule and the dropout draw.
+struct CommFilter {
+    double range_limit;            // RestrictedCommunicationRange; +inf = unrestricted
+    unsigned long long keep;       // kept iff its 32-bit draw < keep: 1 << 32 = no dropout, 0 = NoCommunication
+    unsigned long long seed;       // the handle's Philox key (mate_b200_seed), not the agents' seed
+    uint64_t* delivered;           // [B] nullable: bit 8 s + r = the message of s reached r in this call
+    int32_t* totals;               // [B, N, N] nullable: delivered since the environment's agents were reset
+    int pairwise;                  // greedy targets: decide per (sender, recipient) (N <= 8); 0 = every copy arrives
+};
+
+// RestrictedCommunicationRange: the distance in fp64 without fused multiply-add, so that NumPy decides it identically
+__device__ inline bool comm_in_range(double sx, double sy, double rx, double ry, double limit) {
+    if (isinf(limit)) return true;
+    const double dx = __dsub_rn(sx, rx), dy = __dsub_rn(sy, ry);
+    return __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy))) <= limit;
+}
+
+// the Philox draw of rng_words, out of line on its own (mate_common.cuh, philox_rounds)
+__device__ __noinline__ uint4 philox_comm(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
+    return philox_rounds(c0, c1, c2, c3, k0, k1);
+}
+
+// RandomMessageDropout: word r % 4 of the Philox call keyed on (handle seed, global environment, 'COMM') with counter
+// (call serial, team, sender, r / 4); the draw does not depend on the batch split or on the lane that takes it
+__device__ inline bool comm_kept(const CommFilter& f, uint32_t env, uint32_t serial, uint32_t team, int s, int r) {
+    if (f.keep > 0xFFFFFFFFull) return true;
+    if (f.keep == 0ull) return false;
+    const uint4 w = philox_comm(serial, (STREAM_AGENT_COMM << 16) | (team << 8) | ((uint32_t)s << 2) | ((uint32_t)r >> 2),
+                                env, 0x434F4D4Du /* 'COMM' */, (uint32_t)f.seed, (uint32_t)(f.seed >> 32));
+    const uint32_t x = (r & 3) == 0 ? w.x : (r & 3) == 1 ? w.y : (r & 3) == 2 ? w.z : w.w;
+    return x < f.keep;
+}
+
+// one sender's row of the per-episode totals [N] (sender-major): restarted at the agents' reset, then this call's row added
+__device__ inline void add_edge_row(int32_t* total, int n, uint32_t row, bool reset) {
+    if (!reset && row == 0u) return;
+    for (int r = 0; r < n; ++r) {
+        const int bit = (int)((row >> r) & 1u);
+        if (reset) total[r] = bit;
+        else if (bit) total[r] += 1;
+    }
+}
 
 // one agent's view of a field-major table: entry k of the agent is `stride` doubles after entry k - 1
 struct Field {
@@ -25,7 +71,7 @@ struct Field {
 
 __global__ void greedy_target_kernel(const Params p, const int nt, double* __restrict__ memory, const uint8_t* __restrict__ reset_mask,
                                      const double noise_scale, const unsigned long long seed, const unsigned long long serial,
-                                     const MateAgentReplay replay, float* __restrict__ tgt_act) {
+                                     const MateAgentReplay replay, const CommFilter comm, float* __restrict__ tgt_act) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= p.num_envs) return;
     const size_t bp = p.bpad;
@@ -36,6 +82,7 @@ __global__ void greedy_target_kernel(const Params p, const int nt, double* __res
     const uint32_t draw = (uint32_t)serial * 16u;
     // observe -> process_messages (greedy.py:330-336), and the sets that are broadcast
     uint32_t sent_and = 15u;
+    uint32_t senders = 0u, sent_sets = 0u;   // pairwise: bit s / bits 4 s .. 4 s + 3 = target s broadcasts this set
     for (int t = 0; t < nt; ++t) {
         const Field m{memory + (size_t)t * p.num_envs + e, (size_t)nt * p.num_envs};
         const uint32_t tp = p.tgt_pack[(size_t)t * bp + e];
@@ -57,8 +104,10 @@ __global__ void greedy_target_kernel(const Params p, const int nt, double* __res
             non_empty &= ~seen;
             m[1] = (double)non_empty;
             sent_and &= non_empty;
+            if (comm.pairwise) { senders |= 1u << t; sent_sets |= non_empty << (4 * t); }
         }
     }
+    uint64_t delivered = 0ull;
     // receive_responses (greedy.py:355-365) + act (greedy.py:289-328)
     for (int t = 0; t < nt; ++t) {
         const Field m{memory + (size_t)t * p.num_envs + e, (size_t)nt * p.num_envs};
@@ -66,7 +115,18 @@ __global__ void greedy_target_kernel(const Params p, const int nt, double* __res
         const double x = p.tgt_x[(size_t)t * bp + e], y = p.tgt_y[(size_t)t * bp + e];
         const double step_size = p.tgt_step_size / (double)tp_capacity(tp);
         const bool state_has_goal = tp_goal(tp) >= 0 && tp_weight(tp) > 0;
-        const uint32_t non_empty = (uint32_t)m[1] & sent_and;
+        uint32_t received = sent_and;
+        if (comm.pairwise) {   // recipient t ANDs the sets of the senders whose copy reached it (its own copy changes nothing)
+            received = 15u;
+            for (uint32_t rest = senders; rest != 0u; rest &= rest - 1u) {
+                const int s = __ffs(rest) - 1;
+                if (!comm_in_range(p.tgt_x[(size_t)s * bp + e], p.tgt_y[(size_t)s * bp + e], x, y, comm.range_limit) ||
+                    !comm_kept(comm, key.env, (uint32_t)serial, 1u, s, t)) continue;
+                received &= sent_sets >> (4 * s);
+                delivered |= 1ull << (8 * s + t);
+            }
+        }
+        const uint32_t non_empty = (uint32_t)m[1] & received;
         int goal = (int)m[0];
         if (state_has_goal) goal = tp_goal(tp);
         if (goal < 0 || (!state_has_goal && !((non_empty >> goal) & 1u))) {
@@ -107,6 +167,9 @@ __global__ void greedy_target_kernel(const Params p, const int nt, double* __res
         reinterpret_cast<float2*>(tgt_act)[(size_t)e * nt + t] = make_float2((float)ax, (float)ay);
         m[0] = (double)goal; m[1] = (double)non_empty; m[2] = x; m[3] = y; m[4] = nx; m[5] = ny;
     }
+    if (comm.delivered) comm.delivered[e] = delivered;
+    if (comm.totals)
+        for (int s = 0; s < nt; ++s) add_edge_row(comm.totals + ((size_t)e * nt + s) * nt, nt, (uint32_t)(delivered >> (8 * s)) & 0xFFu, reset);
 }
 
 // =============================================================================================
@@ -134,7 +197,7 @@ __global__ void __launch_bounds__(kCameraAgentThreads)
 greedy_camera_kernel(const Params p, const int nc, const int nt, double* __restrict__ memory,
                      const uint8_t* __restrict__ tracked, const uint8_t* __restrict__ reset_mask,
                      const unsigned long long seed, const unsigned long long serial,
-                     const MateCameraAgentReplay replay, float* __restrict__ cam_act) {
+                     const MateCameraAgentReplay replay, const CommFilter comm, float* __restrict__ cam_act) {
     constexpr int MAXN = 8;
     constexpr uint32_t FULL = 0xffffffffu;
     constexpr double kMemoryPeriod = 25.0, kRangeFactor = 1.1;   // greedy.py:22, 32
@@ -169,6 +232,7 @@ greedy_camera_kernel(const Params p, const int nc, const int nt, double* __restr
     // ---- observe -> process_messages (greedy.py:104-115); send_responses (greedy.py:156-194)
     uint32_t msg_state = 0;                 // bit k: my state goes to camera k
     unsigned long long msg_targets = 0ull;  // byte k: the tracked targets I report to camera k
+    uint32_t delivered_row = 0;             // bit k: my message reached camera k
     {
         uint32_t seen = 0;
         for (int t = 0; t < nt; ++t) seen |= (uint32_t)(tracked[((size_t)e * nc + c) * nt + t] != 0) << t;
@@ -196,6 +260,17 @@ greedy_camera_kernel(const Params p, const int nc, const int nt, double* __restr
         const uint32_t neighbours = (uint32_t)m[6 * nt + 2 + nc];
         const bool has_state = m[6 * nt + 3 + nc] != 0.0;
         for (int k = 0; k < nc; ++k) delay[k] = fmax(delay[k] - 1.0, 0.0);
+        // bit k: a message to camera k would pass the communication wrappers; decided in a pass of its own (uniform
+        // branch) so that the send loop below keeps the registers it had without wrappers
+        uint32_t pass = 0xFFu;
+        if (!isinf(comm.range_limit) || comm.keep <= 0xFFFFFFFFull) {
+            pass = 0u;
+            for (int k = 0; k < nc; ++k) {
+                const double kx = __shfl_sync(active, my_x, lane0 + k), ky = __shfl_sync(active, my_y, lane0 + k);
+                if (comm_in_range(my_x, my_y, kx, ky, comm.range_limit) && comm_kept(comm, key.env, (uint32_t)serial, 0u, c, k))
+                    pass |= 1u << k;
+            }
+        }
         for (int k = 0; k < nc; ++k) {      // every lane takes part in the shuffles; the recipient's location comes from its lane
             const double kx = __shfl_sync(active, my_x, lane0 + k), ky = __shfl_sync(active, my_y, lane0 + k);
             if (!(has_state || seen != 0u) || k == c || delay[k] > 0.0) continue;
@@ -208,15 +283,25 @@ greedy_camera_kernel(const Params p, const int nc, const int nt, double* __restr
                 }
             }
             if (has_state || targets != 0u) {
-                msg_state |= has_state ? (1u << k) : 0u;
-                msg_targets |= (unsigned long long)targets << (8 * k);
                 int d;   // np_random.randint(memory_period // 4, 2 * memory_period)
                 if (replay.delay) d = replay.delay[((size_t)e * nc + c) * nc + k];
                 else d = 6 + (int)rng_below(key, STREAM_AGENT_DELAY, draw + (uint32_t)(c * MAXN + k), 44u);
                 delay[k] = (double)d;
+                // the sender does not know about the communication wrappers: only the recipient misses a dropped message
+                if (!((pass >> k) & 1u)) continue;
+                msg_state |= has_state ? (1u << k) : 0u;
+                msg_targets |= (unsigned long long)targets << (8 * k);
+                delivered_row |= 1u << k;
             }
         }
         if (has_state || seen != 0u) m[6 * nt + 3 + nc] = 0.0;
+    }
+    // each lane adds its own row of the totals; the environment's bit matrix is the OR of its lanes' rows
+    if (comm.totals) add_edge_row(comm.totals + ((size_t)e * nc + c) * nc, nc, delivered_row, reset);
+    if (comm.delivered) {
+        uint64_t bits = (uint64_t)delivered_row << (8 * c);
+        for (int o = 1; o < nc; o <<= 1) bits |= __shfl_xor_sync(active, bits, o);   // the lanes of an environment: an aligned group of nc
+        if (c == 0) comm.delivered[e] = bits;
     }
     // ---- receive_responses (greedy.py:196-232) + act (greedy.py:68-102)
     {

@@ -199,6 +199,7 @@ struct MateSim {
     int refill_period = 512;
     int tile_envs = 32;       // environments per warp tile (Params::tile_envs), chosen from the batch size at creation
     int obs_format = MATE_OBS_FORMAT_F32;   // element type of the observation rows (mate_b200_set_observation_format)
+    MateMessageFilter message_filter = {{INFINITY, INFINITY}, {1.0, 1.0}, {nullptr, nullptr}, {nullptr, nullptr}};   // deliver everything
     bool rows_written = false;              // a reset / step / step_host / observe has run: the format is fixed
     long long steps_since_refill = 0;
     // host-path (step_host) resources
@@ -602,6 +603,38 @@ extern "C" int mate_b200_auxiliary_terms(MateSim* sim, const MateStepAux* aux, c
     return check_launch("auxiliary terms");
 }
 
+// The registered communication wrappers of team 0 (cameras) or 1 (targets) as the agent kernels take them.
+static CommFilter comm_filter(const MateSim* sim, int team) {
+    const MateMessageFilter& f = sim->message_filter;
+    CommFilter c{};
+    c.range_limit = f.range_limit[team];
+    // keep / 2^32 is the keep probability rounded down to a multiple of 2^-32; 1 gives 2^32 (every draw passes), 0 gives 0
+    c.keep = (unsigned long long)floor(f.keep_probability[team] * 4294967296.0);
+    c.seed = sim->seed;
+    c.delivered = f.delivered[team];
+    c.totals = f.total_edges[team];
+    c.pairwise = (!isinf(c.range_limit) || c.keep <= 0xFFFFFFFFull || c.delivered || c.totals) ? 1 : 0;
+    return c;
+}
+
+extern "C" int mate_b200_set_message_filter(MateSim* sim, const MateMessageFilter* filter) {
+    if (!sim) return fail(MATE_EINVAL, "null handle");
+    MateMessageFilter f = {{INFINITY, INFINITY}, {1.0, 1.0}, {nullptr, nullptr}, {nullptr, nullptr}};
+    if (filter) f = *filter;
+    const int team_size[2] = {sim->cfg.num_cameras, sim->cfg.num_targets};
+    for (int t = 0; t < 2; ++t) {
+        if (!(f.range_limit[t] >= 0.0)) return fail(MATE_EINVAL, "range_limit must be >= 0 or +inf");
+        if (!(f.keep_probability[t] >= 0.0 && f.keep_probability[t] <= 1.0)) return fail(MATE_EINVAL, "keep_probability must lie in [0, 1]");
+        if ((uintptr_t)f.delivered[t] & 7) return fail(MATE_EINVAL, "delivered must be 8-byte aligned");
+        if ((uintptr_t)f.total_edges[t] & 3) return fail(MATE_EINVAL, "total_edges must be 4-byte aligned");
+        const bool used = !isinf(f.range_limit[t]) || f.keep_probability[t] < 1.0 || f.delivered[t] || f.total_edges[t];
+        if (used && team_size[t] > 8)
+            return fail(MATE_EINVAL, "message filters and communication edges cover teams of at most 8 agents (bit 8 s + r)");
+    }
+    sim->message_filter = f;
+    return MATE_OK;
+}
+
 extern "C" int mate_b200_greedy_target_actions(MateSim* sim, double* memory, const uint8_t* reset_mask, double noise_scale,
                                                uint64_t seed, uint64_t serial, const MateAgentReplay* replay, float* tgt_act,
                                                void* stream) {
@@ -612,7 +645,7 @@ extern "C" int mate_b200_greedy_target_actions(MateSim* sim, double* memory, con
     if (replay) r = *replay;
     const int threads = 128;
     greedy_target_kernel<<<(sim->num_envs + threads - 1) / threads, threads, 0, (cudaStream_t)stream>>>(
-        sim->base, sim->cfg.num_targets, memory, reset_mask, noise_scale, seed, serial, r, tgt_act);
+        sim->base, sim->cfg.num_targets, memory, reset_mask, noise_scale, seed, serial, r, comm_filter(sim, 1), tgt_act);
     sim->launches += 1;
     return check_launch("greedy target");
 }
@@ -631,7 +664,7 @@ extern "C" int mate_b200_greedy_camera_actions(MateSim* sim, double* memory, con
     if (32 % nc != 0) return fail(MATE_EINVAL, "the batched GreedyCameraAgent needs a number of cameras that divides 32");
     const long long agents = (long long)sim->num_envs * nc;
     greedy_camera_kernel<<<(unsigned)((agents + kCameraAgentThreads - 1) / kCameraAgentThreads), kCameraAgentThreads, 0, (cudaStream_t)stream>>>(
-        sim->base, nc, nt, memory, tracked, reset_mask, seed, serial, r, cam_act);
+        sim->base, nc, nt, memory, tracked, reset_mask, seed, serial, r, comm_filter(sim, 0), cam_act);
     sim->launches += 1;
     return check_launch("greedy camera");
 }

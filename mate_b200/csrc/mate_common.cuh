@@ -134,7 +134,9 @@ __device__ __forceinline__ void sincos_deg(double deg, double* s, double* c) { s
 // ---- Philox4x32-10, same draw scheme as oracle/mate_oracle.c ------------------------------
 struct RngKey { unsigned long long seed; uint32_t env; uint32_t episode; };
 
-__device__ __noinline__ uint4 philox(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
+// the rounds, for a second out-of-line copy (philox_comm, mate_agents.cuh): ptxas allocates registers across every caller
+// of an out-of-line function, so new callers of `philox` would change the step kernel's code
+__device__ __forceinline__ uint4 philox_rounds(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
 #pragma unroll
     for (int r = 0; r < 10; ++r) {
         uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
@@ -144,6 +146,9 @@ __device__ __noinline__ uint4 philox(uint32_t c0, uint32_t c1, uint32_t c2, uint
         k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
     }
     return make_uint4(c0, c1, c2, c3);
+}
+__device__ __noinline__ uint4 philox(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
+    return philox_rounds(c0, c1, c2, c3, k0, k1);
 }
 __device__ inline uint4 rng_words(const RngKey& k, uint32_t stream, uint32_t index) {
     return philox(index, stream, k.env, k.episode, (uint32_t)k.seed, (uint32_t)(k.seed >> 32));

@@ -135,12 +135,19 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         self.message_buffers = (self.camera_message_buffer, self.target_message_buffer)
         self.camera_message_queue, self.target_message_queue = defaultdict(deque), defaultdict(deque)
         self.message_queues = (self.camera_message_queue, self.target_message_queue)
-        self.camera_communication_edges = np.zeros((nc, nc), dtype=np.int64)
-        self.target_communication_edges = np.zeros((nt, nt), dtype=np.int64)
-        self.camera_total_communication_edges = self.camera_communication_edges.copy()
-        self.target_total_communication_edges = self.target_communication_edges.copy()
-        self.communication_edges = (self.camera_communication_edges, self.target_communication_edges)
-        self.total_communication_edges = (self.camera_total_communication_edges, self.target_total_communication_edges)
+        # communication edges: in the single-environment mode the host Message traffic (NumPy, like the reference); in
+        # batched mode the traffic of the batched greedy teams, written by their kernels (DESIGN.md section 7h):
+        # delivered sets of the team's last call (int64 [B], bit 8 s + r) and per-episode totals (int32 [B, N, N])
+        if self.batched:
+            self._delivered_bits = tuple(torch.zeros(self.num_envs, dtype=torch.int64, device=self.device) for _ in range(2))
+            self._total_edges = tuple(torch.zeros((self.num_envs, n, n), dtype=torch.int32, device=self.device) for n in (nc, nt))
+        else:
+            self._edges = (np.zeros((nc, nc), dtype=np.int64), np.zeros((nt, nt), dtype=np.int64))
+            self._total_edges = (np.zeros((nc, nc), dtype=np.int64), np.zeros((nt, nt), dtype=np.int64))
+        # the communication wrappers' combined rule per team (cameras, targets) for the batched greedy teams
+        self.message_rules = {'range_limit': [np.inf, np.inf], 'keep_probability': [1.0, 1.0]}
+        if self.batched:
+            self.register_message_filter()
 
     # ------------------------------------------------------------------ configuration properties
     @property
@@ -209,8 +216,12 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         self.sim.observe(aux=True)   # refresh the mask attributes for the new episode
         self._needs_reset = False
         self._state_serial += 1
-        for edges in self.communication_edges + self.total_communication_edges:   # environment.py:823-830
-            edges.fill(0)
+        if self.batched:   # environment.py:823-830
+            for edges in self._delivered_bits + self._total_edges:
+                edges.zero_()
+        else:
+            for edges in self._edges + self._total_edges:
+                edges.fill(0)
         self._clear_messages()
         return self._format_obs(cam_obs, tgt_obs)
 
@@ -275,6 +286,43 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
             edges.fill(0)
         self._clear_messages()
         return self._format_obs(cam_obs, tgt_obs), (rew[0], rew[1]), done_flag, (camera_infos, target_infos)
+
+    # ------------------------------------------------------------------ communication edges and filter
+    def register_message_filter(self):
+        """Register ``message_rules`` and, in batched mode, the edge tensors with the simulator: the batched greedy
+        teams of ``MultiCamera`` / ``MultiTarget`` apply the rules to the messages they exchange inside their kernels
+        and count what is delivered.  Teams of more than 8 agents are not counted (the bit matrix holds 8)."""
+        nc, nt = self.num_cameras, self.num_targets
+        counted = [self.batched and 0 < n <= 8 for n in (nc, nt)]
+        self.sim.set_message_filter(
+            range_limit=tuple(self.message_rules['range_limit']), keep_probability=tuple(self.message_rules['keep_probability']),
+            delivered=tuple(self._delivered_bits[t] if counted[t] else None for t in range(2)),
+            total_edges=tuple(self._total_edges[t] if counted[t] else None for t in range(2)))
+
+    @staticmethod
+    def _unpack_edges(bits, n):
+        shift = 8 * torch.arange(n, device=bits.device).view(n, 1) + torch.arange(n, device=bits.device).view(1, n)
+        return ((bits.view(-1, 1, 1) >> shift) & 1).bool()
+
+    @property
+    def communication_edges(self):
+        """Per team (cameras, targets): messages delivered since the last step.  Batched: ``[B, N, N]`` bool, the
+        delivered set of the greedy team's last call, sender-major; single environment: the reference's NumPy counts of
+        the host ``Message`` traffic."""
+        if self.batched:
+            return tuple(self._unpack_edges(bits, n) for bits, n in zip(self._delivered_bits, (self.num_cameras, self.num_targets)))
+        return self._edges
+
+    @property
+    def total_communication_edges(self):
+        """Per team: messages delivered in the episode.  Batched: ``[B, N, N]`` int32, since the environment's greedy
+        agents were last reset; single environment: NumPy, since ``reset``."""
+        return self._total_edges
+
+    camera_communication_edges = property(lambda self: self.communication_edges[0])
+    target_communication_edges = property(lambda self: self.communication_edges[1])
+    camera_total_communication_edges = property(lambda self: self._total_edges[0])
+    target_total_communication_edges = property(lambda self: self._total_edges[1])
 
     # ------------------------------------------------------------------ intra-team messages (reference-compatible mode)
     def _clear_messages(self):

@@ -220,6 +220,28 @@ class BatchedSim:
                                                                index.numel(), self._stream()))
         return out
 
+    def set_message_filter(self, range_limit=(np.inf, np.inf), keep_probability=(1.0, 1.0), delivered=(None, None),
+                           total_edges=(None, None)):
+        """Register the communication wrappers with the simulator (mate_b200_set_message_filter): per team (cameras,
+        targets) the range limit and the keep probability the batched greedy teams apply to their messages, and the
+        device tensors their kernels write the delivered sets to (int64 ``[B]``, bit ``8 s + r``) and add them to
+        (int32 ``[B, N, N]``); ``None`` = not counted.  The defaults deliver everything."""
+        tensors = []
+        for team, n in enumerate((self.nc, self.nt)):
+            for name, t, dtype, shape in (('delivered', delivered[team], torch.int64, (self.B,)),
+                                          ('total_edges', total_edges[team], torch.int32, (self.B, n, n))):
+                if t is not None and (t.device != self.device or t.dtype != dtype or tuple(t.shape) != shape or not t.is_contiguous()):
+                    raise ValueError(f'{name}[{team}] must be a contiguous {dtype} tensor of shape {shape} on {self.device}')
+                tensors.append(t)
+        f = _abi.MateMessageFilter()
+        for team in range(2):
+            f.range_limit[team] = float(range_limit[team])
+            f.keep_probability[team] = float(keep_probability[team])
+            f.delivered[team] = None if delivered[team] is None else delivered[team].data_ptr()
+            f.total_edges[team] = None if total_edges[team] is None else total_edges[team].data_ptr()
+        _check(self.lib, self.lib.mate_b200_set_message_filter(self.handle, ctypes.byref(f)))
+        self._message_tensors = tensors   # the library keeps the pointers
+
     # ------------------------------------------------------------------ API
     def seed(self, seed, env_mask=None):
         """``MultiAgentTracking.seed``: new key for the Philox streams, episode counters rewound (mate_b200_seed), so

@@ -468,13 +468,127 @@ class AuxiliaryTargetRewards(_AuxiliaryRewards):
 
 
 # ------------------------------------------------------------------------------------------------------------
+# Communication wrappers (mate/wrappers/message_filter.py and its subclasses; DESIGN.md section 7h).  Batched, the
+# only messages are those the greedy teams behind MultiCamera / MultiTarget exchange inside their kernels: each wrapper
+# merges its rule into the environment's ``message_rules`` and registers them with the simulator, in both modes.  In
+# the single-environment mode the wrappers also filter the host ``Message`` traffic in ``send_messages``.
+# ------------------------------------------------------------------------------------------------------------
+
+class _CommunicationWrapper(Wrapper):
+    """A message filter of the reference: a routed message (broadcasts are one copy per teammate, the sender's own
+    included) reaches its recipient iff every communication wrapper of the stack lets it through."""
+
+    def __init__(self, env):
+        assert not _has_wrapper(env, MultiCamera) and not _has_wrapper(env, MultiTarget), (
+            f'You should use wrapper `{type(self)}` before `MultiCamera` / `MultiTarget`: the single-team wrapper sends '
+            f'its opponents\' messages through the environment below it. Please wrap the environment with wrapper '
+            f'`{type(self)}` first. Got env = {env}.')
+        super().__init__(env)
+
+    def _merge(self, rules):
+        raise NotImplementedError
+
+    def _register(self):
+        base = self.unwrapped
+        self._merge(base.message_rules)
+        base.register_message_filter()
+
+    def _delivers(self, base, message):
+        raise NotImplementedError
+
+    def send_messages(self, messages):
+        base = self.unwrapped
+        base._messages_supported()   # pylint: disable=protected-access
+        if hasattr(messages, 'sender') and hasattr(messages, 'content'):
+            messages = (messages,)
+        self.env.send_messages([m for m in base.route_messages(list(messages)) if self._delivers(base, m)])
+
+
+def _team_of(message):
+    from mate_b200 import constants as consts   # pylint: disable=import-outside-toplevel
+
+    return consts._team_index(message.team)   # pylint: disable=protected-access
+
+
+class RestrictedCommunicationRange(_CommunicationWrapper):
+    """mate/wrappers/message_filter.py: a message is delivered iff sender and recipient are at most ``range_limit``
+    apart (both teams)."""
+
+    def __init__(self, env, range_limit):
+        assert range_limit >= 0, f'The argument `range_limit` should be non-negative. Got range_limit = {range_limit}.'
+        super().__init__(env)
+        self.range_limit = float(range_limit)
+        self._register()
+
+    def _merge(self, rules):
+        rules['range_limit'] = [min(limit, self.range_limit) for limit in rules['range_limit']]
+
+    @staticmethod
+    def within(a, b, range_limit):
+        """The kernels' test: fp64 distance without fused multiply-add, ``<=`` the limit."""
+        dx, dy = float(a[0]) - float(b[0]), float(a[1]) - float(b[1])
+        return float(np.sqrt(dx * dx + dy * dy)) <= range_limit
+
+    def _delivers(self, base, message):
+        agents = base.cameras if _team_of(message) == 0 else base.targets
+        return self.within(agents[message.sender].location, agents[message.recipient].location, self.range_limit)
+
+
+class RandomMessageDropout(_CommunicationWrapper):
+    """mate/wrappers/message_filter.py: every message is dropped independently with probability ``dropout_rate``.
+    Batched, the draws are Philox streams of the simulator (keyed on its seed and the global environment index);
+    in the single-environment mode they come from this wrapper's own ``np_random``."""
+
+    def __init__(self, env, dropout_rate):
+        assert 0.0 <= dropout_rate <= 1.0, f'The argument `dropout_rate` should be in [0, 1]. Got dropout_rate = {dropout_rate}.'
+        super().__init__(env)
+        self.dropout_rate = float(dropout_rate)
+        self.np_random = np.random.RandomState(0)
+        self._register()
+
+    def seed(self, seed=None):
+        self.np_random = np.random.RandomState(seed)
+        return self.env.seed(seed)
+
+    def _merge(self, rules):
+        rules['keep_probability'] = [keep * (1.0 - self.dropout_rate) for keep in rules['keep_probability']]
+
+    def _delivers(self, base, message):
+        return self.np_random.random_sample() >= self.dropout_rate
+
+
+class NoCommunication(_CommunicationWrapper):
+    """mate/wrappers/message_filter.py: drop every message of the named team(s)."""
+
+    def __init__(self, env, team='both'):
+        assert team in TEAMS, f'Invalid argument team {team!r}. Expect one of {TEAMS}.'
+        super().__init__(env)
+        self.team = team
+        self.no_camera_communication = team in ('camera', 'both')
+        self.no_target_communication = team in ('target', 'both')
+        self._register()
+
+    def _merge(self, rules):
+        for t, off in enumerate((self.no_camera_communication, self.no_target_communication)):
+            if off:
+                rules['keep_probability'][t] = 0.0
+
+    def _delivers(self, base, message):
+        return not (self.no_camera_communication, self.no_target_communication)[_team_of(message)]
+
+    def __str__(self):
+        return f'<{type(self).__name__}(team={self.team}){self.env}>'
+
+
+# ------------------------------------------------------------------------------------------------------------
 # SURVEY.md section 8f, N4: single-team wrapper with a batched built-in opponent.
 # ------------------------------------------------------------------------------------------------------------
 
 class _SingleTeamSnapshot:
     """``save_state`` / ``load_state`` of the single-team wrappers: besides the environment they carry the per-environment
     state of the opponent agent (its memory, gathered / scattered along the memory's environment axis with the
-    snapshot's index map) and the pending reset mask; the agent's step serial is restored on resume only."""
+    snapshot's index map), the opponent team's per-episode communication totals (batched mode) and the pending reset
+    mask; the agent's step serial is restored on resume only."""
 
     _MEMORY_AXIS = None   # environment axis of the agent's field-major memory tensor
     _TEAM = None          # index of this wrapper's team in the joint (camera, target) tuples
@@ -492,11 +606,20 @@ class _SingleTeamSnapshot:
         snapshot = self.env.save_state(envs)
         agent = self.opponent_agent
         memory, pending = agent._memory, self._pending_resets()   # pylint: disable=protected-access
+        totals = self._opponent_totals()
         if envs is not None:   # out-of-range device indices: the kernel leaves those entries unwritten, here they are clamped
             index = base.sim._index_map(envs, 'envs', None, 0, base.num_envs).long().clamp_(0, base.num_envs - 1)  # pylint: disable=protected-access
             memory, pending = memory.index_select(self._MEMORY_AXIS, index), pending.index_select(0, index)
+            totals = None if totals is None else totals.index_select(0, index)
         snapshot.extras['opponent'] = {'memory': memory.clone(), 'reset_mask': pending.clone(), 'serial': agent._serial}  # pylint: disable=protected-access
+        if totals is not None:
+            snapshot.extras['opponent']['total_edges'] = totals.clone()
         return snapshot
+
+    def _opponent_totals(self):
+        """The opponent team's per-episode communication totals ``[B, N, N]`` (batched mode), else ``None``."""
+        base = self.unwrapped
+        return base.total_communication_edges[1 - self._TEAM] if base.batched else None
 
     def load_state(self, snapshot, src=None, resume=False):
         base = self.unwrapped
@@ -505,9 +628,16 @@ class _SingleTeamSnapshot:
         agent = self.opponent_agent
         memory, pending = agent._memory, self._pending_resets()   # pylint: disable=protected-access
         saved_memory, saved_pending = saved['memory'].to(memory.device), saved['reset_mask'].to(pending.device)
+        totals, saved_totals = self._opponent_totals(), saved.get('total_edges')
+        if saved_totals is not None and totals is not None:
+            saved_totals = saved_totals.to(totals.device)
+        else:
+            totals = None
         if src is None:
             memory.copy_(saved_memory)
             pending = saved_pending.clone()
+            if totals is not None:
+                totals.copy_(saved_totals)
         else:
             index = base.sim._index_map(src, 'src', base.num_envs, -(1 << 31), snapshot.count).long()  # pylint: disable=protected-access
             keep = (index < 0) | (index >= snapshot.count)
@@ -516,6 +646,8 @@ class _SingleTeamSnapshot:
             shape[self._MEMORY_AXIS] = -1
             memory.copy_(torch.where(keep.view(shape), memory, saved_memory.index_select(self._MEMORY_AXIS, index)))
             pending = torch.where(keep, pending, saved_pending.index_select(0, index))
+            if totals is not None:
+                totals.copy_(torch.where(keep.view(-1, 1, 1), totals, saved_totals.index_select(0, index)))
         self._reset_mask = pending
         if resume:
             agent._serial = saved['serial']   # pylint: disable=protected-access
