@@ -54,7 +54,7 @@ struct KernelInfo {
     void (*launch_wrappers)(const Params&, const ObsOps&, const float*, const float*, int num_envs, cudaStream_t);
     cudaError_t (*prepare_wrappers)();
     void (*launch)(const Params&, int grid, cudaStream_t);
-    int envs_per_cta, smem_bytes, dc, dt, epw;
+    int envs_per_cta, dc, dt;
     cudaError_t (*prepare)();
     void (*launch_fov)(const Params&, const int32_t*, const int32_t*, const double*, double*, long long, cudaStream_t);
     void (*launch_soft)(const Params&, const uint8_t*, const uint8_t*, double*, float*, cudaStream_t);
@@ -166,8 +166,8 @@ static bool find_kernel(int nc, int nt, int no, KernelInfo* out) {
     if (nc == NC && nt == NT && no == NO) {                                                    \
         using S = Shape2<NC, NT, NO>;                                                          \
         *out = KernelInfo{&launch_wrappers_shape<NC, NT, NO>, &prepare_wrappers_shape<NC, NT, NO>,       \
-                          &launch_shape2<NC, NT, NO>, S::ENVS_PER_CTA, S::SMEM_BYTES, S::DC, S::DT, \
-                          32, &prepare_shape2<NC, NT, NO>, &launch_fov_shape<NC, NT, NO>,        \
+                          &launch_shape2<NC, NT, NO>, S::ENVS_PER_CTA, S::DC, S::DT,             \
+                          &prepare_shape2<NC, NT, NO>, &launch_fov_shape<NC, NT, NO>,            \
                           &launch_soft_shape<NC, NT, NO>};                                      \
         return true;                                                                           \
     }
@@ -539,32 +539,30 @@ extern "C" int mate_b200_set_observation_ops(MateSim* sim, const int32_t* ops, i
     f.fast = (num_ops > 0 && k == num_ops) ? 1 : 0;
     if (f.fast && f.rescaled) {
         CUDA_TRY(cudaSetDevice(sim->device));
-        const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets, no = sim->cfg.num_obstacles;
-        const int dc = sim->kernel.dc, dt = sim->kernel.dt;
+        const int nc = sim->cfg.num_cameras;
+        const ObsLayout L{nc, sim->cfg.num_targets, sim->cfg.num_obstacles};
+        const int dc = L.dc(), dt = L.dt();
         std::vector<float> cam((size_t)2 * std::max(dc, 1), 0.f), tgt((size_t)2 * dt, 0.f);
         if (nc) CUDA_TRY(cudaMemcpy(cam.data(), cam_affine, sizeof(float) * 2 * dc, cudaMemcpyDeviceToHost));
         CUDA_TRY(cudaMemcpy(tgt.data(), tgt_affine, sizeof(float) * 2 * dt, cudaMemcpyDeviceToHost));
         auto col = [](const std::vector<float>& t, int c) { return make_float2(t[2 * c], t[2 * c + 1]); };
         auto same = [](float2 a, float2 b) { return a.x == b.x && a.y == b.y; };
         bool uniform = true;
-        for (int j = 0; j < 13; ++j) { f.pres[j] = col(tgt, j); if (nc) uniform = uniform && same(f.pres[j], col(cam, j)); }
-        for (int j = 0; j < 14; ++j) f.tself[j] = col(tgt, 13 + j);
-        for (int j = 0; j < 9 && nc; ++j) f.cself[j] = col(cam, 13 + j);
-        const int t_tgt = 27 + 7 * nc + 4 * no, t_obs = 27 + 7 * nc, t_cam = 27, c_tgt = 22, c_obs = 22 + 5 * nt, c_cam = 22 + 5 * nt + 4 * no;
-        for (int j = 0; j < 5; ++j) f.tgt[j] = col(tgt, t_tgt + j);
-        for (int j = 0; j < 4 && no; ++j) f.obs[j] = col(tgt, t_obs + j);
-        for (int j = 0; j < 7 && nc; ++j) f.cam[j] = col(tgt, t_cam + j);
-        // every entry of a kind has the same bounds in both teams' rows (mate/constants.py:195-254): checked, not assumed
-        for (int e = 0; e < nt; ++e) for (int j = 0; j < 5; ++j) {
-            uniform = uniform && same(f.tgt[j], col(tgt, t_tgt + 5 * e + j));
-            if (nc) uniform = uniform && same(f.tgt[j], col(cam, c_tgt + 5 * e + j));
+        for (int j = 0; j < ObsLayout::PRESERVED; ++j) { f.pres[j] = col(tgt, j); if (nc) uniform = uniform && same(f.pres[j], col(cam, j)); }
+        for (int j = 0; j < ObsLayout::TGT_PRIVATE; ++j) f.tself[j] = col(tgt, ObsLayout::SELF + j);
+        for (int j = 0; j < ObsLayout::CAM_PRIVATE && nc; ++j) f.cself[j] = col(cam, ObsLayout::SELF + j);
+        // an entry of each kind from the target rows; every entry of a kind has the same bounds in both teams' rows
+        // (mate/constants.py:195-254): checked, not assumed
+        float2* const entry[3] = {f.tgt, f.obs, f.cam};   // by EntityKind
+        for (int kind = KIND_TARGET; kind <= KIND_CAMERA; ++kind) {
+            if (L.count(kind) == 0) continue;
+            const int w = ObsLayout::width(kind);
+            for (int j = 0; j < w; ++j) entry[kind][j] = col(tgt, L.entry_offset(false, kind, 0) + j);
+            for (int e = 0; e < L.count(kind); ++e) for (int j = 0; j < w; ++j) {
+                uniform = uniform && same(entry[kind][j], col(tgt, L.entry_offset(false, kind, e) + j));
+                if (nc) uniform = uniform && same(entry[kind][j], col(cam, L.entry_offset(true, kind, e) + j));
+            }
         }
-        for (int e = 0; e < no; ++e) for (int j = 0; j < 4; ++j) {
-            uniform = uniform && same(f.obs[j], col(tgt, t_obs + 4 * e + j));
-            if (nc) uniform = uniform && same(f.obs[j], col(cam, c_obs + 4 * e + j));
-        }
-        for (int e = 0; e < nc; ++e) for (int j = 0; j < 7; ++j)
-            uniform = uniform && same(f.cam[j], col(tgt, t_cam + 7 * e + j)) && same(f.cam[j], col(cam, c_cam + 7 * e + j));
         if (!uniform) f.fast = 0;   // tables of the caller's own: generic path
     }
     if (const char* v = getenv("MATE_B200_FOLD")) { if (v[0] == '0') f.fast = 0; }   // tests: force the generic shared-memory path

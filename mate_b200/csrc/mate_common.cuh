@@ -37,6 +37,46 @@ __host__ __device__ inline int tp_capacity(uint32_t p) { return (int)((p >> 21) 
 __host__ __device__ inline int tp_empty(uint32_t p) { return (int)((p >> 23) & 15); }
 __host__ __device__ inline int tp_colliding(uint32_t p) { return (int)((p >> 27) & 1); }
 
+// ---- observation row layout (mate/constants.py:267-300), the reference's format ----------------
+// A row is the preserved block, the observer's own (private) state, then one entry per entity: its public state and a
+// visibility flag.  Camera rows list targets, obstacles, cameras; target rows list cameras, obstacles, targets.
+// Kernels use it as `constexpr ObsLayout L{NC, NT, NO}` (every value a compile-time constant), the host with run-time counts.
+enum EntityKind : int { KIND_TARGET = 0, KIND_OBSTACLE = 1, KIND_CAMERA = 2 };
+
+struct ObsLayout {
+    int nc, nt, no;
+    // preserved block, the same in both teams' rows: counts (3), own index, warehouse locations (2 NW), warehouse radius
+    static constexpr int PRESERVED = 3 + 1 + 2 * NW + 1;
+    static constexpr int WAREHOUSE = 3 + 1;                   // first of the 2 NW warehouse coordinates (x, y per warehouse)
+    // own state: location in columns SELF, SELF + 1; a target's ends with its NW empty bits
+    static constexpr int SELF = PRESERVED;
+    static constexpr int CAM_PRIVATE = 9, TGT_PRIVATE = 6 + 2 * NW;
+    static constexpr int TGT_EMPTY = SELF + TGT_PRIVATE - NW;
+    // one entry of an entity list: public state + flag
+    static constexpr int TGT_ENTRY = 4 + 1, OBS_ENTRY = 3 + 1, CAM_ENTRY = 6 + 1;
+    __host__ __device__ static constexpr int width(int kind) {
+        return kind == KIND_TARGET ? TGT_ENTRY : (kind == KIND_OBSTACLE ? OBS_ENTRY : CAM_ENTRY);
+    }
+    __host__ __device__ constexpr int count(int kind) const { return kind == KIND_TARGET ? nt : (kind == KIND_OBSTACLE ? no : nc); }
+    // first column of the entity list of `kind` in a camera / target row
+    __host__ __device__ constexpr int block(bool cam_row, int kind) const {
+        const int c_tgt = SELF + CAM_PRIVATE, c_obs = c_tgt + TGT_ENTRY * nt, c_cam = c_obs + OBS_ENTRY * no;
+        const int t_cam = SELF + TGT_PRIVATE, t_obs = t_cam + CAM_ENTRY * nc, t_tgt = t_obs + OBS_ENTRY * no;
+        return cam_row ? (kind == KIND_TARGET ? c_tgt : (kind == KIND_OBSTACLE ? c_obs : c_cam))
+                       : (kind == KIND_CAMERA ? t_cam : (kind == KIND_OBSTACLE ? t_obs : t_tgt));
+    }
+    __host__ __device__ constexpr int entry_offset(bool cam_row, int kind, int index) const {
+        return block(cam_row, kind) + width(kind) * index;
+    }
+    __host__ __device__ constexpr int dc() const { return block(true, KIND_CAMERA) + CAM_ENTRY * nc; }
+    __host__ __device__ constexpr int dt() const { return block(false, KIND_TARGET) + TGT_ENTRY * nt; }
+    // (scale, shift) columns of the packer's RescaledObservation (FoldOps): preserved | target own state | camera own
+    // state | one target, obstacle and camera entry
+    static constexpr int AFF_PRES = 0, AFF_TSELF = AFF_PRES + PRESERVED, AFF_CSELF = AFF_TSELF + TGT_PRIVATE;
+    static constexpr int AFF_TGT = AFF_CSELF + CAM_PRIVATE, AFF_OBS = AFF_TGT + TGT_ENTRY, AFF_CAM = AFF_OBS + OBS_ENTRY;
+    static constexpr int AFF_COLS = AFF_CAM + CAM_ENTRY;
+};
+
 // observation wrappers (mate_wrappers.cuh), innermost first
 constexpr int kMaxObsOps = MATE_MAX_OBS_OPS;
 struct ObsOps { int n; int op[kMaxObsOps]; };
@@ -52,9 +92,9 @@ struct FoldOps {
     int fast;                           // the registered stack has the canonical form; 0 = generic shared-memory path
     int n_mask; int mask_op[kMaxObsOps];
     int relative, rescaled;
-    float2 pres[13];                    // (scale, shift) of the preserved block's columns (the same for both teams)
-    float2 cself[9], tself[14];         // private state of a camera / a target row
-    float2 tgt[5], obs[4], cam[7];      // a target / obstacle / camera entry with its flag
+    float2 pres[ObsLayout::PRESERVED];  // (scale, shift) of the preserved block's columns (the same for both teams)
+    float2 cself[ObsLayout::CAM_PRIVATE], tself[ObsLayout::TGT_PRIVATE];                        // private state of a camera / a target row
+    float2 tgt[ObsLayout::TGT_ENTRY], obs[ObsLayout::OBS_ENTRY], cam[ObsLayout::CAM_ENTRY];     // a target / obstacle / camera entry with its flag
 };
 
 struct Params {

@@ -58,8 +58,7 @@ __device__ __forceinline__ void tl_mark(const int env0, const int k) {
 
 template <int NC, int NT, int NO>
 struct Shape2 {
-    static constexpr int DC = 22 + 5 * NT + 4 * NO + 7 * NC;   // mate/constants.py:267-282
-    static constexpr int DT = 27 + 7 * NC + 4 * NO + 5 * NT;   // mate/constants.py:285-300
+    static constexpr int DC = ObsLayout{NC, NT, NO}.dc(), DT = ObsLayout{NC, NT, NO}.dt();
     static constexpr int CAM_ROW = NC * DC, TGT_ROW = NT * DT; // floats per environment
     static constexpr int R = NC + NT;                          // observer rows per environment
     // mask words per observer row: word 0 = cameras (bits 0-7), targets (bits 8-15) and, when
@@ -83,7 +82,9 @@ struct Shape2 {
     // (16 bytes / 8 bytes / odd) into rounds of 32 / NO rows, and a round stores with the widest aligned type
     // (1, 2 or 3 instructions instead of 4) -- unless the grouping needs more than one round more than plain row order.
     struct ORounds { int n; int grouped; int row[40][4]; int cls[40]; };   // cls: 0 = 16-byte aligned, 2 = 8-byte, 1 = odd, -1 = mixed (scalar stores)
-    __host__ __device__ static constexpr int o_offset(int row) { return row < NC ? row * (DC + CAM_SKEW) + 22 + 5 * NT : STAGE_CAM + (row - NC) * DT + 27 + 7 * NC; }
+    __host__ __device__ static constexpr int o_offset(int row) {
+        return (row < NC ? row * (DC + CAM_SKEW) : STAGE_CAM + (row - NC) * DT) + ObsLayout{NC, NT, NO}.block(row < NC, KIND_OBSTACLE);
+    }
     __host__ __device__ static constexpr ORounds make_orounds() {
         ORounds r{};
         const int rpr = NO > 0 ? 32 / NO : 1, plain = (R + rpr - 1) / rpr;
@@ -118,7 +119,7 @@ struct Shape2 {
     static constexpr int OFF_Q2 = OFF_Q + QCAP * 2;             // second queue: pairs that need the exact polyline
     static constexpr int WARP_BYTES = ((OFF_Q2 + QCAP * 2 + 15) / 16) * 16;
     // scratch of the observation wrappers folded into the packer (apply_obs_ops), behind the block, only when some are registered
-    static constexpr int FOLD_SCR = 4 * (NT + NO + NC) + R * MW + 1 + 2 * (13 + 14 + 9 + 5 + 4 + 7);   // fp64 locations, mask words, (scale, shift) of the own-row columns
+    static constexpr int FOLD_SCR = 4 * (NT + NO + NC) + R * MW + 1 + 2 * ObsLayout::AFF_COLS;   // fp64 locations, mask words, (scale, shift) of the own-row columns
     static constexpr int OPS_FLOATS = WShape<NC, NT, NO>::SCR > FOLD_SCR ? WShape<NC, NT, NO>::SCR : FOLD_SCR;
     static constexpr int OPS_BYTES = ((OPS_FLOATS * 4 + 15) / 16) * 16;
     static constexpr int SMEM_BYTES = WARPS * WARP_BYTES;
@@ -687,6 +688,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     constexpr int R = S::R, MW = S::MW, DC = S::DC, DT = S::DT, CV = S::CV;
     constexpr int NCX = NC > 0 ? NC : 1;
     constexpr uint32_t FULLMASK = 0xffffffffu;
+    constexpr ObsLayout L{NC, NT, NO};
     const int lane = threadIdx.x & 31;
     // ---- folded wrappers: which ones, and the scratch they use (behind the warp's block, present when wrappers are registered)
     const bool fast = FOLD && p.fold.fast != 0;
@@ -694,10 +696,15 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     constexpr int EALL = NT + NO + NC;
     double* const fpos = reinterpret_cast<double*>(ops_scratch);                       // [EALL][2] fp64 locations: targets, obstacles, cameras
     uint32_t* const mmod = reinterpret_cast<uint32_t*>(ops_scratch) + 4 * EALL;       // [R * MW] mask words after the mask wrappers
-    float2* const aff_own = reinterpret_cast<float2*>(ops_scratch + 4 * EALL + R * MW + ((R * MW) & 1));   // [13 | 14 | 9 | 5 | 4 | 7] preserved, target private, camera private, target / obstacle / camera entries
+    float2* const aff_own = reinterpret_cast<float2*>(ops_scratch + 4 * EALL + R * MW + ((R * MW) & 1));   // [ObsLayout::AFF_COLS] (scale, shift)
     if (FOLD && f_resc) {   // staged once per tile: the parameter block is only reachable through slow generic loads here
-        for (int k = lane; k < 52; k += 32)
-            aff_own[k] = k < 13 ? p.fold.pres[k] : (k < 27 ? p.fold.tself[k - 13] : (k < 36 ? p.fold.cself[k - 27] : (k < 41 ? p.fold.tgt[k - 36] : (k < 45 ? p.fold.obs[k - 41] : p.fold.cam[k - 45]))));
+        using A = ObsLayout;
+        for (int k = lane; k < A::AFF_COLS; k += 32)
+            aff_own[k] = k < A::AFF_TSELF ? p.fold.pres[k - A::AFF_PRES]
+                       : (k < A::AFF_CSELF ? p.fold.tself[k - A::AFF_TSELF]
+                       : (k < A::AFF_TGT ? p.fold.cself[k - A::AFF_CSELF]
+                       : (k < A::AFF_OBS ? p.fold.tgt[k - A::AFF_TGT]
+                       : (k < A::AFF_CAM ? p.fold.obs[k - A::AFF_OBS] : p.fold.cam[k - A::AFF_CAM]))));
     }
     // launch parameters used inside the loop, read once (a reference to the parameter block is a generic
     // pointer: the compiler would re-load through it after every store)
@@ -711,8 +718,9 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     //     the same entity for all rounds of a kind); a pair writes the entity's public state and flag if
     //     the observer's mask bit is set and zeros otherwise (masked-out entries are all-zero);
     //   * lanes 0..R-1 write the preserved block and the private state of "their" observer row.
-    constexpr int C_SELF = 13, C_TGT = 22, C_OBS = 22 + 5 * NT, C_CAM = 22 + 5 * NT + 4 * NO;
-    constexpr int T_SELF = 13, T_CAM = 27, T_OBS = 27 + 7 * NC, T_TGT = 27 + 7 * NC + 4 * NO;
+    // first columns of the entity lists in a camera (C_*) / target (T_*) row, as constants (see apply_obs_ops)
+    constexpr int C_TGT = L.block(true, KIND_TARGET), C_OBS = L.block(true, KIND_OBSTACLE), C_CAM = L.block(true, KIND_CAMERA);
+    constexpr int T_TGT = L.block(false, KIND_TARGET), T_OBS = L.block(false, KIND_OBSTACLE), T_CAM = L.block(false, KIND_CAMERA);
     constexpr int NOX = NO > 0 ? NO : 1;
     constexpr int RPR_T = 32 / NT, RPR_O = 32 / NOX, RPR_C = 32 / NCX;          // observer rows per round
     constexpr typename S::ORounds ORND = S::make_orounds();
@@ -736,7 +744,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     for (int rd = 0; rd < RND_T; ++rd) {
         const int row = rd * RPR_T + t_sub;
         const bool on = t_sub < RPR_T && row < R;
-        q_ptr[rd] = stage + (on ? row_base(row) + (row < NC ? C_TGT : T_TGT) + 5 * t_idx : 0);
+        q_ptr[rd] = stage + (on ? row_base(row) + (row < NC ? C_TGT : T_TGT) + ObsLayout::TGT_ENTRY * t_idx : 0);
         m_idx[rd] = on ? row * MW : 0;
         on_bits |= (uint32_t)on << rd;
     }
@@ -751,7 +759,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
                 for (int j = 0; j < 4; ++j) row = (j < RPR_O && o_sub == j) ? ORND.row[rd][j] : row;
                 on = row >= 0;
             }
-            q_ptr[RND_T + rd] = stage + (on ? row_base(row) + (row < NC ? C_OBS : T_OBS) + 4 * o_idx : 0);
+            q_ptr[RND_T + rd] = stage + (on ? row_base(row) + (row < NC ? C_OBS : T_OBS) + ObsLayout::OBS_ENTRY * o_idx : 0);
             m_idx[RND_T + rd] = on ? row * MW + (MW - 1) : 0;
             on_bits |= (uint32_t)on << (RND_T + rd);
         }
@@ -761,7 +769,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
         for (int rd = 0; rd < RND_C; ++rd) {
             const int row = rd * RPR_C + c_sub;
             const bool on = c_sub < RPR_C && row < R;
-            q_ptr[NRND - RND_C + rd] = stage + (on ? row_base(row) + (row < NC ? C_CAM : T_CAM) + 7 * c_idx : 0);
+            q_ptr[NRND - RND_C + rd] = stage + (on ? row_base(row) + (row < NC ? C_CAM : T_CAM) + ObsLayout::CAM_ENTRY * c_idx : 0);
             m_idx[NRND - RND_C + rd] = on ? row * MW : 0;
             on_bits |= (uint32_t)on << (NRND - RND_C + rd);
         }
@@ -779,16 +787,19 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
             const int row = lane;
             float* q = stage + row_base(row);
             auto put = [&](const int col, const float x, const int aff) { q[col] = (FOLD && f_resc) ? fmaf(x, aff_own[aff].x, aff_own[aff].y) : x; };
-            put(0, (float)NC, 0); put(1, (float)NT, 1); put(2, (float)NO, 2); put(3, (float)(row < NC ? row : row - NC), 3);
-            put(4, 925.f, 4); put(5, 925.f, 5); put(6, -925.f, 6); put(7, 925.f, 7); put(8, -925.f, 8); put(9, -925.f, 9); put(10, 925.f, 10); put(11, -925.f, 11);
-            put(12, 75.f, 12);
-            if (row < NC) { put(C_SELF + 2, f_crad, 27 + 2); put(C_SELF + 6, f_rmax, 27 + 6); put(C_SELF + 7, f_rot, 27 + 7); put(C_SELF + 8, f_zoom, 27 + 8); }
-            else put(T_SELF + 2, f_sr, 13 + 2);
+            static_assert(ObsLayout::PRESERVED == 13 && ObsLayout::WAREHOUSE == 4, "the preserved block is written column by column");
+            auto pres = [&](const int col, const float x) { put(col, x, ObsLayout::AFF_PRES + col); };
+            pres(0, (float)NC); pres(1, (float)NT); pres(2, (float)NO); pres(3, (float)(row < NC ? row : row - NC));
+            pres(4, 925.f); pres(5, 925.f); pres(6, -925.f); pres(7, 925.f); pres(8, -925.f); pres(9, -925.f); pres(10, 925.f); pres(11, -925.f);   // warehouses
+            pres(12, 75.f);
+            constexpr int C = ObsLayout::SELF, AC = ObsLayout::AFF_CSELF;
+            if (row < NC) { put(C + 2, f_crad, AC + 2); put(C + 6, f_rmax, AC + 6); put(C + 7, f_rot, AC + 7); put(C + 8, f_zoom, AC + 8); }
+            else put(C + 2, f_sr, ObsLayout::AFF_TSELF + 2);
         }
     };
     stage_constants();
-    float* const self_t = stage + S::STAGE_CAM + t_idx * DT + T_SELF;   // used by lanes 0..NT-1
-    float* const self_c = stage + c_idx * DCS + C_SELF;                  // used by the NC lanes from NT on
+    float* const self_t = stage + S::STAGE_CAM + t_idx * DT + ObsLayout::SELF;   // used by lanes 0..NT-1
+    float* const self_c = stage + c_idx * DCS + ObsLayout::SELF;                 // used by the NC lanes from NT on
     // obstacle entries are fetched two environments ahead (an L2 round trip is longer than one iteration)
     const float4* ob_ptr = obs_f4 + (size_t)o_idx * bp + env0;
     float4 ob_next = make_float4(0.f, 0.f, 0.f, 0.f), ob_next2 = ob_next;
@@ -903,7 +914,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
                 {   // targets + flag
                     float2 a[5];
 #pragma unroll
-                    for (int j = 0; j < 5; ++j) a[j] = f_resc ? aff_own[36 + j] : make_float2(1.f, 0.f);
+                    for (int j = 0; j < 5; ++j) a[j] = f_resc ? aff_own[ObsLayout::AFF_TGT + j] : make_float2(1.f, 0.f);
                     double ex = 0.0, ey = 0.0;
                     if (f_rel) { ex = fpos[2 * t_idx]; ey = fpos[2 * t_idx + 1]; }
                     // the lane keeps its entity for all rounds: the entries are rescaled once per environment, a round selects
@@ -933,7 +944,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
                 if (NO > 0) {   // obstacles + flag
                     float2 a[4];
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) a[j] = f_resc ? aff_own[41 + j] : make_float2(1.f, 0.f);
+                    for (int j = 0; j < 4; ++j) a[j] = f_resc ? aff_own[ObsLayout::AFF_OBS + j] : make_float2(1.f, 0.f);
                     double ex = 0.0, ey = 0.0;
                     if (f_rel) { ex = fpos[2 * (NT + o_idx)]; ey = fpos[2 * (NT + o_idx) + 1]; }
                     const float e_in[4] = {ob.x, ob.y, ob.z, 1.f};
@@ -961,7 +972,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
                 if (NC > 0) {   // cameras + flag
                     float2 a[7];
 #pragma unroll
-                    for (int j = 0; j < 7; ++j) a[j] = f_resc ? aff_own[45 + j] : make_float2(1.f, 0.f);
+                    for (int j = 0; j < 7; ++j) a[j] = f_resc ? aff_own[ObsLayout::AFF_CAM + j] : make_float2(1.f, 0.f);
                     double ex = 0.0, ey = 0.0;
                     if (f_rel) { ex = fpos[2 * (NT + NO + c_idx)]; ey = fpos[2 * (NT + NO + c_idx) + 1]; }
                     const float e_in[7] = {c0, c1, f_crad, c3, c4, c5, 1.f};
@@ -1059,19 +1070,20 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
             // warehouse coordinates of the row (the agent's own location stays absolute, mate/constants.py:372-427)
             const bool is_t = lane < NT, is_c = NC > 0 && lane >= NT && lane < NT + NC;
             float* const q = is_t ? self_t : self_c;
-            const int aff0 = is_t ? 13 : 27;
+            const int aff0 = is_t ? ObsLayout::AFF_TSELF : ObsLayout::AFF_CSELF;
             auto put = [&](const int j, const float x) { q[j] = (FOLD && f_resc) ? fmaf(x, aff_own[aff0 + j].x, aff_own[aff0 + j].y) : x; };
             if (is_t || is_c) {
                 put(0, is_t ? t0 : c0); put(1, is_t ? t1 : c1); put(3, is_t ? t3 : c3); put(4, is_t ? s_step : c4); put(5, is_t ? s_cap : c5);
                 if (FOLD && f_rel) {
                     const int ko = is_t ? lane : NT + NO + c_idx;
-                    float* const pr = q - 13;      // the row's preserved block (C_SELF == T_SELF == 13)
+                    float* const pr = q - ObsLayout::SELF;   // the row's preserved block
                     const double ox = fpos[2 * ko], oy = fpos[2 * ko + 1];
 #pragma unroll
-                    for (int j = 0; j < 8; ++j) {
+                    for (int j = 0; j < 2 * NW; ++j) {
                         const float wh = (j == 0 || j == 1 || j == 3 || j == 6) ? 925.f : -925.f;   // (+,+) (-,+) (-,-) (+,-)
                         const float x = (float)((double)wh - ((j & 1) ? oy : ox));
-                        pr[4 + j] = f_resc ? fmaf(x, aff_own[4 + j].x, aff_own[4 + j].y) : x;
+                        constexpr int WH = ObsLayout::WAREHOUSE, AW = ObsLayout::AFF_PRES + WH;
+                        pr[WH + j] = f_resc ? fmaf(x, aff_own[AW + j].x, aff_own[AW + j].y) : x;
                     }
                 }
             }

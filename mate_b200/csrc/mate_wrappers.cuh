@@ -20,7 +20,7 @@ namespace mate {
 
 template <int NC, int NT, int NO>
 struct WShape {
-    static constexpr int DC = 22 + 5 * NT + 4 * NO + 7 * NC, DT = 27 + 7 * NC + 4 * NO + 5 * NT;
+    static constexpr int DC = ObsLayout{NC, NT, NO}.dc(), DT = ObsLayout{NC, NT, NO}.dt();
     static constexpr int CAM_ROW = NC * DC, TGT_ROW = NT * DT;
     static constexpr int BLOCK = CAM_ROW + TGT_ROW;            // floats per environment
     static constexpr int E = NT + NO + NC;                     // entity slots per observer row
@@ -32,21 +32,6 @@ struct WShape {
     static constexpr bool VEC = (CAM_ROW % 4 == 0) && (TGT_ROW % 4 == 0);
 };
 
-// slot k of an observer row: kind 0 = target, 1 = obstacle, 2 = camera; camera rows list targets,
-// obstacles, cameras; target rows list cameras, obstacles, targets (mate/constants.py:267-300)
-template <int NC, int NT, int NO>
-__device__ __forceinline__ void slot_of(bool cam_row, int k, int* kind, int* idx, int* off, int* width) {
-    if (cam_row) {
-        if (k < NT) { *kind = 0; *idx = k; *off = 22 + 5 * k; *width = 5; }
-        else if (k < NT + NO) { *kind = 1; *idx = k - NT; *off = 22 + 5 * NT + 4 * (k - NT); *width = 4; }
-        else { *kind = 2; *idx = k - NT - NO; *off = 22 + 5 * NT + 4 * NO + 7 * (k - NT - NO); *width = 7; }
-    } else {
-        if (k < NC) { *kind = 2; *idx = k; *off = 27 + 7 * k; *width = 7; }
-        else if (k < NC + NO) { *kind = 1; *idx = k - NC; *off = 27 + 7 * NC + 4 * (k - NC); *width = 4; }
-        else { *kind = 0; *idx = k - NC - NO; *off = 27 + 7 * NC + 4 * NO + 5 * (k - NC - NO); *width = 5; }
-    }
-}
-
 // The registered observation wrappers applied IN PLACE to the rows of one environment that a warp holds in shared
 // memory: B = camera rows [NC][DC], T = target rows [NT][DT]; `scr` = S::SCR floats of scratch (8-byte aligned).
 // Called by all 32 lanes.  Used by obs_transform_kernel (a pass over observation tensors) and by the step kernel's
@@ -56,6 +41,9 @@ __device__ __forceinline__ void apply_obs_ops(const Params& p, const ObsOps& ops
                                               const float* aff_cam, const float* aff_tgt) {
     using S = WShape<NC, NT, NO>;
     constexpr int DC = S::DC, DT = S::DT, E = S::E, R = S::R;
+    // Entry offsets are L.entry_offset(observer is a camera, kind, index), written as block start + width * index with the
+    // block starts as compile-time constants: the call with run-time arguments compiles to different code.
+    constexpr ObsLayout L{NC, NT, NO};
     const int lane = threadIdx.x & 31;
     float* ob = scr;                                           // [NO][4] obstacle_states_flagged
     float* shm = ob + 4 * (NO > 0 ? NO : 1);                   // [2][E] shared view masks (camera team, target team)
@@ -85,25 +73,23 @@ __device__ __forceinline__ void apply_obs_ops(const Params& p, const ObsOps& ops
     // f(row pointer, row, entity index, slot offset in that row).
     auto pairs = [&](auto k, const int r0, const int n, auto&& f) {
         constexpr int K = decltype(k)::value;
-        constexpr int N = K == 0 ? NT : (K == 1 ? NO : NC);
-        constexpr int W = K == 0 ? 5 : (K == 1 ? 4 : 7);
+        constexpr int N = L.count(K), W = ObsLayout::width(K), OC = L.block(true, K), OT = L.block(false, K);
         if constexpr (N > 0) {
         for (int q = lane; q < n * N; q += 32) {
             const int r = r0 + q / (N > 0 ? N : 1), idx = q % (N > 0 ? N : 1);
-            const int off = r < NC ? (K == 0 ? 22 : (K == 1 ? 22 + 5 * NT : 22 + 5 * NT + 4 * NO)) + W * idx
-                                   : (K == 2 ? 27 : (K == 1 ? 27 + 7 * NC : 27 + 7 * NC + 4 * NO)) + W * idx;
+            const int off = r < NC ? OC + W * idx : OT + W * idx;
             f(row_ptr(r), r, idx, off);
         }
         }
     };
-    using K0 = std::integral_constant<int, 0>;
-    using K1 = std::integral_constant<int, 1>;
-    using K2 = std::integral_constant<int, 2>;
+    using K0 = std::integral_constant<int, KIND_TARGET>;
+    using K1 = std::integral_constant<int, KIND_OBSTACLE>;
+    using K2 = std::integral_constant<int, KIND_CAMERA>;
     // write the public state (+ flag 1) of entity `idx` of kind K, or zeros
     auto fill = [&](auto k, float* dst, const int idx, const bool on) {
         constexpr int K = decltype(k)::value;
-        constexpr int W = K == 0 ? 5 : (K == 1 ? 4 : 7);
-        const float* src = K == 0 ? T + idx * DT + 13 : (K == 1 ? ob + 4 * idx : B + idx * DC + 13);
+        constexpr int W = ObsLayout::width(K);
+        const float* src = K == 0 ? T + idx * DT + ObsLayout::SELF : (K == 1 ? ob + 4 * idx : B + idx * DC + ObsLayout::SELF);
 #pragma unroll
         for (int j = 0; j < W - 1; ++j) dst[j] = on ? src[j] : 0.f;
         dst[W - 1] = on ? 1.f : 0.f;
@@ -123,16 +109,18 @@ __device__ __forceinline__ void apply_obs_ops(const Params& p, const ObsOps& ops
                 for (int k = lane; k < E; k += 32) {
                     const int kind = k < NT ? 0 : (k < NT + NO ? 1 : 2);
                     const int idx = k < NT ? k : (k < NT + NO ? k - NT : k - NT - NO);
-                    const int w = kind == 0 ? 5 : (kind == 1 ? 4 : 7);
-                    const int off = cam_team ? (kind == 0 ? 22 : (kind == 1 ? 22 + 5 * NT : 22 + 5 * NT + 4 * NO)) + w * idx
-                                             : (kind == 2 ? 27 : (kind == 1 ? 27 + 7 * NC : 27 + 7 * NC + 4 * NO)) + w * idx;
+                    constexpr int C0 = L.block(true, KIND_TARGET), C1 = L.block(true, KIND_OBSTACLE), C2 = L.block(true, KIND_CAMERA);
+                    constexpr int T0 = L.block(false, KIND_TARGET), T1 = L.block(false, KIND_OBSTACLE), T2 = L.block(false, KIND_CAMERA);
+                    const int w = kind == 0 ? ObsLayout::TGT_ENTRY : (kind == 1 ? ObsLayout::OBS_ENTRY : ObsLayout::CAM_ENTRY);
+                    const int off = cam_team ? (kind == 0 ? C0 : (kind == 1 ? C1 : C2)) + w * idx
+                                             : (kind == 2 ? T2 : (kind == 1 ? T1 : T0)) + w * idx;
                     bool any = cam_team ? kind == 2 : kind == 0;   // teammates are always shared (flag 1)
                     for (int r = 0; r < nrows; ++r) any = any || row_ptr(r0 + r)[off + w - 1] != 0.f;
                     shm[k] = any ? 1.f : 0.f;
                 }
                 if (!cam_team && lane < NW) {
                     bool any = false;
-                    for (int t = 0; t < NT; ++t) any = any || row_ptr(NC + t)[13 + 10 + lane] != 0.f;
+                    for (int t = 0; t < NT; ++t) any = any || row_ptr(NC + t)[ObsLayout::TGT_EMPTY + lane] != 0.f;
                     she[lane] = any ? 1.f : 0.f;
                 }
             } else if (!cam_team && lane < NW) {   // np.logical_not(remaining_cargoes).all(axis=-1)
@@ -146,7 +134,7 @@ __device__ __forceinline__ void apply_obs_ops(const Params& p, const ObsOps& ops
             pairs(K1{}, r0, nrows, [&](float* row, int, int idx, int off) { fill(K1{}, row + off, idx, !shared || shm[SH1 + idx] != 0.f); });
             pairs(K2{}, r0, nrows, [&](float* row, int, int idx, int off) { fill(K2{}, row + off, idx, !shared || shm[SH2 + idx] != 0.f); });
             if (!cam_team) {
-                for (int q = lane; q < NT * NW; q += 32) row_ptr(NC + q / NW)[13 + 10 + (q % NW)] = she[q % NW];
+                for (int q = lane; q < NT * NW; q += 32) row_ptr(NC + q / NW)[ObsLayout::TGT_EMPTY + (q % NW)] = she[q % NW];
             }
             __syncwarp();
         } else if (op == MATE_OBS_RELATIVE) {
@@ -156,13 +144,13 @@ __device__ __forceinline__ void apply_obs_ops(const Params& p, const ObsOps& ops
             for (int j = 0; j < i; ++j) exact = exact && ops.op[j] != MATE_OBS_RESCALED;
             auto relative = [&](auto k, float* row, const int r, const int idx, const int off) {
                 constexpr int K = decltype(k)::value;
-                constexpr int W = K == 0 ? 5 : (K == 1 ? 4 : 7);
+                constexpr int W = ObsLayout::width(K);
                 if (row[off + W - 1] == 0.f) return;
                 if (exact) {
                     const int ke = (K == 0 ? SH0 : (K == 1 ? SH1 : SH2)) + idx, ko = r < NC ? SH2 + r : r - NC;
                     row[off] = (float)(pos[2 * ke] - pos[2 * ko]); row[off + 1] = (float)(pos[2 * ke + 1] - pos[2 * ko + 1]);
                 } else {
-                    row[off] -= row[13]; row[off + 1] -= row[14];
+                    row[off] -= row[ObsLayout::SELF]; row[off + 1] -= row[ObsLayout::SELF + 1];
                 }
             };
             pairs(K0{}, 0, R, [&](float* row, int r, int idx, int off) { relative(K0{}, row, r, idx, off); });
@@ -172,8 +160,9 @@ __device__ __forceinline__ void apply_obs_ops(const Params& p, const ObsOps& ops
                 const int r = q / (2 * NW), j = q % (2 * NW);
                 float* row = row_ptr(r);
                 const int ko = r < NC ? SH2 + r : r - NC;
-                if (exact) row[4 + j] = (float)((double)row[4 + j] - pos[2 * ko + (j & 1)]);
-                else row[4 + j] -= row[13 + (j & 1)];
+                constexpr int WH = ObsLayout::WAREHOUSE;
+                if (exact) row[WH + j] = (float)((double)row[WH + j] - pos[2 * ko + (j & 1)]);
+                else row[WH + j] -= row[ObsLayout::SELF + (j & 1)];
             }
             __syncwarp();
         } else if (op == MATE_OBS_RESCALED) {

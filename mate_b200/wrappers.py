@@ -18,7 +18,7 @@ import functools
 import numpy as np
 import torch
 
-from mate_b200 import _abi, spaces
+from mate_b200 import _abi, constants, spaces
 
 TEAMS = ('both', 'camera', 'target', 'none')
 
@@ -333,19 +333,20 @@ class MoreTrainingInformation(Wrapper):
             'individual_done': tgt_terms[..., 5] != 0, 'is_tracked': tgt_terms[..., 7] != 0, 'is_colliding': tgt_terms[..., 8] != 0,
         })
         # full observability (more_training_information.py:84-98)
-        offset = 13   # PRESERVED_DIM
+        cam_self = slice(constants.PRESERVED_DIM, constants.PRESERVED_DIM + constants.CAMERA_STATE_DIM_PRIVATE)
+        tgt_self = slice(constants.PRESERVED_DIM, constants.PRESERVED_DIM + constants.TARGET_STATE_DIM_PRIVATE)
         shared = {
             'camera_target_view_mask': aux['mask_ct'].bool(), 'camera_obstacle_view_mask': aux['mask_co'].bool(),
             'target_camera_view_mask': aux['mask_tc'].bool(), 'target_obstacle_view_mask': aux['mask_to'].bool(),
             'target_target_view_mask': aux['mask_tt'].bool(),
         }
         if base.batched:
-            shared['camera_states'] = camera_joint_observation[..., offset:offset + 9]
-            shared['target_states'] = target_joint_observation[..., offset:offset + 14]
+            shared['camera_states'] = camera_joint_observation[..., cam_self]
+            shared['target_states'] = target_joint_observation[..., tgt_self]
         else:
             shared = {k: v[0].cpu().numpy() for k, v in shared.items()}
-            shared['camera_states'] = np.array(camera_joint_observation[..., offset:offset + 9])
-            shared['target_states'] = np.array(target_joint_observation[..., offset:offset + 14])
+            shared['camera_states'] = np.array(camera_joint_observation[..., cam_self])
+            shared['target_states'] = np.array(target_joint_observation[..., tgt_self])
         if self.full_observability:
             remaining = np.asarray(base.remaining_cargoes)
             shared.update(state=base.state(), obstacle_states=np.asarray(base.obstacle_states), remaining_cargoes=remaining,
@@ -744,8 +745,8 @@ class MultiTarget(_SingleTeamSnapshot, Wrapper):
         """Target flags of the cameras' current observations ``[B, Nc, Nt]`` (also right for environments that were
         auto-reset in the last step, whose auxiliary masks still describe the finished step)."""
         base = self.unwrapped
-        nt = base.num_targets
-        flags = base.sim.cam_obs[..., 22 + 4:22 + 5 * nt:5]   # camera observation layout, mate/constants.py:267-282
+        mask = constants.camera_observation_slices_of(base.num_cameras, base.num_targets, base.num_obstacles)['opponent_mask']
+        flags = base.sim.cam_obs[..., mask]
         return (flags > 0.5).to(torch.uint8)
 
     def step(self, action):
