@@ -213,7 +213,8 @@ int mate_b200_step_host(MateSim* sim, const float* cam_act, const float* tgt_act
 
 /* State view / injection (host arrays; synchronises the device).  A view, not a complete checkpoint: it leaves out the
  * running coverage sum, the line-of-sight cache, the Philox seed and the episode statistics; use mate_b200_save_state
- * to save and restore a batch exactly. */
+ * to save and restore a batch exactly.  A set_state refused for a value out of range (MATE_EINVAL) leaves the handle
+ * unchanged. */
 int mate_b200_get_state(MateSim* sim, MateStateView* view);
 int mate_b200_set_state(MateSim* sim, const MateStateView* view);
 

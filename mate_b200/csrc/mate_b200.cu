@@ -184,6 +184,8 @@ struct MateSim {
     Params base{};            // state pointers + scalars; per-call fields are filled per launch
     void* state_block = nullptr;
     size_t state_bytes = 0;
+    void* host_block = nullptr;   // pinned host copy of the state block (get_state / set_state), made on first use
+    Params host{};                // the state pointers of host_block, carved like those of base
     double* d_ranges = nullptr;
     unsigned long long seed = 0;
     uint64_t config_hash = 0; // fingerprint of cfg (config_fingerprint): snapshots load only into handles of the same configuration
@@ -252,6 +254,7 @@ struct MateSim {
         cudaFree(next_block);
         cudaFree(d_next);
         cudaFree(state_block);
+        cudaFreeHost(host_block);
         cudaFree(d_ranges);
         if (l2_window) l2_keep_release(device);
     }
@@ -1075,81 +1078,61 @@ extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const flo
 }
 
 // ---- state get / set (host arrays, synchronous) --------------------------------------------------
-template <typename T>
-static int download(std::vector<T>& host, const T* dev, size_t n) {
-    host.resize(n);
-    CUDA_TRY(cudaMemcpy(host.data(), dev, n * sizeof(T), cudaMemcpyDeviceToHost));
+// Both move the whole state block through its host copy (MateSim::host) and convert each field between the
+// struct-of-arrays values [row * bpad + env] and the batched rows [B][rows][comps] of a MateStateView.
+// The host copy is carved like the device block, so host code reads and writes the state at the device's offsets.  It is
+// pinned, since pageable copies of the block made both calls slower than the per-array copies they replace, and made on
+// first use, since pinning it in create made create + destroy 17 times as long (MATE-4v8-9 x 65 536, one B200).
+static int ensure_host_copy(MateSim* sim) {
+    if (sim->host_block) return MATE_OK;
+    if (cudaMallocHost(&sim->host_block, sim->state_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        sim->host_block = nullptr;
+        return fail(MATE_ENOMEM, "cudaMallocHost(state copy) failed");
+    }
+    carve_state(sim->host, (char*)sim->host_block, sim->cfg.num_cameras, sim->cfg.num_targets, sim->cfg.num_obstacles, sim->bpad, false);
     return MATE_OK;
-}
-template <typename T>
-static int upload(const std::vector<T>& host, T* dev) {
-    CUDA_TRY(cudaMemcpy(dev, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return MATE_OK;
-}
-// struct-of-arrays values [rows][bpad] -> component k of the batched rows [B][rows][comps] of a MateStateView field
-template <typename T>
-static void gather_rows(const MateSim* sim, const std::vector<T>& soa, int rows, T* out, int comps, int k) {
-    for (size_t e = 0; e < (size_t)sim->num_envs; ++e)
-        for (int r = 0; r < rows; ++r) out[(e * rows + r) * comps + k] = soa[r * (size_t)sim->bpad + e];
-}
-// component k of the batched rows [B][rows][comps] of a MateStateView field -> struct-of-arrays values [rows][bpad]
-template <typename T>
-static void scatter_rows(const MateSim* sim, const T* in, int rows, int comps, int k, std::vector<T>& soa) {
-    for (size_t e = 0; e < (size_t)sim->num_envs; ++e)
-        for (int r = 0; r < rows; ++r) soa[r * (size_t)sim->bpad + e] = in[(e * rows + r) * comps + k];
 }
 
 extern "C" int mate_b200_get_state(MateSim* sim, MateStateView* v) {
     if (!sim || !v) return fail(MATE_EINVAL, "null argument");
     CUDA_TRY(cudaSetDevice(sim->device));
     CUDA_TRY(cudaDeviceSynchronize());
+    if (int rc = ensure_host_copy(sim)) return rc;
+    const Params& h = sim->host;
+    CUDA_TRY(cudaMemcpy(sim->host_block, sim->state_block, sim->state_bytes, cudaMemcpyDeviceToHost));
     const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets, no = sim->cfg.num_obstacles;
     const size_t bp = sim->bpad, B = sim->num_envs;
-    const Params& p = sim->base;
-    std::vector<double> a, b2, c, d;
-    if (nc && (v->cam_xy || v->cam_phi || v->cam_theta)) {
-        if (download(a, p.cam_x, nc * bp) || download(b2, p.cam_y, nc * bp) || download(c, p.cam_phi, nc * bp) || download(d, p.cam_theta, nc * bp)) return MATE_ECUDA;
-        if (v->cam_xy) { gather_rows(sim, a, nc, v->cam_xy, 2, 0); gather_rows(sim, b2, nc, v->cam_xy, 2, 1); }
-        if (v->cam_phi) gather_rows(sim, c, nc, v->cam_phi, 1, 0);
-        if (v->cam_theta) gather_rows(sim, d, nc, v->cam_theta, 1, 0);
-    }
-    if (v->tgt_xy) {
-        if (download(a, p.tgt_x, nt * bp) || download(b2, p.tgt_y, nt * bp)) return MATE_ECUDA;
-        gather_rows(sim, a, nt, v->tgt_xy, 2, 0);
-        gather_rows(sim, b2, nt, v->tgt_xy, 2, 1);
-    }
-    if (no && v->obs_xyr) {
-        if (download(a, p.obs_x, no * bp) || download(b2, p.obs_y, no * bp) || download(c, p.obs_r, no * bp)) return MATE_ECUDA;
-        gather_rows(sim, a, no, v->obs_xyr, 3, 0);
-        gather_rows(sim, b2, no, v->obs_xyr, 3, 1);
-        gather_rows(sim, c, no, v->obs_xyr, 3, 2);
-    }
-    {
-        std::vector<uint32_t> pack;
-        if (download(pack, p.tgt_pack, nt * bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < nt; ++k) {
-                const uint32_t q = pack[k * bp + e];
-                if (v->tgt_capacity) v->tgt_capacity[e * nt + k] = tp_capacity(q);
-                if (v->tgt_goal) v->tgt_goal[e * nt + k] = tp_goal(q);
-                if (v->tgt_weight) v->tgt_weight[e * nt + k] = tp_weight(q);
-                if (v->tgt_bounty) v->tgt_bounty[e * nt + k] = tp_bounty(q);
-                if (v->tgt_empty_bits) v->tgt_empty_bits[e * nt + k] = tp_empty(q);
-            }
-    }
-    {
-        std::vector<uint4> cargo, ea;
-        std::vector<int4> eb;
-        if (download(cargo, p.cargo, 2 * bp) || download(ea, p.env_a, bp) || download(eb, p.env_b, bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e) {
-            const uint32_t words[8] = {cargo[e].x, cargo[e].y, cargo[e].z, cargo[e].w, cargo[bp + e].x, cargo[bp + e].y, cargo[bp + e].z, cargo[bp + e].w};
-            if (v->remaining) for (int i = 0; i < 16; ++i) v->remaining[e * 16 + i] = (int32_t)((words[i >> 1] >> ((i & 1) * 16)) & 0xFFFF);
-            if (v->awaiting) { v->awaiting[e * 4 + 0] = ea[e].x & 0xFFFF; v->awaiting[e * 4 + 1] = ea[e].x >> 16; v->awaiting[e * 4 + 2] = ea[e].y & 0xFFFF; v->awaiting[e * 4 + 3] = ea[e].y >> 16; }
-            if (v->episode_step) v->episode_step[e] = (int32_t)ea[e].z;
-            if (v->num_delivered) v->num_delivered[e] = (int32_t)ea[e].w;
-            if (v->episode_reward) { v->episode_reward[e * 2] = (double)eb[e].x; v->episode_reward[e * 2 + 1] = (double)eb[e].y; }
-            if (v->episode_id) v->episode_id[e] = eb[e].w;
+    for (size_t e = 0; e < B; ++e) {
+        for (int r = 0; r < nc; ++r) {
+            const size_t s = r * bp + e, i = e * nc + r;
+            if (v->cam_xy) { v->cam_xy[2 * i] = h.cam_x[s]; v->cam_xy[2 * i + 1] = h.cam_y[s]; }
+            if (v->cam_phi) v->cam_phi[i] = h.cam_phi[s];
+            if (v->cam_theta) v->cam_theta[i] = h.cam_theta[s];
         }
+        for (int r = 0; r < nt; ++r) {
+            const size_t s = r * bp + e, i = e * nt + r;
+            if (v->tgt_xy) { v->tgt_xy[2 * i] = h.tgt_x[s]; v->tgt_xy[2 * i + 1] = h.tgt_y[s]; }
+            const uint32_t q = h.tgt_pack[s];
+            if (v->tgt_capacity) v->tgt_capacity[i] = tp_capacity(q);
+            if (v->tgt_goal) v->tgt_goal[i] = tp_goal(q);
+            if (v->tgt_weight) v->tgt_weight[i] = tp_weight(q);
+            if (v->tgt_bounty) v->tgt_bounty[i] = tp_bounty(q);
+            if (v->tgt_empty_bits) v->tgt_empty_bits[i] = tp_empty(q);
+        }
+        for (int r = 0; r < no; ++r) {
+            const size_t s = r * bp + e, i = e * no + r;
+            if (v->obs_xyr) { v->obs_xyr[3 * i] = h.obs_x[s]; v->obs_xyr[3 * i + 1] = h.obs_y[s]; v->obs_xyr[3 * i + 2] = h.obs_r[s]; }
+        }
+        const uint4 c0 = h.cargo[e], c1 = h.cargo[bp + e], a = h.env_a[e];
+        const int4 b = h.env_b[e];
+        const uint32_t words[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
+        if (v->remaining) for (int k = 0; k < 16; ++k) v->remaining[e * 16 + k] = (int32_t)((words[k >> 1] >> ((k & 1) * 16)) & 0xFFFF);
+        if (v->awaiting) { v->awaiting[e * 4 + 0] = a.x & 0xFFFF; v->awaiting[e * 4 + 1] = a.x >> 16; v->awaiting[e * 4 + 2] = a.y & 0xFFFF; v->awaiting[e * 4 + 3] = a.y >> 16; }
+        if (v->episode_step) v->episode_step[e] = (int32_t)a.z;
+        if (v->num_delivered) v->num_delivered[e] = (int32_t)a.w;
+        if (v->episode_reward) { v->episode_reward[e * 2] = (double)b.x; v->episode_reward[e * 2 + 1] = (double)b.y; }
+        if (v->episode_id) v->episode_id[e] = b.w;
     }
     return MATE_OK;
 }
@@ -1158,78 +1141,63 @@ extern "C" int mate_b200_set_state(MateSim* sim, const MateStateView* v) {
     if (!sim || !v) return fail(MATE_EINVAL, "null argument");
     CUDA_TRY(cudaSetDevice(sim->device));
     CUDA_TRY(cudaDeviceSynchronize());
-    if (sim->refill_mode) CUDA_TRY(cudaMemset(sim->base.ready, 0, sizeof(uint32_t) * sim->bpad));   // prepared episodes may no longer match
+    if (int rc = ensure_host_copy(sim)) return rc;
+    const Params& h = sim->host;
+    CUDA_TRY(cudaMemcpy(sim->host_block, sim->state_block, sim->state_bytes, cudaMemcpyDeviceToHost));
     const int nc = sim->cfg.num_cameras, nt = sim->cfg.num_targets, no = sim->cfg.num_obstacles;
     const size_t bp = sim->bpad, B = sim->num_envs;
-    const Params& p = sim->base;
-    std::vector<double> a, b2, c, d;
-    if (nc) {
-        if (download(a, p.cam_x, nc * bp) || download(b2, p.cam_y, nc * bp) || download(c, p.cam_phi, nc * bp) || download(d, p.cam_theta, nc * bp)) return MATE_ECUDA;
-        if (v->cam_theta)
-            for (size_t i = 0; i < B * nc; ++i)
-                if (!(v->cam_theta[i] > 0.0) || v->cam_theta[i] > 180.0) return fail(MATE_EINVAL, "cam_theta out of (0, 180]");
-        if (v->cam_xy) { scatter_rows(sim, v->cam_xy, nc, 2, 0, a); scatter_rows(sim, v->cam_xy, nc, 2, 1, b2); }
-        if (v->cam_phi) scatter_rows(sim, v->cam_phi, nc, 1, 0, c);
-        if (v->cam_theta) scatter_rows(sim, v->cam_theta, nc, 1, 0, d);
-        if (upload(a, p.cam_x) || upload(b2, p.cam_y) || upload(c, p.cam_phi) || upload(d, p.cam_theta)) return MATE_ECUDA;
-    }
-    if (v->cam_xy || v->obs_xyr)   // geometry changed: invalidate the per-episode camera line-of-sight cache
-        CUDA_TRY(cudaMemset(p.cc_clear, 0, sizeof(unsigned long long) * bp));
-    if (v->tgt_xy) {
-        a.assign(nt * bp, 0.0); b2.assign(nt * bp, 0.0);
-        scatter_rows(sim, v->tgt_xy, nt, 2, 0, a);
-        scatter_rows(sim, v->tgt_xy, nt, 2, 1, b2);
-        if (upload(a, p.tgt_x) || upload(b2, p.tgt_y)) return MATE_ECUDA;
-    }
-    if (no && v->obs_xyr) {
-        a.assign(no * bp, 0.0); b2.assign(no * bp, 0.0); c.assign(no * bp, 0.0);
-        scatter_rows(sim, v->obs_xyr, no, 3, 0, a);
-        scatter_rows(sim, v->obs_xyr, no, 3, 1, b2);
-        scatter_rows(sim, v->obs_xyr, no, 3, 2, c);
-        if (upload(a, p.obs_x) || upload(b2, p.obs_y) || upload(c, p.obs_r)) return MATE_ECUDA;
-        std::vector<float4> f4(no * bp);   // fp32 shadow read by the prefilters and the observation packer
-        for (size_t i = 0; i < f4.size(); ++i) f4[i] = make_float4((float)a[i], (float)b2[i], (float)c[i], 0.f);
-        if (upload(f4, p.obs_f4)) return MATE_ECUDA;
-    }
-    {
-        std::vector<uint32_t> pack;
-        if (download(pack, p.tgt_pack, nt * bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e)
-            for (int k = 0; k < nt; ++k) {
-                const uint32_t q = pack[k * bp + e];
-                int capacity = v->tgt_capacity ? v->tgt_capacity[e * nt + k] : tp_capacity(q);
-                int goal = v->tgt_goal ? v->tgt_goal[e * nt + k] : tp_goal(q);
-                int weight = v->tgt_weight ? v->tgt_weight[e * nt + k] : tp_weight(q);
-                int bounty = v->tgt_bounty ? v->tgt_bounty[e * nt + k] : tp_bounty(q);
-                int empty = v->tgt_empty_bits ? v->tgt_empty_bits[e * nt + k] : tp_empty(q);
-                if (capacity < 1 || capacity > 2 || goal < -1 || goal > 3 || weight < 0 || weight > 3 || bounty < 0 || bounty > 65535)
-                    return fail(MATE_EINVAL, "target integer state out of range");
-                pack[k * bp + e] = pack_target(bounty, goal, weight, capacity, empty, tp_colliding(q));
-            }
-        if (upload(pack, p.tgt_pack)) return MATE_ECUDA;
-    }
-    {
-        std::vector<uint4> cargo, ea;
-        std::vector<int4> eb;
-        if (download(cargo, p.cargo, 2 * bp) || download(ea, p.env_a, bp) || download(eb, p.env_b, bp)) return MATE_ECUDA;
-        for (size_t e = 0; e < B; ++e) {
-            if (v->remaining) {
-                uint32_t words[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-                for (int i = 0; i < 16; ++i) words[i >> 1] |= ((uint32_t)v->remaining[e * 16 + i] & 0xFFFF) << ((i & 1) * 16);
-                cargo[e] = make_uint4(words[0], words[1], words[2], words[3]);
-                cargo[bp + e] = make_uint4(words[4], words[5], words[6], words[7]);
-            }
-            if (v->awaiting) {
-                ea[e].x = ((uint32_t)v->awaiting[e * 4 + 0] & 0xFFFF) | ((uint32_t)v->awaiting[e * 4 + 1] << 16);
-                ea[e].y = ((uint32_t)v->awaiting[e * 4 + 2] & 0xFFFF) | ((uint32_t)v->awaiting[e * 4 + 3] << 16);
-            }
-            if (v->episode_step) ea[e].z = (uint32_t)v->episode_step[e];
-            if (v->num_delivered) ea[e].w = (uint32_t)v->num_delivered[e];
-            if (v->episode_reward) { eb[e].x = (int)std::lrint(v->episode_reward[e * 2]); eb[e].y = (int)std::lrint(v->episode_reward[e * 2 + 1]); eb[e].z = 0; }
-            if (v->episode_id) eb[e].w = v->episode_id[e];
+    if (v->cam_theta)
+        for (size_t i = 0; i < B * nc; ++i)
+            if (!(v->cam_theta[i] > 0.0) || v->cam_theta[i] > 180.0) return fail(MATE_EINVAL, "cam_theta out of (0, 180]");
+    // Until the upload below only the host copy changes (each call downloads it afresh): a view refused on the way leaves
+    // the handle as it was.
+    for (size_t e = 0; e < B; ++e) {
+        for (int r = 0; r < nc; ++r) {
+            const size_t s = r * bp + e, i = e * nc + r;
+            if (v->cam_xy) { h.cam_x[s] = v->cam_xy[2 * i]; h.cam_y[s] = v->cam_xy[2 * i + 1]; }
+            if (v->cam_phi) h.cam_phi[s] = v->cam_phi[i];
+            if (v->cam_theta) h.cam_theta[s] = v->cam_theta[i];
         }
-        if (upload(cargo, p.cargo) || upload(ea, p.env_a) || upload(eb, p.env_b)) return MATE_ECUDA;
+        for (int r = 0; r < nt; ++r) {
+            const size_t s = r * bp + e, i = e * nt + r;
+            if (v->tgt_xy) { h.tgt_x[s] = v->tgt_xy[2 * i]; h.tgt_y[s] = v->tgt_xy[2 * i + 1]; }
+            const uint32_t q = h.tgt_pack[s];
+            const int capacity = v->tgt_capacity ? v->tgt_capacity[i] : tp_capacity(q);
+            const int goal = v->tgt_goal ? v->tgt_goal[i] : tp_goal(q);
+            const int weight = v->tgt_weight ? v->tgt_weight[i] : tp_weight(q);
+            const int bounty = v->tgt_bounty ? v->tgt_bounty[i] : tp_bounty(q);
+            const int empty = v->tgt_empty_bits ? v->tgt_empty_bits[i] : tp_empty(q);
+            if (capacity < 1 || capacity > 2 || goal < -1 || goal > 3 || weight < 0 || weight > 3 || bounty < 0 || bounty > 65535)
+                return fail(MATE_EINVAL, "target integer state out of range");
+            h.tgt_pack[s] = pack_target(bounty, goal, weight, capacity, empty, tp_colliding(q));
+        }
+        for (int r = 0; r < no; ++r) {
+            const size_t s = r * bp + e, i = e * no + r;
+            if (v->obs_xyr) {
+                h.obs_x[s] = v->obs_xyr[3 * i]; h.obs_y[s] = v->obs_xyr[3 * i + 1]; h.obs_r[s] = v->obs_xyr[3 * i + 2];
+                h.obs_f4[s] = make_float4((float)h.obs_x[s], (float)h.obs_y[s], (float)h.obs_r[s], 0.f);   // fp32 shadow read by the prefilters and the observation packer
+            }
+        }
+        if (v->cam_xy || v->obs_xyr) h.cc_clear[e] = 0;   // geometry changed: invalidate the per-episode camera line-of-sight cache
+        uint4& a = h.env_a[e];
+        int4& b = h.env_b[e];
+        if (v->remaining) {
+            uint32_t words[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+            for (int k = 0; k < 16; ++k) words[k >> 1] |= ((uint32_t)v->remaining[e * 16 + k] & 0xFFFF) << ((k & 1) * 16);
+            h.cargo[e] = make_uint4(words[0], words[1], words[2], words[3]);
+            h.cargo[bp + e] = make_uint4(words[4], words[5], words[6], words[7]);
+        }
+        if (v->awaiting) {
+            a.x = ((uint32_t)v->awaiting[e * 4 + 0] & 0xFFFF) | ((uint32_t)v->awaiting[e * 4 + 1] << 16);
+            a.y = ((uint32_t)v->awaiting[e * 4 + 2] & 0xFFFF) | ((uint32_t)v->awaiting[e * 4 + 3] << 16);
+        }
+        if (v->episode_step) a.z = (uint32_t)v->episode_step[e];
+        if (v->num_delivered) a.w = (uint32_t)v->num_delivered[e];
+        if (v->episode_reward) { b.x = (int)std::lrint(v->episode_reward[e * 2]); b.y = (int)std::lrint(v->episode_reward[e * 2 + 1]); b.z = 0; }
+        if (v->episode_id) b.w = v->episode_id[e];
     }
+    CUDA_TRY(cudaMemcpy(sim->state_block, sim->host_block, sim->state_bytes, cudaMemcpyHostToDevice));
+    if (sim->refill_mode) CUDA_TRY(cudaMemset(sim->base.ready, 0, sizeof(uint32_t) * sim->bpad));   // prepared episodes may no longer match
     return launch_prepare(sim, nullptr);   // prepare the next episodes of the new state right away
 }
 

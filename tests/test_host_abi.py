@@ -112,3 +112,42 @@ def test_destroy_returns_device_memory(monkeypatch):
         # mate_b200_destroy had before MateSim got a destructor and with the destructor: every round came back to the
         # baseline to the byte.  The 2 MiB tolerance (one large-page granule) is far below what one leaked buffer costs.
         assert abs(free - baseline) <= 2 << 20, (k, free - baseline)
+
+
+@pytest.mark.parametrize('preset', ['MATE-4v8-9.yaml', 'MATE-Navigation.yaml'])
+def test_refused_set_state_changes_nothing(preset):
+    """set_state checks the whole view before it writes: a view with valid new positions and episode clocks but one
+    out-of-range value in its last environment is refused (ValueError) with the handle unchanged, the parts that
+    get_state leaves out (line-of-sight cache, coverage sum, statistics) included."""
+    from mate_b200.config import flatten_config, read_config
+    from mate_b200.sim import BatchedSim
+
+    cfg = flatten_config(read_config(preset))
+    nc, nt = cfg['num_cameras'], cfg['num_targets']
+    B = 1000
+    sim = BatchedSim(cfg, B, device=0)
+    sim.reset(seed=5)
+    rng = np.random.default_rng(2)
+    for _ in range(3):
+        cam_act = torch.from_numpy((rng.uniform(-1, 1, (B, max(nc, 1), 2)) * [5.0, 2.5]).astype(np.float32)).cuda()
+        tgt_act = torch.from_numpy((rng.uniform(-1, 1, (B, nt, 2)) * 20.0).astype(np.float32)).cuda()
+        sim.step(cam_act, tgt_act, auto_reset=True)
+    before = sim.get_state()
+    saved = sim.save_state().payload.clone()
+    valid = {key: _new_values(key, before[key], rng).astype(before[key].dtype)
+             for key in ('cam_xy', 'tgt_xy', 'obs_xyr', 'episode_step') if before[key].size}
+    bad_goal = before['tgt_goal'].copy()
+    bad_goal[-1] = 5
+    views = [{**valid, 'tgt_goal': bad_goal}]
+    if nc:
+        bad_theta = before['cam_theta'].copy()
+        bad_theta[-1] = 0.0
+        views.append({**valid, 'cam_theta': bad_theta})
+    for view in views:
+        with pytest.raises(ValueError):
+            sim.set_state(view)
+        after = sim.get_state()
+        for key in before:
+            assert np.array_equal(after[key], before[key]), key
+        assert torch.equal(sim.save_state().payload, saved)
+    sim.close()
