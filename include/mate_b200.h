@@ -403,6 +403,40 @@ typedef struct MateMessageFilter {
 } MateMessageFilter;
 int mate_b200_set_message_filter(MateSim* sim, const MateMessageFilter* filter);
 
+/* The tensor message channel of a learning team (DESIGN.md section 7i): every agent s of the team sends one message of
+ * `dim` floats, content[b][s][:], to the teammates r with recipients[b][s][r] != 0 (NULL = broadcast: to every
+ * teammate, its own copy included, like a broadcast Message).  A routed message is delivered iff it passes the team's
+ * registered filter (mate_b200_set_message_filter) exactly as the greedy teams' messages do: the range rule on the
+ * positions of the current state, then the dropout draw, word r % 4 of the Philox call keyed on (the handle's seed, the
+ * global environment index, 'COMM') with counter (serial, 22 << 16 | team << 8 | s << 2 | r >> 2).  The caller advances
+ * `serial` once per call; the draws do not depend on the batch split.
+ *   - MATE_MESSAGES_NONE: inbox [B, N(r), N(s), dim]; inbox[b][r][s] is s's message, bit for bit, if it reached r, else 0.
+ *   - MATE_MESSAGES_SUM:  inbox [B, N(r), dim], the float32 sum of the delivered messages, added in ascending s from 0.
+ *   - MATE_MESSAGES_MEAN: that sum divided (IEEE, round to nearest) by the number of delivered senders; 0 without any.
+ * A message that is not delivered is never read.  Every element of inbox (and of delivered) is written.  delivered
+ * [B, N(r), N(s)] (nullable) gets 1 where s's message reached r, else 0.  When the team's edge tensors are registered
+ * the call writes the delivered set to delivered[team][b] (bit 8 s + r) and adds it to total_edges[team]; an
+ * environment's totals restart from this call's set when its episode id differs from episode[b], which is then set to
+ * it (the caller sets episode[b] = -1 to restart them at the next call).  The call enqueues one kernel on `stream` and
+ * never synchronises.  MATE_EINVAL, nothing launched, for a team other than 0 / 1, a team of 0 or more than 8 agents,
+ * dim < 1 (or N * N * dim above 2^31 - 1), an unknown reduction, a NULL content, inbox or episode, or content / inbox /
+ * episode not 4-byte aligned. */
+#define MATE_MESSAGES_NONE 0
+#define MATE_MESSAGES_SUM 1
+#define MATE_MESSAGES_MEAN 2
+typedef struct MateMessageExchange {
+    const float* content;          /* dev [B, N, dim]                                                                 */
+    const uint8_t* recipients;     /* dev [B, N(s), N(r)]: non-zero = s sends to r; NULL = broadcast                  */
+    float* inbox;                  /* dev [B, N, N, dim] (NONE) or [B, N, dim] (SUM / MEAN)                           */
+    uint8_t* delivered;            /* dev [B, N(r), N(s)]: 1 = s's message reached r; nullable                        */
+    int32_t* episode;              /* dev [B]: the episode id the team's totals belong to, -1 = restart them          */
+    int32_t team;                  /* 0 = cameras, 1 = targets                                                        */
+    int32_t dim;                   /* floats per message, >= 1                                                        */
+    int32_t reduction;             /* MATE_MESSAGES_NONE / _SUM / _MEAN                                               */
+    int32_t reserved;              /* 0                                                                               */
+} MateMessageExchange;
+int mate_b200_exchange_messages(MateSim* sim, const MateMessageExchange* exchange, uint64_t serial, void* stream);
+
 /* DiscreteCamera / DiscreteTarget.action (mate/wrappers/discrete_action_spaces.py:98-117, 204-228): grid
  * indices (dev int64 [count]) -> continuous actions (dev float32 [count][2]) through the wrapper's table
  * (dev float32 [table_size][2]). */

@@ -118,6 +118,17 @@ class MateMessageFilter(ctypes.Structure):
                 ('delivered', ctypes.c_void_p * 2), ('total_edges', ctypes.c_void_p * 2)]
 
 
+class MateMessageExchange(ctypes.Structure):
+    _fields_ = [('content', ctypes.c_void_p), ('recipients', ctypes.c_void_p), ('inbox', ctypes.c_void_p),
+                ('delivered', ctypes.c_void_p), ('episode', ctypes.c_void_p), ('team', ctypes.c_int32),
+                ('dim', ctypes.c_int32), ('reduction', ctypes.c_int32), ('reserved', ctypes.c_int32)]
+
+
+# reductions of mate_b200_exchange_messages (MATE_MESSAGES_*)
+MATE_MESSAGES_NONE, MATE_MESSAGES_SUM, MATE_MESSAGES_MEAN = 0, 1, 2
+MESSAGE_REDUCTIONS = {'none': MATE_MESSAGES_NONE, 'sum': MATE_MESSAGES_SUM, 'mean': MATE_MESSAGES_MEAN}
+
+
 class MateReplay(ctypes.Structure):
     _fields_ = [('transmit', c_uint8_p), ('goal_choice', c_int8_p)]
 
@@ -228,8 +239,10 @@ def load_library():
                                                     ctypes.POINTER(MateCameraAgentReplay), void_p, void_p]
     lib.mate_b200_soft_coverage.argtypes = [void_p, void_p, void_p, void_p, void_p]
     lib.mate_b200_set_message_filter.argtypes = [void_p, ctypes.POINTER(MateMessageFilter)]
+    lib.mate_b200_exchange_messages.argtypes = [void_p, ctypes.POINTER(MateMessageExchange), ctypes.c_uint64, void_p]
     for name in ('create', 'destroy', 'obs_dims', 'set_observation_format', 'reset', 'seed', 'step', 'observe', 'step_host',
-                 'get_state', 'set_state', 'snapshot_bytes', 'save_state', 'load_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions', 'set_message_filter'):
+                 'get_state', 'set_state', 'snapshot_bytes', 'save_state', 'load_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions', 'set_message_filter',
+                 'exchange_messages'):
         getattr(lib, 'mate_b200_' + name).restype = ctypes.c_int
     _LIB = lib
     return lib
@@ -242,7 +255,7 @@ EXPORTED_SYMBOLS = [
     'mate_b200_load_state',
     'mate_b200_episode_stats', 'mate_b200_launch_count', 'mate_b200_host_leg_info', 'mate_b200_transform_observations', 'mate_b200_set_observation_ops',
     'mate_b200_decode_actions', 'mate_b200_auxiliary_terms', 'mate_b200_fov_range', 'mate_b200_soft_coverage', 'mate_b200_greedy_target_actions', 'mate_b200_greedy_camera_actions',
-    'mate_b200_set_message_filter',
+    'mate_b200_set_message_filter', 'mate_b200_exchange_messages',
 ]
 
 # observation wrapper codes (include/mate_b200.h)

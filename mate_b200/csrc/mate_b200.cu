@@ -21,6 +21,7 @@
 #include "mate_agents.cuh"
 #include "mate_hostpath.cuh"
 #include "mate_snapshot.cuh"
+#include "mate_messages.cuh"
 
 using namespace mate;
 
@@ -668,6 +669,34 @@ extern "C" int mate_b200_greedy_camera_actions(MateSim* sim, double* memory, con
         sim->base, nc, nt, memory, tracked, reset_mask, seed, serial, r, comm_filter(sim, 0), cam_act);
     sim->launches += 1;
     return check_launch("greedy camera");
+}
+
+extern "C" int mate_b200_exchange_messages(MateSim* sim, const MateMessageExchange* exchange, uint64_t serial, void* stream) {
+    if (!sim || !exchange) return fail(MATE_EINVAL, "null argument");
+    const MateMessageExchange m = *exchange;
+    if (m.team != 0 && m.team != 1) return fail(MATE_EINVAL, "team must be 0 (cameras) or 1 (targets)");
+    const int n = m.team == 0 ? sim->cfg.num_cameras : sim->cfg.num_targets;
+    if (n < 1 || n > 8) return fail(MATE_EINVAL, "the message exchange covers teams of 1 to 8 agents (bit 8 s + r)");
+    if (m.dim < 1 || (long long)n * n * m.dim > 0x7FFFFFFFll) return fail(MATE_EINVAL, "dim must be >= 1 and N * N * dim < 2^31");
+    if (m.reduction != MATE_MESSAGES_NONE && m.reduction != MATE_MESSAGES_SUM && m.reduction != MATE_MESSAGES_MEAN)
+        return fail(MATE_EINVAL, "reduction must be MATE_MESSAGES_NONE, _SUM or _MEAN");
+    if (!m.content || !m.inbox || !m.episode) return fail(MATE_EINVAL, "content, inbox and episode are required");
+    if (((uintptr_t)m.content & 3) || ((uintptr_t)m.inbox & 3) || ((uintptr_t)m.episode & 3))
+        return fail(MATE_EINVAL, "content, inbox and episode must be 4-byte aligned");
+    CUDA_TRY(cudaSetDevice(sim->device));
+    const Params& p = sim->base;
+    ExchangeArgs a{};
+    a.content = m.content; a.recipients = m.recipients; a.inbox = m.inbox; a.delivered = m.delivered; a.episode = m.episode;
+    a.x = m.team == 0 ? p.cam_x : p.tgt_x;
+    a.y = m.team == 0 ? p.cam_y : p.tgt_y;
+    a.env_b = p.env_b;
+    a.comm = comm_filter(sim, m.team);
+    a.num_envs = sim->num_envs; a.bpad = sim->bpad; a.n = n; a.dim = m.dim; a.reduction = m.reduction;
+    a.vec = m.dim % 4 == 0 && !((uintptr_t)m.content & 15) && !((uintptr_t)m.inbox & 15);
+    a.team = (uint32_t)m.team; a.serial = (uint32_t)serial; a.env_index_base = p.env_index_base;
+    message_exchange_kernel<<<(sim->num_envs + kExchangeWarps - 1) / kExchangeWarps, kExchangeWarps * 32, 0, (cudaStream_t)stream>>>(a);
+    sim->launches += 1;
+    return check_launch("message exchange");
 }
 
 extern "C" int mate_b200_decode_actions(const int64_t* index, const float* table, int32_t table_size, float* out,

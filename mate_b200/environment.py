@@ -141,6 +141,10 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         if self.batched:
             self._delivered_bits = tuple(torch.zeros(self.num_envs, dtype=torch.int64, device=self.device) for _ in range(2))
             self._total_edges = tuple(torch.zeros((self.num_envs, n, n), dtype=torch.int32, device=self.device) for n in (nc, nt))
+            # the tensor message channel (exchange_messages), per team: the episode id its totals belong to (-1 = restart
+            # them at the next exchange) and the call serial that keys its dropout draws
+            self._exchange_episode = tuple(torch.full((self.num_envs,), -1, dtype=torch.int32, device=self.device) for _ in range(2))
+            self._exchange_serials = [0, 0]
         else:
             self._edges = (np.zeros((nc, nc), dtype=np.int64), np.zeros((nt, nt), dtype=np.int64))
             self._total_edges = (np.zeros((nc, nc), dtype=np.int64), np.zeros((nt, nt), dtype=np.int64))
@@ -197,6 +201,8 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         self._seed = int(seed)
         self._np_random = np.random.RandomState(self._seed % (2 ** 32))
         self.sim.seed(self._seed % (2 ** 64))   # rewinds the episode counters: seed(s) + reset() is reproducible
+        if self.batched:
+            self._exchange_serials = [0, 0]       # and the message channel's drops
         return [self._seed]
 
     def load_config(self, config=None) -> None:
@@ -219,6 +225,8 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         if self.batched:   # environment.py:823-830
             for edges in self._delivered_bits + self._total_edges:
                 edges.zero_()
+            for episode in self._exchange_episode:
+                episode.fill_(-1)
         else:
             for edges in self._edges + self._total_edges:
                 edges.fill(0)
@@ -324,6 +332,31 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
     camera_total_communication_edges = property(lambda self: self._total_edges[0])
     target_total_communication_edges = property(lambda self: self._total_edges[1])
 
+    # ------------------------------------------------------------------ tensor messages of a learning team (batched mode)
+    def exchange_messages(self, team, content, recipients=None, reduction: str = 'none'):
+        """Send one message per agent of ``team`` (``'camera'`` / ``'target'``, 0 / 1 or ``Team``) and receive them, for
+        every environment in one kernel (DESIGN.md section 7i).  ``content`` float32 ``[B, N, D]`` on the environment's
+        device; ``recipients`` bool / uint8 ``[B, N, N]`` sender-major (entry ``[e, s, r]``: s sends to r), ``None`` =
+        broadcast to every teammate, the sender included.  A message is delivered iff it is sent and passes the
+        communication wrappers registered for the team (range on the current positions, dropout).  Returns ``(inbox,
+        delivered)``: ``inbox`` float32 ``[B, N(r), N(s), D]`` with s's message where it reached r and zeros elsewhere
+        (``reduction='none'``), or ``[B, N(r), D]``, the sum / mean over the delivered senders (``'sum'`` / ``'mean'``,
+        0 without any); ``delivered`` bool ``[B, N(r), N(s)]``.  The delivered set also becomes the team's
+        ``communication_edges`` and is added to its ``total_communication_edges``, which restart at the first exchange of
+        an episode."""
+        if not self.batched:
+            raise NotImplementedError('exchange_messages is the message channel of the batched mode (num_envs=B); the '
+                                      'single-environment mode exchanges Message objects with send_messages / receive_messages')
+        try:
+            index = consts._team_index(team)   # pylint: disable=protected-access
+        except (KeyError, TypeError, ValueError):
+            index = None
+        if index not in (0, 1):
+            raise ValueError(f"team must be 'camera' / 'target', 0 / 1 or a Team, got {team!r}")
+        out = self.sim.exchange_messages(index, content, recipients, reduction, self._exchange_serials[index], self._exchange_episode[index])
+        self._exchange_serials[index] += 1
+        return out
+
     # ------------------------------------------------------------------ intra-team messages (reference-compatible mode)
     def _clear_messages(self):
         for table in self.message_buffers + self.message_queues:
@@ -332,8 +365,9 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
     def _messages_supported(self):
         if self.batched:
             raise NotImplementedError(
-                'Message objects are a host API of the single-environment mode (num_envs=None); the batched greedy '
-                'teams exchange their messages inside their CUDA kernels (mate_b200.MultiCamera / MultiTarget)')
+                'Message objects are a host API of the single-environment mode (num_envs=None); in batched mode learning '
+                'teams exchange tensor messages with exchange_messages, and the greedy teams exchange theirs inside '
+                'their CUDA kernels (mate_b200.MultiCamera / MultiTarget)')
 
     def send_messages(self, messages) -> None:
         """Buffer messages from an agent to teammates; they are delivered by ``receive_messages`` and through the
@@ -417,8 +451,16 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         this object's seed and NumPy RNG state (a :class:`mate_b200.sim.StateSnapshot`; ``torch.save`` keeps it)."""
         snapshot = self.sim.save_state(envs)
         kind, key, pos, has_gauss, cached = self._np_random.get_state()
-        snapshot.extras['environment'] = {'seed': self._seed,
-                                          'np_random': (kind, torch.from_numpy(key.astype(np.int64)), pos, has_gauss, cached)}
+        saved = {'seed': self._seed, 'np_random': (kind, torch.from_numpy(key.astype(np.int64)), pos, has_gauss, cached)}
+        if self.batched:   # both teams' communication totals and the message channel's bookkeeping
+            index = None
+            if envs is not None:   # out-of-range device indices: the kernel leaves those entries unwritten, here they are clamped
+                index = self.sim._index_map(envs, 'envs', None, 0, self.num_envs).long().clamp_(0, self.num_envs - 1)  # pylint: disable=protected-access
+            pick = lambda t: (t if index is None else t.index_select(0, index)).clone()   # noqa: E731
+            saved.update(total_edges=tuple(pick(t) for t in self._total_edges),
+                         exchange_episode=tuple(pick(t) for t in self._exchange_episode),
+                         exchange_serials=list(self._exchange_serials))
+        snapshot.extras['environment'] = saved
         return snapshot
 
     def load_state(self, snapshot, src=None, resume: bool = False):
@@ -433,15 +475,38 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
             kind, key, pos, has_gauss, cached = saved['np_random']
             self._seed = saved['seed']
             self._np_random.set_state((kind, key.numpy().astype(np.uint32), pos, has_gauss, cached))
+        if self.batched and saved is not None and 'total_edges' in saved:   # older snapshots do not carry them
+            self._load_rows(self._total_edges + self._exchange_episode, saved['total_edges'] + saved['exchange_episode'],
+                            src, snapshot.count)
+            if resume:
+                self._exchange_serials = list(saved['exchange_serials'])
         cam_obs, tgt_obs = self.sim.observe(aux=True)   # the mask attributes of the loaded state
         self._needs_reset = False
         self._state_serial += 1
         return self._format_obs(cam_obs, tgt_obs)
 
+    def _load_rows(self, live, saved, src, count):
+        """Per-environment tensors (environment axis first) from a snapshot's entries along its index map, with the
+        simulator's rules: ``src=None`` takes entry d for environment d, a negative or out-of-range entry keeps d."""
+        index = None
+        if src is not None:
+            index = self.sim._index_map(src, 'src', self.num_envs, -(1 << 31), count).long()  # pylint: disable=protected-access
+            keep = (index < 0) | (index >= count)
+            index = index.clamp(0, count - 1)
+        for tensor, rows in zip(live, saved):
+            rows = rows.to(tensor.device)
+            if index is None:
+                tensor.copy_(rows)
+            else:
+                tensor.copy_(torch.where(keep.view((-1,) + (1,) * (tensor.dim() - 1)), tensor, rows.index_select(0, index)))
+
     def set_state(self, arrays: Dict[str, np.ndarray]) -> None:
         """Inject a state (the reference has no equivalent; used by the parity harness).  For checkpoint / resume use
         ``save_state`` / ``load_state``."""
         self.sim.set_state(arrays)
+        if self.batched:   # the message channel's totals restart at the next exchange
+            for episode in self._exchange_episode:
+                episode.fill_(-1)
         self.sim.observe(aux=True)
         self._needs_reset = False
         self._state_serial += 1

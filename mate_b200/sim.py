@@ -242,6 +242,46 @@ class BatchedSim:
         _check(self.lib, self.lib.mate_b200_set_message_filter(self.handle, ctypes.byref(f)))
         self._message_tensors = tensors   # the library keeps the pointers
 
+    def exchange_messages(self, team, content, recipients, reduction, serial, episode):
+        """The tensor message channel of team 0 (cameras) or 1 (targets) (mate_b200_exchange_messages): ``content``
+        float32 ``[B, N, D]``, one message per sender; ``recipients`` bool / uint8 ``[B, N, N]`` sender-major (``None`` =
+        broadcast); ``reduction`` ``'none'`` / ``'sum'`` / ``'mean'``; ``serial`` keys the dropout draws; ``episode`` is the
+        team's int32 ``[B]`` bookkeeping of the episode its totals belong to.  Returns fresh ``(inbox, delivered)``:
+        ``inbox`` float32 ``[B, N(r), N(s), D]`` (``'none'``) or ``[B, N(r), D]``, ``delivered`` bool ``[B, N(r), N(s)]``.
+        Every argument is checked here, before any library call; nothing synchronises."""
+        if team not in (0, 1):
+            raise ValueError(f'team must be 0 (cameras) or 1 (targets), got {team!r}')
+        n = (self.nc, self.nt)[team]
+        if not 0 < n <= 8:
+            raise ValueError(f'the message exchange covers teams of 1 to 8 agents (bit 8 s + r); team {team} has {n}')
+        if reduction not in _abi.MESSAGE_REDUCTIONS:
+            raise ValueError(f"reduction must be one of {sorted(_abi.MESSAGE_REDUCTIONS)}, got {reduction!r}")
+
+        def check(name, t, dtypes, shape):
+            if not torch.is_tensor(t) or t.dtype not in dtypes or t.device != self.device or t.dim() != len(shape) \
+                    or any(want is not None and got != want for got, want in zip(t.shape, shape)) or not t.is_contiguous():
+                kinds = ' or '.join(str(d) for d in dtypes)
+                raise ValueError(f'{name} must be a contiguous {kinds} tensor of shape {tuple("D" if s is None else s for s in shape)} '
+                                 f'on {self.device}, got {type(t).__name__} {getattr(t, "dtype", "")} {tuple(getattr(t, "shape", ()))} '
+                                 f'on {getattr(t, "device", "")}')
+
+        check('content', content, (torch.float32,), (self.B, n, None))
+        dim = int(content.shape[2])
+        if dim < 1 or n * n * dim >= 1 << 31:
+            raise ValueError(f'content must hold 1 to {((1 << 31) - 1) // (n * n)} floats per message, got {dim}')
+        if recipients is not None:
+            check('recipients', recipients, (torch.bool, torch.uint8), (self.B, n, n))
+        check('episode', episode, (torch.int32,), (self.B,))
+        out_shape = (self.B, n, n, dim) if reduction == 'none' else (self.B, n, dim)
+        inbox = torch.empty(out_shape, dtype=torch.float32, device=self.device)
+        delivered = torch.empty((self.B, n, n), dtype=torch.bool, device=self.device)
+        x = _abi.MateMessageExchange(content=content.data_ptr(), recipients=None if recipients is None else recipients.data_ptr(),
+                                     inbox=inbox.data_ptr(), delivered=delivered.data_ptr(), episode=episode.data_ptr(),
+                                     team=team, dim=dim, reduction=_abi.MESSAGE_REDUCTIONS[reduction], reserved=0)
+        with torch.cuda.device(self.device):
+            _check(self.lib, self.lib.mate_b200_exchange_messages(self.handle, ctypes.byref(x), int(serial) % (1 << 64), self._stream()))
+        return inbox, delivered
+
     # ------------------------------------------------------------------ API
     def seed(self, seed, env_mask=None):
         """``MultiAgentTracking.seed``: new key for the Philox streams, episode counters rewound (mate_b200_seed), so

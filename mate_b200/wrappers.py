@@ -588,8 +588,8 @@ class NoCommunication(_CommunicationWrapper):
 class _SingleTeamSnapshot:
     """``save_state`` / ``load_state`` of the single-team wrappers: besides the environment they carry the per-environment
     state of the opponent agent (its memory, gathered / scattered along the memory's environment axis with the
-    snapshot's index map), the opponent team's per-episode communication totals (batched mode) and the pending reset
-    mask; the agent's step serial is restored on resume only."""
+    snapshot's index map) and the pending reset mask; the agent's step serial is restored on resume only.  Both teams'
+    communication totals travel with the environment's part of the snapshot."""
 
     _MEMORY_AXIS = None   # environment axis of the agent's field-major memory tensor
     _TEAM = None          # index of this wrapper's team in the joint (camera, target) tuples
@@ -607,20 +607,11 @@ class _SingleTeamSnapshot:
         snapshot = self.env.save_state(envs)
         agent = self.opponent_agent
         memory, pending = agent._memory, self._pending_resets()   # pylint: disable=protected-access
-        totals = self._opponent_totals()
         if envs is not None:   # out-of-range device indices: the kernel leaves those entries unwritten, here they are clamped
             index = base.sim._index_map(envs, 'envs', None, 0, base.num_envs).long().clamp_(0, base.num_envs - 1)  # pylint: disable=protected-access
             memory, pending = memory.index_select(self._MEMORY_AXIS, index), pending.index_select(0, index)
-            totals = None if totals is None else totals.index_select(0, index)
         snapshot.extras['opponent'] = {'memory': memory.clone(), 'reset_mask': pending.clone(), 'serial': agent._serial}  # pylint: disable=protected-access
-        if totals is not None:
-            snapshot.extras['opponent']['total_edges'] = totals.clone()
         return snapshot
-
-    def _opponent_totals(self):
-        """The opponent team's per-episode communication totals ``[B, N, N]`` (batched mode), else ``None``."""
-        base = self.unwrapped
-        return base.total_communication_edges[1 - self._TEAM] if base.batched else None
 
     def load_state(self, snapshot, src=None, resume=False):
         base = self.unwrapped
@@ -629,16 +620,9 @@ class _SingleTeamSnapshot:
         agent = self.opponent_agent
         memory, pending = agent._memory, self._pending_resets()   # pylint: disable=protected-access
         saved_memory, saved_pending = saved['memory'].to(memory.device), saved['reset_mask'].to(pending.device)
-        totals, saved_totals = self._opponent_totals(), saved.get('total_edges')
-        if saved_totals is not None and totals is not None:
-            saved_totals = saved_totals.to(totals.device)
-        else:
-            totals = None
         if src is None:
             memory.copy_(saved_memory)
             pending = saved_pending.clone()
-            if totals is not None:
-                totals.copy_(saved_totals)
         else:
             index = base.sim._index_map(src, 'src', base.num_envs, -(1 << 31), snapshot.count).long()  # pylint: disable=protected-access
             keep = (index < 0) | (index >= snapshot.count)
@@ -647,8 +631,6 @@ class _SingleTeamSnapshot:
             shape[self._MEMORY_AXIS] = -1
             memory.copy_(torch.where(keep.view(shape), memory, saved_memory.index_select(self._MEMORY_AXIS, index)))
             pending = torch.where(keep, pending, saved_pending.index_select(0, index))
-            if totals is not None:
-                totals.copy_(torch.where(keep.view(-1, 1, 1), totals, saved_totals.index_select(0, index)))
         self._reset_mask = pending
         if resume:
             agent._serial = saved['serial']   # pylint: disable=protected-access
