@@ -166,7 +166,8 @@ int mate_b200_set_observation_format(MateSim* sim, int32_t format);
 /* MultiAgentTracking.reset (environment.py:679-834) for the envs with env_mask[b] != 0
  * (dev, NULL = all); Philox streams keyed on (seed, global env index, episode id).
  * Writes the first joint observation of the reset envs (other rows are rewritten with
- * their current observation); cam_obs / tgt_obs in the handle's observation format. */
+ * their current observation); cam_obs / tgt_obs in the handle's observation format.  Either may be NULL: that
+ * team's rows are then neither composed nor written (one team learning against built-in agents). */
 int mate_b200_reset(MateSim* sim, const uint8_t* env_mask, uint64_t seed,
                     float* cam_obs, float* tgt_obs, void* stream);
 
@@ -180,7 +181,9 @@ int mate_b200_seed(MateSim* sim, const uint8_t* env_mask, uint64_t seed, void* s
 /* MultiAgentTracking.step (environment.py:590-676) for all envs: _simulate,
  * _update_view, _assign_goals, joint_observation, reward/done.
  *   cam_act [B,Nc,2], tgt_act [B,Nt,2] float32 dev (finite);
- *   cam_obs [B,Nc,Dc], tgt_obs [B,Nt,Dt] dev, float32 or float16 (mate_b200_set_observation_format);
+ *   cam_obs [B,Nc,Dc], tgt_obs [B,Nt,Dt] dev, float32 or float16 (mate_b200_set_observation_format); either may be
+ *     NULL: that team's rows are neither composed nor written, and everything else is what a call with both
+ *     buffers computes;
  *   rewards [B,2] float32 dev = (camera_team_reward, target_team_reward);
  *   done [B] uint8 dev. */
 int mate_b200_step(MateSim* sim, const float* cam_act, const float* tgt_act,
@@ -190,7 +193,7 @@ int mate_b200_step(MateSim* sim, const float* cam_act, const float* tgt_act,
 
 /* joint_observation() of the current state without stepping (_update_view +
  * joint_observation, environment.py:1356-1388, 908-983); used after set_state.  cam_obs / tgt_obs in the
- * handle's observation format. */
+ * handle's observation format; either may be NULL (that team's rows are not written). */
 int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs,
                       const MateStepAux* aux, const MateReplay* replay, void* stream);
 
@@ -206,7 +209,10 @@ int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs,
  * (INTEGRATION.md), compacted: non-zero 16-byte chunks only, or -- with MATE_STEP_HOST_ROWS_KEPT -- only the 64-byte
  * groups that differ from the previous call's rows; host threads of the library put them in place before the call
  * returns.  The buffers hold the same bytes in every case.  Row buffers must be 4-byte aligned (16-byte aligned for full
- * speed) and of the handle's observation format (float16 rows halve the bytes on the link). */
+ * speed) and of the handle's observation format (float16 rows halve the bytes on the link).  cam_obs or tgt_obs may be
+ * NULL: that team's rows are not composed and nothing of them crosses the link.  MATE_STEP_HOST_ROWS_KEPT needs the same
+ * pointers, NULL included, as the previous call: a call that switches a team between NULL and a buffer writes every
+ * byte of the rows it is given. */
 int mate_b200_step_host(MateSim* sim, const float* cam_act, const float* tgt_act,
                         float* cam_obs, float* tgt_obs, float* rewards, uint8_t* done,
                         uint32_t flags);
@@ -449,7 +455,8 @@ int64_t mate_b200_launch_count(const MateSim* sim);
 /* What the last mate_b200_step_host call on this handle did on its device -> host leg (bench bookkeeping): *leg = 0 the rows
  * were copied densely, 1 their non-zero 16-byte chunks crossed the link and the rows were rebuilt in the caller's buffers,
  * 2 only the 64-byte groups that differ from the previous call's rows crossed and were patched in (MATE_STEP_HOST_ROWS_KEPT);
- * *row_bytes_on_link = bytes of observation rows (and their bitmaps) that crossed the link in that call. */
+ * *row_bytes_on_link = bytes of observation rows (and their bitmaps) that crossed the link in that call (the teams with a
+ * NULL buffer contribute none). */
 int mate_b200_host_leg_info(const MateSim* sim, int32_t* leg, uint64_t* row_bytes_on_link);
 
 #ifdef __cplusplus

@@ -817,7 +817,7 @@ extern "C" int mate_b200_seed(MateSim* sim, const uint8_t* env_mask, uint64_t se
 
 extern "C" int mate_b200_reset(MateSim* sim, const uint8_t* env_mask, uint64_t seed, float* cam_obs,
                                float* tgt_obs, void* stream) {
-    if (!sim || !tgt_obs || (sim->cfg.num_cameras > 0 && !cam_obs)) return fail(MATE_EINVAL, "null argument");
+    if (!sim) return fail(MATE_EINVAL, "null argument");
     if (int rc = check_obs_alignment(cam_obs, tgt_obs)) return rc;
     CUDA_TRY(cudaSetDevice(sim->device));
     sim->seed = seed;
@@ -834,8 +834,8 @@ extern "C" int mate_b200_reset(MateSim* sim, const uint8_t* env_mask, uint64_t s
 extern "C" int mate_b200_step(MateSim* sim, const float* cam_act, const float* tgt_act, float* cam_obs,
                               float* tgt_obs, float* rewards, uint8_t* done, const MateStepAux* aux,
                               const MateReplay* replay, uint32_t flags, void* stream) {
-    if (!sim || !tgt_act || !tgt_obs || !rewards || !done) return fail(MATE_EINVAL, "null argument");
-    if (sim->cfg.num_cameras > 0 && (!cam_act || !cam_obs)) return fail(MATE_EINVAL, "null camera buffers");
+    if (!sim || !tgt_act || !rewards || !done) return fail(MATE_EINVAL, "null argument");
+    if (sim->cfg.num_cameras > 0 && !cam_act) return fail(MATE_EINVAL, "null camera actions");
     if (int rc = check_obs_alignment(cam_obs, tgt_obs)) return rc;
     if (((uintptr_t)cam_act & 7) || ((uintptr_t)tgt_act & 7) || ((uintptr_t)rewards & 7)) return fail(MATE_EINVAL, "action/reward buffers must be 8-byte aligned");
     if (int rc = check_aux_alignment(aux)) return rc;
@@ -851,7 +851,7 @@ extern "C" int mate_b200_step(MateSim* sim, const float* cam_act, const float* t
 
 extern "C" int mate_b200_observe(MateSim* sim, float* cam_obs, float* tgt_obs, const MateStepAux* aux,
                                  const MateReplay* replay, void* stream) {
-    if (!sim || !tgt_obs || (sim->cfg.num_cameras > 0 && !cam_obs)) return fail(MATE_EINVAL, "null argument");
+    if (!sim) return fail(MATE_EINVAL, "null argument");
     if (int rc = check_obs_alignment(cam_obs, tgt_obs)) return rc;
     if (int rc = check_aux_alignment(aux)) return rc;
     CUDA_TRY(cudaSetDevice(sim->device));
@@ -954,12 +954,12 @@ static int dense_leg(MateSim* sim, const Params& p, int chunk, const float* cam_
         const int count = std::min(chunk, B - begin);
         cudaStream_t s = sim->hstreams[k % MateSim::kHostStreams];
         if (int rc = step_chunk(sim, p, cam_act, tgt_act, begin, count, s)) return rc;
-        if (sim->cfg.num_cameras) CUDA_TRY(cudaMemcpyAsync(env_rows(sim, cam_obs, 0, begin), env_rows(sim, p.cam_obs, 0, begin), count * env_row_bytes(sim, 0), cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(cudaMemcpyAsync(env_rows(sim, tgt_obs, 1, begin), env_rows(sim, p.tgt_obs, 1, begin), count * env_row_bytes(sim, 1), cudaMemcpyDeviceToHost, s));
+        if (sim->cfg.num_cameras && cam_obs) CUDA_TRY(cudaMemcpyAsync(env_rows(sim, cam_obs, 0, begin), env_rows(sim, p.cam_obs, 0, begin), count * env_row_bytes(sim, 0), cudaMemcpyDeviceToHost, s));
+        if (tgt_obs) CUDA_TRY(cudaMemcpyAsync(env_rows(sim, tgt_obs, 1, begin), env_rows(sim, p.tgt_obs, 1, begin), count * env_row_bytes(sim, 1), cudaMemcpyDeviceToHost, s));
         if (int rc = copy_rewards_done(sim, rewards, done, begin, count, s)) return rc;
     }
     for (int i = 0; i < MateSim::kHostStreams; ++i) CUDA_TRY(cudaStreamSynchronize(sim->hstreams[i]));
-    sim->last_leg = 0; sim->last_link_bytes = (unsigned long long)B * (env_row_bytes(sim, 0) + env_row_bytes(sim, 1));
+    sim->last_leg = 0; sim->last_link_bytes = (unsigned long long)B * ((cam_obs ? env_row_bytes(sim, 0) : 0) + (tgt_obs ? env_row_bytes(sim, 1) : 0));
     return MATE_OK;
 }
 
@@ -974,8 +974,9 @@ static int compact_leg(MateSim* sim, const Params& p, int chunk, bool delta, con
     double t_enq = 0, t_counts = 0, t_last_stream = 0;
     const int B = sim->num_envs;
     const int num_chunks = (B + chunk - 1) / chunk;
-    const size_t per_env[2] = {env_row_bytes(sim, 0), env_row_bytes(sim, 1)};
     float* const host_rows[2] = {cam_obs, tgt_obs};
+    // a team without a buffer is a region of no rows: no compaction, no table, no stream, no expansion
+    const size_t per_env[2] = {cam_obs ? env_row_bytes(sim, 0) : 0, tgt_obs ? env_row_bytes(sim, 1) : 0};
     const float* const dev_rows[2] = {p.cam_obs, p.tgt_obs};
     std::vector<long long> table_base(2 * (num_chunks + 1), 0);
     CUDA_TRY(cudaMemsetAsync(sim->d_count, 0, sizeof(unsigned int) * MateSim::kMaxHostChunks * 2, sim->hstreams[0]));
@@ -998,8 +999,8 @@ static int compact_leg(MateSim* sim, const Params& p, int chunk, bool delta, con
                                                                    nchunks, sim->d_compact[r] + first, table, sim->d_count + 2 * kc + r);
             else compact_chunks_kernel<<<1184, 128, 0, s>>>(reinterpret_cast<const uint4*>(dev_rows[r]) + first, nchunks,
                                                             sim->d_compact[r] + first, table, sim->d_count + 2 * kc + r);
+            sim->launches += 1;
         }
-        sim->launches += (sim->cfg.num_cameras ? 2 : 1);
         // The sizes of the chunk's compact streams go to the host by a store into pinned memory, not by a copy: a copy
         // would queue behind the compact streams of earlier chunks on the copy engine, and the next stream could only be
         // enqueued after the previous one had crossed the link (a bubble per chunk).
@@ -1063,9 +1064,9 @@ static int compact_leg(MateSim* sim, const Params& p, int chunk, bool delta, con
 
 extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const float* tgt_act, float* cam_obs,
                                    float* tgt_obs, float* rewards, uint8_t* done, uint32_t flags) {
-    if (!sim || !tgt_act || !tgt_obs || !rewards || !done) return fail(MATE_EINVAL, "null argument");
+    if (!sim || !tgt_act || !rewards || !done) return fail(MATE_EINVAL, "null argument");
     const int nc = sim->cfg.num_cameras;
-    if (nc > 0 && (!cam_act || !cam_obs)) return fail(MATE_EINVAL, "null camera buffers");
+    if (nc > 0 && !cam_act) return fail(MATE_EINVAL, "null camera actions");
     CUDA_TRY(cudaSetDevice(sim->device));
     sim->rows_written = true;
     if (int rc = ensure_host_path(sim)) return rc;
@@ -1080,7 +1081,8 @@ extern "C" int mate_b200_step_host(MateSim* sim, const float* cam_act, const flo
     const bool two_buffers = sim->compact_mode && sim->h_rows2[1] != nullptr && (nc == 0 || sim->h_rows2[0] != nullptr);
     float* const rows_now[2] = {two_buffers && sim->row_parity ? sim->h_rows2[0] : sim->h_cam_obs, two_buffers && sim->row_parity ? sim->h_rows2[1] : sim->h_tgt_obs};
     float* const rows_before[2] = {two_buffers && !sim->row_parity ? sim->h_rows2[0] : sim->h_cam_obs, two_buffers && !sim->row_parity ? sim->h_rows2[1] : sim->h_tgt_obs};
-    p.cam_act = sim->h_cam_act; p.tgt_act = sim->h_tgt_act; p.cam_obs = rows_now[0]; p.tgt_obs = rows_now[1];
+    // a team without a host buffer has no rows composed on the device either
+    p.cam_act = sim->h_cam_act; p.tgt_act = sim->h_tgt_act; p.cam_obs = cam_obs ? rows_now[0] : nullptr; p.tgt_obs = tgt_obs ? rows_now[1] : nullptr;
     p.rewards = sim->h_rewards; p.done = sim->h_done;
     fill_aux(p, nullptr, nullptr);
     // work queued earlier on the legacy default stream (torch's default) or on blocking streams is finished first;

@@ -81,20 +81,21 @@ struct Shape2 {
     // apart are 4-way bank conflicts.  Observer rows are therefore grouped by the ALIGNMENT of their obstacle block
     // (16 bytes / 8 bytes / odd) into rounds of 32 / NO rows, and a round stores with the widest aligned type
     // (1, 2 or 3 instructions instead of 4) -- unless the grouping needs more than one round more than plain row order.
+    // Only the observer rows [r0, r1) that the launch composes take part.
     struct ORounds { int n; int grouped; int row[40][4]; int cls[40]; };   // cls: 0 = 16-byte aligned, 2 = 8-byte, 1 = odd, -1 = mixed (scalar stores)
     __host__ __device__ static constexpr int o_offset(int row) {
         return (row < NC ? row * (DC + CAM_SKEW) : STAGE_CAM + (row - NC) * DT) + ObsLayout{NC, NT, NO}.block(row < NC, KIND_OBSTACLE);
     }
-    __host__ __device__ static constexpr ORounds make_orounds() {
+    __host__ __device__ static constexpr ORounds make_orounds(const int r0, const int r1) {
         ORounds r{};
-        const int rpr = NO > 0 ? 32 / NO : 1, plain = (R + rpr - 1) / rpr;
+        const int rpr = NO > 0 ? 32 / NO : 1, plain = (r1 - r0 + rpr - 1) / rpr;
         for (int i = 0; i < 40; ++i) { r.cls[i] = -1; for (int j = 0; j < 4; ++j) r.row[i][j] = -1; }
         if (NO == 0) { r.n = 0; return r; }
         const int order[3] = {0, 2, 1};
         int n = 0;
         for (int k = 0; k < 3; ++k) {
             int fill = 0;
-            for (int row = 0; row < R; ++row) {
+            for (int row = r0; row < r1; ++row) {
                 const int al = o_offset(row) & 3, cls = al == 0 ? 0 : (al == 2 ? 2 : 1);
                 if (cls != order[k]) continue;
                 if (fill == 0) r.cls[n] = cls;
@@ -105,7 +106,7 @@ struct Shape2 {
         }
         if (n <= plain + 1) { r.n = n; r.grouped = 1; return r; }
         for (int i = 0; i < 40; ++i) { r.cls[i] = -1; for (int j = 0; j < 4; ++j) r.row[i][j] = -1; }
-        for (int row = 0; row < R; ++row) r.row[row / rpr][row % rpr] = row;
+        for (int row = r0; row < r1; ++row) r.row[(row - r0) / rpr][(row - r0) % rpr] = row;
         r.n = plain;
         return r;
     }
@@ -675,17 +676,28 @@ __device__ __forceinline__ void store_team_rows(OutT* dst, const float* src) {
     }
 }
 
+// The observer rows a launch composes and stores: the camera rows [0, NC), the target rows [NC, NC + NT) or both
+// (a NULL row pointer of the call drops its team, DESIGN.md section 7j)
+enum : int { ROWS_CAM = 1, ROWS_TGT = 2, ROWS_BOTH = 3 };
+
 // FOLD = the instantiation that also applies the registered observation wrappers (FoldOps, mate_common.cuh) while
 // the rows are composed; the common case (no wrappers) runs the FOLD = false instantiation, which has none of it.
 // OutT = element type of the rows in HBM (Params::obs_format): float, or __half rounded once from the staged fp32 rows
 // while they leave the SM.  Everything before the copy-out is the same for both.
-template <int NC, int NT, int NO, bool FOLD, class OutT>
-__device__ __noinline__ void pack_observations(const Params& p, const int env0, const int nvalid, float* stage,
-                                               const uint32_t* mk, const float* val, float* ops_scratch) {
+// ROWS = the observer rows composed (ROWS_*): a row outside the set gets no pair scatter, no own-row block and no
+// store, and the rounds of the scatter cover only the rows inside it.  The wrappers outside the canonical form
+// (fold_obs_ops) still run over the whole staged block; EnhancedObservation copies entity states from the own-row
+// blocks of the other team, so on that path the own-row blocks of every row are composed.
+template <int NC, int NT, int NO, bool FOLD, class OutT, int ROWS>
+__device__ __noinline__ void pack_rows(const Params& p, const int env0, const int nvalid, float* stage,
+                                       const uint32_t* mk, const float* val, float* ops_scratch) {
     using S = Shape2<NC, NT, NO>;
     constexpr bool F16 = std::is_same<OutT, __half>::value;
     static_assert(F16 || std::is_same<OutT, float>::value, "observation rows are float or __half");
+    static_assert(ROWS == ROWS_BOTH || ((ROWS == ROWS_CAM || ROWS == ROWS_TGT) && NC > 0), "a single team's rows need cameras");
     constexpr int R = S::R, MW = S::MW, DC = S::DC, DT = S::DT, CV = S::CV;
+    constexpr bool WANT_C = (ROWS & ROWS_CAM) != 0, WANT_T = (ROWS & ROWS_TGT) != 0;
+    constexpr int R0 = WANT_C ? 0 : NC, R1 = WANT_T ? R : NC;   // the composed rows [R0, R1)
     constexpr int NCX = NC > 0 ? NC : 1;
     constexpr uint32_t FULLMASK = 0xffffffffu;
     constexpr ObsLayout L{NC, NT, NO};
@@ -723,8 +735,9 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     constexpr int T_TGT = L.block(false, KIND_TARGET), T_OBS = L.block(false, KIND_OBSTACLE), T_CAM = L.block(false, KIND_CAMERA);
     constexpr int NOX = NO > 0 ? NO : 1;
     constexpr int RPR_T = 32 / NT, RPR_O = 32 / NOX, RPR_C = 32 / NCX;          // observer rows per round
-    constexpr typename S::ORounds ORND = S::make_orounds();
-    constexpr int RND_T = (R + RPR_T - 1) / RPR_T, RND_O = NO > 0 ? ORND.n : 1, RND_C = (R + RPR_C - 1) / RPR_C;
+    constexpr typename S::ORounds ORND = S::make_orounds(R0, R1);
+    constexpr int RW = R1 - R0;
+    constexpr int RND_T = (RW + RPR_T - 1) / RPR_T, RND_O = NO > 0 ? ORND.n : 1, RND_C = (RW + RPR_C - 1) / RPR_C;
     const float f_sr = (float)p.tgt_sight_range, f_crad = (float)p.cam_radius;
     const float f_rmax = (float)p.cam_rmax, f_rot = (float)p.cam_rot_step, f_zoom = (float)p.cam_zoom_step;
     const float f_step1 = (float)p.tgt_step_size, f_step2 = (float)(p.tgt_step_size / 2.0);
@@ -742,8 +755,8 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     uint32_t on_bits = 0; // bit rd: the lane has a pair in round rd
 #pragma unroll
     for (int rd = 0; rd < RND_T; ++rd) {
-        const int row = rd * RPR_T + t_sub;
-        const bool on = t_sub < RPR_T && row < R;
+        const int row = R0 + rd * RPR_T + t_sub;
+        const bool on = t_sub < RPR_T && row < R1;
         q_ptr[rd] = stage + (on ? row_base(row) + (row < NC ? C_TGT : T_TGT) + ObsLayout::TGT_ENTRY * t_idx : 0);
         m_idx[rd] = on ? row * MW : 0;
         on_bits |= (uint32_t)on << rd;
@@ -751,8 +764,8 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     if (NO > 0) {
 #pragma unroll
         for (int rd = 0; rd < RND_O; ++rd) {
-            int row = rd * RPR_O + o_sub;
-            bool on = o_sub < RPR_O && row < R;
+            int row = R0 + rd * RPR_O + o_sub;
+            bool on = o_sub < RPR_O && row < R1;
             if (ORND.grouped) {
                 row = -1;
 #pragma unroll
@@ -767,8 +780,8 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     if (NC > 0) {
 #pragma unroll
         for (int rd = 0; rd < RND_C; ++rd) {
-            const int row = rd * RPR_C + c_sub;
-            const bool on = c_sub < RPR_C && row < R;
+            const int row = R0 + rd * RPR_C + c_sub;
+            const bool on = c_sub < RPR_C && row < R1;
             q_ptr[NRND - RND_C + rd] = stage + (on ? row_base(row) + (row < NC ? C_CAM : T_CAM) + ObsLayout::CAM_ENTRY * c_idx : 0);
             m_idx[NRND - RND_C + rd] = on ? row * MW : 0;
             on_bits |= (uint32_t)on << (NRND - RND_C + rd);
@@ -783,7 +796,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
     // (with RescaledObservation folded in, the constants are staged already rescaled; RelativeCoordinates rewrites the
     //  eight warehouse coordinates of a row for every environment, everything else here stays)
     auto stage_constants = [&]() {
-        if (lane < R) {
+        if (lane < R && (ROWS == ROWS_BOTH || has_ops || (lane >= R0 && lane < R1))) {
             const int row = lane;
             float* q = stage + row_base(row);
             auto put = [&](const int col, const float x, const int aff) { q[col] = (FOLD && f_resc) ? fmaf(x, aff_own[aff].x, aff_own[aff].y) : x; };
@@ -1068,7 +1081,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
             // c_idx (NC consecutive lanes hold NC different cameras) -- one instruction stream for both kinds of rows.
             // With wrappers folded in: RescaledObservation is one FMA per entry, RelativeCoordinates moves the eight
             // warehouse coordinates of the row (the agent's own location stays absolute, mate/constants.py:372-427)
-            const bool is_t = lane < NT, is_c = NC > 0 && lane >= NT && lane < NT + NC;
+            const bool is_t = lane < NT && (WANT_T || has_ops), is_c = NC > 0 && lane >= NT && lane < NT + NC && (WANT_C || has_ops);
             float* const q = is_t ? self_t : self_c;
             const int aff0 = is_t ? ObsLayout::AFF_TSELF : ObsLayout::AFF_CSELF;
             auto put = [&](const int j, const float x) { q[j] = (FOLD && f_resc) ? fmaf(x, aff_own[aff0 + j].x, aff_own[aff0 + j].y) : x; };
@@ -1102,7 +1115,7 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
         // ---- staged rows -> HBM
         static_assert(!(S::DENSE16 && S::CAM_SKEW != 0), "the 16-byte copy of the whole block expects dense camera rows");
         __syncwarp();
-        if constexpr (!F16 && S::DENSE16) {
+        if constexpr (ROWS == ROWS_BOTH && !F16 && S::DENSE16) {
             // plain 16-byte copies of the whole block: every warp store covers 512 contiguous bytes; unlike a bulk copy
             // there is nothing to wait for before the block is reused (see DESIGN.md)
             const float4* src4 = reinterpret_cast<const float4*>(stage);
@@ -1119,10 +1132,24 @@ __device__ __noinline__ void pack_observations(const Params& p, const int env0, 
                 }
             }
         } else {
-            store_team_rows<OutT, S::CAM_ROW, DC, DCS - DC>(cam_obs0 + (size_t)i * S::CAM_ROW, stage);
-            store_team_rows<OutT, S::TGT_ROW, DT, 0>(tgt_obs0 + (size_t)i * S::TGT_ROW, stage + S::STAGE_CAM);
+            if constexpr (WANT_C) store_team_rows<OutT, S::CAM_ROW, DC, DCS - DC>(cam_obs0 + (size_t)i * S::CAM_ROW, stage);
+            if constexpr (WANT_T) store_team_rows<OutT, S::TGT_ROW, DT, 0>(tgt_obs0 + (size_t)i * S::TGT_ROW, stage + S::STAGE_CAM);
         }
         __syncwarp();
+    }
+}
+
+// joint_observation for the rows the launch's pointers ask for (without cameras, "targets only" is "both"); no pointer:
+// nothing.  Each row set is an instantiation of its own, so the step kernel keeps one call per (FOLD, OutT) and the
+// both-teams packer its code (ptxas allocates registers across the calls of a kernel).
+template <int NC, int NT, int NO, bool FOLD, class OutT>
+__device__ __noinline__ void pack_observations(const Params& p, const int env0, const int nvalid, float* stage,
+                                               const uint32_t* mk, const float* val, float* ops_scratch) {
+    const bool want_c = NC > 0 && p.cam_obs != nullptr, want_t = p.tgt_obs != nullptr;
+    if (want_t && (want_c || NC == 0)) pack_rows<NC, NT, NO, FOLD, OutT, ROWS_BOTH>(p, env0, nvalid, stage, mk, val, ops_scratch);
+    else if constexpr (NC > 0) {
+        if (want_c) pack_rows<NC, NT, NO, FOLD, OutT, ROWS_CAM>(p, env0, nvalid, stage, mk, val, ops_scratch);
+        else if (want_t) pack_rows<NC, NT, NO, FOLD, OutT, ROWS_TGT>(p, env0, nvalid, stage, mk, val, ops_scratch);
     }
 }
 

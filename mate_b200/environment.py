@@ -33,7 +33,7 @@ from mate_b200 import spaces
 from mate_b200.config import DEFAULT_CONFIG_FILE, flatten_config, read_config
 from mate_b200.entities import CameraView, ObstacleView, TargetView
 from mate_b200.messages import Message, Team
-from mate_b200.sim import BatchedSim, check_observation_dtype
+from mate_b200.sim import BatchedSim, check_observation_dtype, check_observed_team
 
 __all__ = ['MultiAgentTracking', 'EnvMeta', 'Message', 'Team', 'read_config', 'DEFAULT_CONFIG_FILE']
 
@@ -67,23 +67,33 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
 
     def __init__(self, config: Optional[Union[Dict[str, Any], str]] = None, num_envs: Optional[int] = None,
                  device: Union[int, str, torch.device] = 0, env_index_base: int = 0,
-                 observation_dtype: torch.dtype = torch.float32, **kwargs) -> None:
+                 observation_dtype: torch.dtype = torch.float32, observed_team: str = 'both', **kwargs) -> None:
         # observation_dtype: element type of the batched observation tensors, torch.float32 or torch.float16 (the float32
         # rows rounded once to nearest even); the observation spaces keep describing the reference's float64 Boxes
         check_observation_dtype(observation_dtype)
         if num_envs is None and observation_dtype != torch.float32:
             raise ValueError('observation_dtype applies to the batched mode (num_envs=B); the single-environment mode '
                              'returns the float64 NumPy observations of the reference')
+        # observed_team: whose observation rows the simulator composes ('both', 'camera' or 'target'); the joint
+        # observations carry None in the other team's slot (one team learning against built-in agents)
+        check_observed_team(observed_team)
+        if num_envs is None and observed_team != 'both':
+            raise ValueError("observed_team applies to the batched mode (num_envs=B); the single-environment mode "
+                             "observes both teams")
         if config is None:
             config = {} if len(kwargs) > 0 else self.DEFAULT_CONFIG_FILE   # environment.py:338-339
-        self._init_args = (config, num_envs, device, env_index_base, dict(kwargs), observation_dtype)
+        self._init_args = (config, num_envs, device, env_index_base, dict(kwargs), observation_dtype, observed_team)
         self.config = read_config(config, **kwargs)
         self.flat_config = flatten_config(self.config)
+        check_observed_team(observed_team, self.flat_config['num_cameras'])
         self.batched = num_envs is not None
         self.num_envs = int(num_envs) if self.batched else 1
         self.observation_dtype = observation_dtype
-        # the default is not passed on: simulator classes substituted for BatchedSim need not know the argument
+        self.observed_team = observed_team
+        # the defaults are not passed on: simulator classes substituted for BatchedSim need not know the arguments
         sim_kwargs = {} if observation_dtype == torch.float32 else {'observation_dtype': observation_dtype}
+        if observed_team != 'both':
+            sim_kwargs['observed_team'] = observed_team
         self.sim = self._sim_class(self.flat_config, self.num_envs, device=device, env_index_base=env_index_base, **sim_kwargs)
         self.device = self.sim.device
         nc, nt, no = self.num_cameras, self.num_targets, self.num_obstacles
@@ -208,10 +218,10 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
     def load_config(self, config=None) -> None:
         """Re-initialise from another configuration, keeping wrappers (environment.py:564-588)."""
         seed = int(self._np_random.randint(2 ** 31 - 1))
-        _, num_envs, device, base, _, observation_dtype = self._init_args
+        _, num_envs, device, base, _, observation_dtype, observed_team = self._init_args
         self.sim.close()
         self.__init__(config=config, num_envs=num_envs, device=device, env_index_base=base,  # pylint: disable=unnecessary-dunder-call
-                      observation_dtype=observation_dtype)
+                      observation_dtype=observation_dtype, observed_team=observed_team)
         self.seed(seed)
 
     def reset(self, *, seed: Optional[int] = None):
@@ -427,7 +437,8 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         self.render_callbacks[name] = callback
 
     def joint_observation(self):
-        """Joint observations of both teams for the current state (environment.py:908-983)."""
+        """Joint observations of both teams for the current state (environment.py:908-983); ``None`` for a team that is
+        not observed (``observed_team``)."""
         cam_obs, tgt_obs = self.sim.observe(aux=True)
         return self._format_obs(cam_obs, tgt_obs)
 

@@ -57,6 +57,19 @@ def check_observation_dtype(dtype):
     return dtype
 
 
+OBSERVED_TEAMS = ('both', 'camera', 'target')
+
+
+def check_observed_team(team, num_cameras=None):
+    """Whose observation rows a batched simulator composes and writes: ``'both'``, ``'camera'`` or ``'target'``, else
+    ``ValueError``; ``'camera'`` also needs cameras (``num_cameras``, when given)."""
+    if not isinstance(team, str) or team not in OBSERVED_TEAMS:
+        raise ValueError(f'observed_team must be one of {OBSERVED_TEAMS}, got {team!r}')
+    if team == 'camera' and num_cameras == 0:
+        raise ValueError("observed_team='camera' needs a configuration with cameras")
+    return team
+
+
 class StateSnapshot:
     """The complete state of some environments of a batch, saved on the device (:meth:`BatchedSim.save_state`).
 
@@ -87,10 +100,13 @@ torch.serialization.add_safe_globals([StateSnapshot])   # torch.load(weights_onl
 
 class BatchedSim:
     """One batch of MultiAgentTracking environments resident on one GPU.  ``observation_dtype`` is the element type of
-    the observation rows (``cam_obs`` / ``tgt_obs``); everything else stays float32."""
+    the observation rows (``cam_obs`` / ``tgt_obs``); everything else stays float32.  ``observed_team`` (``'both'``,
+    ``'camera'`` or ``'target'``) is whose rows are composed and written: the other team's tensor is ``None`` and its
+    rows cost nothing; everything else is what a ``'both'`` simulator computes."""
 
-    def __init__(self, flat_config, num_envs, device=0, env_index_base=0, observation_dtype=torch.float32):
+    def __init__(self, flat_config, num_envs, device=0, env_index_base=0, observation_dtype=torch.float32, observed_team='both'):
         self.observation_dtype = check_observation_dtype(observation_dtype)
+        self.observed_team = check_observed_team(observed_team, int(dict(flat_config)['num_cameras']))
         if not torch.cuda.is_available():
             raise RuntimeError('mate_b200 needs a CUDA device (there is no CPU fallback)')
         self.lib = _abi.load_library()
@@ -110,8 +126,9 @@ class BatchedSim:
         _check(self.lib, self.lib.mate_b200_obs_dims(self.handle, ctypes.byref(dc), ctypes.byref(dt)))
         self.dc, self.dt = dc.value, dt.value
         dev = self.device
-        self.cam_obs = torch.zeros((self.B, self.nc, self.dc), dtype=self.observation_dtype, device=dev)
-        self.tgt_obs = torch.zeros((self.B, self.nt, self.dt), dtype=self.observation_dtype, device=dev)
+        self.cam_obs, self.tgt_obs = (
+            torch.zeros(shape, dtype=self.observation_dtype, device=dev) if self.observed_team in ('both', team) else None
+            for team, shape in (('camera', (self.B, self.nc, self.dc)), ('target', (self.B, self.nt, self.dt))))
         self.rewards = torch.zeros((self.B, 2), dtype=torch.float32, device=dev)
         self.done = torch.zeros((self.B,), dtype=torch.uint8, device=dev)
         self._stats = torch.zeros(16, dtype=torch.float32, device=dev)
@@ -205,6 +222,9 @@ class BatchedSim:
         the wrappers registered (those are transformed already)."""
         if not self._obs_ops:
             return
+        if self.tgt_obs is None or (self.nc and self.cam_obs is None):
+            raise ValueError(f"transform_observations needs both teams' rows; this simulator observes {self.observed_team!r} only "
+                             '(register the wrappers with set_observation_wrappers instead)')
         cam_aff, tgt_aff = self._affine if self._affine is not None else (None, None)
         with torch.cuda.device(self.device):
             _check(self.lib, self.lib.mate_b200_transform_observations(
@@ -381,9 +401,14 @@ class BatchedSim:
         rewards, done) are CPU tensors (pinned for full PCIe speed).  `rows_kept=True` promises that
         `out` is the tuple of the previous `step_host` call and has not been written to since
         (MATE_STEP_HOST_ROWS_KEPT, include/mate_b200.h): parts of the rows that stay zero are then not rewritten.
-        cam_obs / tgt_obs have the simulator's ``observation_dtype``."""
+        cam_obs / tgt_obs have the simulator's ``observation_dtype``; the slot of a team that is not observed is ``None``."""
         cam_obs, tgt_obs, rewards, done = out
-        for name, rows in (('cam_obs', cam_obs if self.nc else None), ('tgt_obs', tgt_obs)):
+        for name, rows, observed in (('cam_obs', cam_obs if self.nc else None, self.cam_obs is not None),
+                                     ('tgt_obs', tgt_obs, self.tgt_obs is not None)):
+            if observed and rows is None and (name == 'tgt_obs' or self.nc):
+                raise ValueError(f'step_host: {name} is None, but this simulator observes {self.observed_team!r}')
+            if not observed and rows is not None:
+                raise ValueError(f'step_host: {name} must be None, this simulator observes {self.observed_team!r} only')
             if rows is not None and rows.dtype != self.observation_dtype:   # the C call sees only a pointer
                 raise ValueError(f'step_host: {name} is {rows.dtype}, the simulator writes {self.observation_dtype} rows')
         flags = (_abi.MATE_STEP_AUTO_RESET if auto_reset else 0) | (_abi.MATE_STEP_HOST_ROWS_KEPT if rows_kept else 0)

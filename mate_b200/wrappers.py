@@ -340,9 +340,11 @@ class MoreTrainingInformation(Wrapper):
             'target_camera_view_mask': aux['mask_tc'].bool(), 'target_obstacle_view_mask': aux['mask_to'].bool(),
             'target_target_view_mask': aux['mask_tt'].bool(),
         }
-        if base.batched:
-            shared['camera_states'] = camera_joint_observation[..., cam_self]
-            shared['target_states'] = target_joint_observation[..., tgt_self]
+        if base.batched:   # a team that is not observed (observed_team) has no rows to take its states from
+            if camera_joint_observation is not None:
+                shared['camera_states'] = camera_joint_observation[..., cam_self]
+            if target_joint_observation is not None:
+                shared['target_states'] = target_joint_observation[..., tgt_self]
         else:
             shared = {k: v[0].cpu().numpy() for k, v in shared.items()}
             shared['camera_states'] = np.array(camera_joint_observation[..., cam_self])
@@ -655,6 +657,9 @@ class MultiCamera(_SingleTeamSnapshot, Wrapper):
             f'You should provide an instance of target agent. Got target_agent = {target_agent!r}.')
         assert not _has_wrapper(env, MultiCamera), f'You should not use wrapper `{type(self)}` more than once.'
         assert env.num_cameras > 0, 'There must be at least one camera in the environment.'
+        if env.unwrapped.observed_team not in ('both', 'camera'):
+            raise ValueError(f'MultiCamera returns the camera rows, but this environment observes '
+                             f'{env.unwrapped.observed_team!r} only (use observed_team=\'camera\' or \'both\')')
         super().__init__(env)
         self.opponent_agent = target_agent
         self.num_teammates, self.num_opponents = env.num_cameras, env.num_targets
@@ -706,6 +711,12 @@ class MultiTarget(_SingleTeamSnapshot, Wrapper):
         assert not _has_wrapper(env, MultiTarget) and not _has_wrapper(env, MultiCamera), (
             f'You should not use wrapper `{type(self)}` with another single-team wrapper.')
         assert env.num_cameras > 0, 'There must be at least one camera in the environment.'
+        if env.unwrapped.observed_team != 'both':
+            # the learning targets need their own rows, and the greedy camera team reads its target flags from the camera
+            # rows (_tracked_flags): skipping those would need the flags as a separate output of the step kernel
+            raise ValueError(f'MultiTarget needs the target rows it returns and the camera rows: the greedy camera team '
+                             f'reads its target flags from them (_tracked_flags); this environment observes '
+                             f'{env.unwrapped.observed_team!r} only (use observed_team=\'both\')')
         super().__init__(env)
         self.opponent_agent = camera_agent
         self.num_teammates, self.num_opponents = env.num_targets, env.num_cameras
