@@ -319,6 +319,52 @@ int mate_b200_set_observation_ops(MateSim* sim, const int32_t* ops, int32_t num_
 int mate_b200_fov_range(MateSim* sim, const int32_t* env, const int32_t* camera, const double* angle_deg,
                         double* out, int64_t n, void* stream);
 
+/* rgb_array frames of chosen environments, drawn from the live state by a CUDA kernel (DESIGN.md section 7k).
+ * out: dev uint8 [count][size][size][3]; frame i is environment env[i] (dev int32 [count]; NULL = every environment,
+ * which requires count == num_envs).  An entry of env outside [0, num_envs) leaves frame i unwritten.  The call only
+ * enqueues work on `stream`: it never synchronises, changes nothing in the handle and reads the state as it is, like
+ * mate_b200_fov_range.  MATE_EINVAL, nothing launched, for a NULL sim or out, count <= 0, a NULL env with count !=
+ * num_envs, or a size outside [MATE_RENDER_MIN_SIZE, MATE_RENDER_MAX_SIZE].
+ *
+ * The picture.  Row 0 is the top (y = +V), column 0 the left (x = -V), V = MATE_RENDER_HALF_EXTENT.  Pixel (i, j) is
+ * decided at its centre x_j = ((2j + 1 - S) V) / S, y_i = ((S - 2i - 1) V) / S (fp64: one exact product, one correctly
+ * rounded division); the pixel pitch is p = 2V / S.  Colours are 0xRRGGBB, stored as the bytes R, G, B.  Layers, in order:
+ *   1. MATE_RENDER_TERRAIN where |x| <= 1000 and |y| <= 1000, else MATE_RENDER_OUTSIDE;
+ *   2. warehouse w (centre MATE_RENDER_WAREHOUSE_CENTER * (+-1, +-1) in the order (+,+), (-,+), (-,-), (+,-)) where
+ *      max(|x - wx|, |y - wy|) <= MATE_RENDER_WAREHOUSE_HALF_SIZE, colour MATE_RENDER_WAREHOUSE_<w>;
+ *   3. with k the number of cameras that would see a target at the pixel centre (Camera.perceive with a transmission draw
+ *      of 0: the step's range + sector test and its occlusion test dist <= sight_range_at(bearing) * (1 + 1e-6)),
+ *      MATE_RENDER_FOV blended k times: dst = (dst * (255 - a) + src * a + 127) / 255 per channel, a = MATE_RENDER_FOV_ALPHA;
+ *   4. MATE_RENDER_OBSTACLE where dx^2 + dy^2 <= r^2;
+ *   5. MATE_RENDER_CAMERA where dx^2 + dy^2 <= camera_radius^2;
+ *   6. targets in index order, with r_in = max(MATE_RENDER_TARGET_INNER, MATE_RENDER_TARGET_INNER_PITCH * p) and r_out =
+ *      max(MATE_RENDER_TARGET_OUTER, MATE_RENDER_TARGET_OUTER_PITCH * p): d^2 <= r_in^2 gets the colour of the goal
+ *      warehouse if the target is loaded (goal >= 0 and weight > 0), else MATE_RENDER_TARGET_EMPTY; r_in^2 < d^2 <= r_out^2
+ *      gets MATE_RENDER_TRACKED if some camera sees the target's location by the predicate of layer 3.
+ * Layers 2, 4, 5 and 6 compute in fp64 without fused multiply-add.  A frame is a function of its environment's state. */
+#define MATE_RENDER_MIN_SIZE 16
+#define MATE_RENDER_MAX_SIZE 4096
+#define MATE_RENDER_HALF_EXTENT 1050.0          /* 1.05 * terrain size */
+#define MATE_RENDER_WAREHOUSE_CENTER 925.0
+#define MATE_RENDER_WAREHOUSE_HALF_SIZE 75.0
+#define MATE_RENDER_FOV_ALPHA 64
+#define MATE_RENDER_TARGET_INNER 12.0
+#define MATE_RENDER_TARGET_INNER_PITCH 1.25
+#define MATE_RENDER_TARGET_OUTER 22.0
+#define MATE_RENDER_TARGET_OUTER_PITCH 2.25
+#define MATE_RENDER_TERRAIN 0xF4F4F4u
+#define MATE_RENDER_OUTSIDE 0x404040u
+#define MATE_RENDER_WAREHOUSE_0 0xE69F00u
+#define MATE_RENDER_WAREHOUSE_1 0x56B4E9u
+#define MATE_RENDER_WAREHOUSE_2 0x009E73u
+#define MATE_RENDER_WAREHOUSE_3 0xCC79A7u
+#define MATE_RENDER_FOV 0x0072B2u
+#define MATE_RENDER_OBSTACLE 0x808080u
+#define MATE_RENDER_CAMERA 0x003E7Du
+#define MATE_RENDER_TRACKED 0xD55E00u
+#define MATE_RENDER_TARGET_EMPTY 0x202020u
+int mate_b200_render(MateSim* sim, const int32_t* env, int32_t count, int32_t size, uint8_t* out, void* stream);
+
 /* Per-agent terms of the reference's auxiliary-reward and training-information wrappers (SURVEY.md section
  * 8f, N3) from the auxiliary outputs of the LAST step (so they describe the finished step even where the
  * environment was auto-reset), one pass, no host round trip:

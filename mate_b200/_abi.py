@@ -232,6 +232,7 @@ def load_library():
     lib.mate_b200_set_observation_ops.argtypes = [void_p, c_int32_p, ctypes.c_int32, void_p, void_p]
     lib.mate_b200_decode_actions.argtypes = [void_p, void_p, ctypes.c_int32, void_p, ctypes.c_int64, void_p]
     lib.mate_b200_fov_range.argtypes = [void_p, void_p, void_p, void_p, void_p, ctypes.c_int64, void_p]
+    lib.mate_b200_render.argtypes = [void_p, void_p, ctypes.c_int32, ctypes.c_int32, void_p, void_p]
     lib.mate_b200_auxiliary_terms.argtypes = [void_p, ctypes.POINTER(MateStepAux), void_p, void_p, void_p, void_p, void_p]
     lib.mate_b200_greedy_target_actions.argtypes = [void_p, void_p, void_p, ctypes.c_double, ctypes.c_uint64, ctypes.c_uint64,
                                                     ctypes.POINTER(MateAgentReplay), void_p, void_p]
@@ -242,7 +243,7 @@ def load_library():
     lib.mate_b200_exchange_messages.argtypes = [void_p, ctypes.POINTER(MateMessageExchange), ctypes.c_uint64, void_p]
     for name in ('create', 'destroy', 'obs_dims', 'set_observation_format', 'reset', 'seed', 'step', 'observe', 'step_host',
                  'get_state', 'set_state', 'snapshot_bytes', 'save_state', 'load_state', 'episode_stats', 'transform_observations', 'set_observation_ops', 'decode_actions', 'auxiliary_terms', 'fov_range', 'soft_coverage', 'greedy_target_actions', 'greedy_camera_actions', 'set_message_filter',
-                 'exchange_messages'):
+                 'exchange_messages', 'render'):
         getattr(lib, 'mate_b200_' + name).restype = ctypes.c_int
     _LIB = lib
     return lib
@@ -255,10 +256,11 @@ EXPORTED_SYMBOLS = [
     'mate_b200_load_state',
     'mate_b200_episode_stats', 'mate_b200_launch_count', 'mate_b200_host_leg_info', 'mate_b200_transform_observations', 'mate_b200_set_observation_ops',
     'mate_b200_decode_actions', 'mate_b200_auxiliary_terms', 'mate_b200_fov_range', 'mate_b200_soft_coverage', 'mate_b200_greedy_target_actions', 'mate_b200_greedy_camera_actions',
-    'mate_b200_set_message_filter', 'mate_b200_exchange_messages',
+    'mate_b200_set_message_filter', 'mate_b200_exchange_messages', 'mate_b200_render',
 ]
 
 # observation wrapper codes (include/mate_b200.h)
 OBS_ENHANCED_CAMERA, OBS_ENHANCED_TARGET, OBS_SHARED_CAMERA, OBS_SHARED_TARGET, OBS_RELATIVE, OBS_RESCALED = range(1, 7)
 MAX_OBS_OPS = 8
 CAM_TERMS, TGT_TERMS = 8, 16   # MATE_CAM_TERMS / MATE_TGT_TERMS
+RENDER_MIN_SIZE, RENDER_MAX_SIZE = 16, 4096   # MATE_RENDER_MIN_SIZE / MATE_RENDER_MAX_SIZE

@@ -22,6 +22,7 @@
 #include "mate_hostpath.cuh"
 #include "mate_snapshot.cuh"
 #include "mate_messages.cuh"
+#include "mate_render.cuh"
 
 using namespace mate;
 
@@ -59,6 +60,7 @@ struct KernelInfo {
     cudaError_t (*prepare)();
     void (*launch_fov)(const Params&, const int32_t*, const int32_t*, const double*, double*, long long, cudaStream_t);
     void (*launch_soft)(const Params&, const uint8_t*, const uint8_t*, double*, float*, cudaStream_t);
+    void (*launch_render)(const Params&, const int32_t*, int count, int size, uint8_t*, cudaStream_t);
 };
 
 // ---- L2 persistence for the fp32 obstacle entries -------------------------------------------------
@@ -143,6 +145,13 @@ static void launch_soft_shape(const Params& p, const uint8_t* mask_ct, const uin
     soft_coverage_kernel<NC, NT, NO><<<(unsigned)((warps + 3) / 4), 128, 0, stream>>>(p, mask_ct, done, edges, out);
 }
 template <int NC, int NT, int NO>
+static void launch_render_shape(const Params& p, const int32_t* env, int count, int size, uint8_t* out, cudaStream_t stream) {
+    const int tiles = ((size + kRenderRows - 1) / kRenderRows) * ((size + kRenderCols - 1) / kRenderCols);
+    const int words = size % 4 == 0 && ((uintptr_t)out & 3) == 0;   // every 4-pixel group is 3 aligned words
+    render_kernel<NC, NT, NO><<<dim3((unsigned)tiles, (unsigned)std::min(count, 65535)), kRenderThreads, 0, stream>>>(
+        p, env, count, size, words, out);
+}
+template <int NC, int NT, int NO>
 static cudaError_t prepare_shape2() {
     using S = Shape2<NC, NT, NO>;
     return cudaFuncSetAttribute(mate_step_kernel2<NC, NT, NO>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -169,7 +178,7 @@ static bool find_kernel(int nc, int nt, int no, KernelInfo* out) {
         *out = KernelInfo{&launch_wrappers_shape<NC, NT, NO>, &prepare_wrappers_shape<NC, NT, NO>,       \
                           &launch_shape2<NC, NT, NO>, S::ENVS_PER_CTA, S::DC, S::DT,             \
                           &prepare_shape2<NC, NT, NO>, &launch_fov_shape<NC, NT, NO>,            \
-                          &launch_soft_shape<NC, NT, NO>};                                      \
+                          &launch_soft_shape<NC, NT, NO>, &launch_render_shape<NC, NT, NO>};    \
         return true;                                                                           \
     }
     MATE_SHAPES(X)
@@ -499,6 +508,17 @@ extern "C" int mate_b200_fov_range(MateSim* sim, const int32_t* env, const int32
     sim->kernel.launch_fov(sim->base, env, camera, angle_deg, out, n, (cudaStream_t)stream);
     sim->launches += 1;
     return check_launch("fov_range");
+}
+
+extern "C" int mate_b200_render(MateSim* sim, const int32_t* env, int32_t count, int32_t size, uint8_t* out, void* stream) {
+    if (!sim || !out) return fail(MATE_EINVAL, "null argument");
+    if (count <= 0) return fail(MATE_EINVAL, "count must be positive");
+    if (!env && count != sim->num_envs) return fail(MATE_EINVAL, "without an environment list every environment is rendered: count must be num_envs");
+    if (size < MATE_RENDER_MIN_SIZE || size > MATE_RENDER_MAX_SIZE) return fail(MATE_EINVAL, "size must lie in [MATE_RENDER_MIN_SIZE, MATE_RENDER_MAX_SIZE]");
+    CUDA_TRY(cudaSetDevice(sim->device));
+    sim->kernel.launch_render(sim->base, env, count, size, out, (cudaStream_t)stream);
+    sim->launches += 1;
+    return check_launch("render");
 }
 
 extern "C" int64_t mate_b200_launch_count(const MateSim* sim) { return sim ? sim->launches : 0; }

@@ -529,9 +529,11 @@ __device__ __forceinline__ double sight_range_quad(const ObsRef ob, double cx, d
 }
 
 // Camera.perceive (mate/entities.py:491-505) up to the stochastic draw, exact arithmetic of
-// the reference: returns 0 = not in range/sector, 1 = reached the draw.
-__device__ __noinline__ int fov_reach_exact(double cx, double cy, double phi, double theta, double rs,
-                                            double qx, double qy) {
+// the reference: returns 0 = not in range/sector, 1 = reached the draw.  The test itself is inline for callers
+// outside the step (the renderer): ptxas allocates registers across every caller of an out-of-line function, so
+// a new caller of `fov_reach_exact` would change the step kernel's code.
+__device__ __forceinline__ int fov_reach_test(double cx, double cy, double phi, double theta, double rs,
+                                              double qx, double qy) {
     const double relx = qx - cx, rely = qy - cy;
     const double dist = norm2(relx, rely);
     if (dist > rs) return 0;
@@ -540,6 +542,10 @@ __device__ __noinline__ int fov_reach_exact(double cx, double cy, double phi, do
     ra = fmin(ra, 360.0 - ra);
     if (ra * 2.0 > theta) return 0;
     return 1;
+}
+__device__ __noinline__ int fov_reach_exact(double cx, double cy, double phi, double theta, double rs,
+                                            double qx, double qy) {
+    return fov_reach_test(cx, cy, phi, theta, rs, qx, qy);
 }
 
 // Conservative occlusion classification of the query point q = cam + rel against all obstacle

@@ -33,7 +33,7 @@ from mate_b200 import spaces
 from mate_b200.config import DEFAULT_CONFIG_FILE, flatten_config, read_config
 from mate_b200.entities import CameraView, ObstacleView, TargetView
 from mate_b200.messages import Message, Team
-from mate_b200.sim import BatchedSim, check_observation_dtype, check_observed_team
+from mate_b200.sim import BatchedSim, check_index_map, check_observation_dtype, check_observed_team, check_render_size
 
 __all__ = ['MultiAgentTracking', 'EnvMeta', 'Message', 'Team', 'read_config', 'DEFAULT_CONFIG_FILE']
 
@@ -60,7 +60,7 @@ class EnvMeta(type):
 class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instance-attributes,too-many-public-methods
     """Batched Multi-Agent Tracking Environment (cameras vs. cargo-hauling targets)."""
 
-    metadata = {'render.modes': []}
+    metadata = {'render.modes': ['rgb_array']}
     DEFAULT_CONFIG_FILE = DEFAULT_CONFIG_FILE
     spec = None
     _sim_class = BatchedSim   # the simulator behind the class (tests substitute a recorded one to exercise this host layer without a GPU)
@@ -433,7 +433,8 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
         return routed
 
     def add_render_callback(self, name: str, callback) -> None:
-        """Kept for wrappers that register one (mate/environment.py:1181-1186); never called: there is no renderer."""
+        """Kept for wrappers that register one (mate/environment.py:1181-1186); never called: the callbacks draw pyglet
+        geometry, and ``render`` draws its frames on the GPU."""
         self.render_callbacks[name] = callback
 
     def joint_observation(self):
@@ -655,8 +656,26 @@ class MultiAgentTracking(metaclass=EnvMeta):  # pylint: disable=too-many-instanc
             'mean_delivered': values[3] / episodes, 'mean_coverage': values[4] / episodes, 'env_steps': values[5],
         }
 
-    def render(self, mode='human', **kwargs):
-        raise NotImplementedError('rendering is outside the B200 step path (see DESIGN.md, out of scope)')
+    def render(self, mode='human', window_size=800, envs=None):
+        """An ``rgb_array`` frame of the current state, drawn on the GPU (DESIGN.md section 7k): the terrain, warehouses,
+        the cameras' fields of view (darker where several cameras overlap), obstacles, cameras and targets (filled with
+        the goal warehouse's colour when loaded, ringed when tracked).  Single environment: NumPy uint8
+        ``[window_size, window_size, 3]``, the reference's type.  Batched: a CUDA uint8 tensor ``[K, S, S, 3]`` of the
+        environments ``envs`` (default: environment 0 only), written on the current stream.  ``mode='human'`` (a
+        window) is not supported.  The registered ``render_callbacks`` are kept but never called: they draw pyglet
+        geometry."""
+        if mode != 'rgb_array':
+            raise NotImplementedError(f"render mode {mode!r} is not supported: this environment has no window; use "
+                                      "render(mode='rgb_array') for frames")
+        if self._needs_reset:
+            raise RuntimeError('call reset() before render()')
+        if not self.batched and envs is not None:
+            raise ValueError('envs applies to the batched mode (num_envs=B)')
+        check_render_size(window_size)
+        envs = [0] if envs is None else envs
+        check_index_map(envs, 'envs', None, 0, self.num_envs)
+        frames = self.sim.render(envs, size=window_size)
+        return frames if self.batched else frames[0].cpu().numpy()
 
     def close(self) -> None:
         self.sim.close()

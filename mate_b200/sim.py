@@ -70,6 +70,36 @@ def check_observed_team(team, num_cameras=None):
     return team
 
 
+def check_index_map(index, name, length, low, high):
+    """The checks of an environment / snapshot index map, before any library call: 1-D integers, ``length`` of them if
+    given, and for a host sequence (or CPU tensor) each in ``[low, high)``, else ``ValueError``.  Returns the host indices
+    as a NumPy array, or ``None`` for ``None`` and for a device tensor (its entries are not read here)."""
+    if index is None:
+        return None
+    if torch.is_tensor(index) and index.is_cuda:
+        if index.dtype.is_floating_point or index.dtype.is_complex or index.dtype == torch.bool:
+            raise ValueError(f'{name} must hold integers, got {index.dtype}')
+        host = None
+    else:
+        host = index.numpy() if torch.is_tensor(index) else np.asarray(index)
+        if host.dtype.kind not in 'iu':
+            raise ValueError(f'{name} must hold integers, got {host.dtype}')
+    size = tuple(index.shape) if host is None else host.shape
+    if len(size) != 1 or size[0] == 0 or (length is not None and size[0] != length):
+        raise ValueError(f'{name} must be a 1-D sequence of {length if length is not None else "one or more"} indices, got shape {size}')
+    if host is not None and (host.min() < low or host.max() >= high):
+        raise ValueError(f'{name} has entries outside [{low}, {high})')
+    return host
+
+
+def check_render_size(size):
+    """The edge of a rendered frame in pixels: an integer in ``[MATE_RENDER_MIN_SIZE, MATE_RENDER_MAX_SIZE]``, else
+    ``ValueError``."""
+    if isinstance(size, bool) or not isinstance(size, (int, np.integer)) or not _abi.RENDER_MIN_SIZE <= size <= _abi.RENDER_MAX_SIZE:
+        raise ValueError(f'the frame size must be an integer in [{_abi.RENDER_MIN_SIZE}, {_abi.RENDER_MAX_SIZE}], got {size!r}')
+    return int(size)
+
+
 class StateSnapshot:
     """The complete state of some environments of a batch, saved on the device (:meth:`BatchedSim.save_state`).
 
@@ -367,6 +397,20 @@ class BatchedSim:
                                                           angle.numel(), self._stream()))
         return out
 
+    def render(self, envs=None, size=800):
+        """``rgb_array`` frames of the environments ``envs`` (``None`` = every environment, entry i = environment
+        ``envs[i]``), drawn from the current state by a CUDA kernel (mate_b200_render, the picture is defined in
+        ``include/mate_b200.h``): a new uint8 tensor ``[K, size, size, 3]`` on the simulator's device, written on the
+        current stream without a synchronisation.  Host indices are checked here; the frame of an out-of-range device index
+        is left unwritten."""
+        size = check_render_size(size)
+        index = self._index_map(envs, 'envs', None, 0, self.B)
+        count = self.B if index is None else int(index.numel())
+        out = torch.empty((count, size, size, 3), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _check(self.lib, self.lib.mate_b200_render(self.handle, _dptr(index), count, size, _dptr(out), self._stream()))
+        return out
+
     def soft_coverage(self, auto_reset=True):
         """``AuxiliaryCameraRewards.compute_soft_coverage_scores`` for the current state and the camera-target masks
         of the last step: ``[B, Nc, Nt]`` float32 (mate_b200_soft_coverage).  With ``auto_reset`` the environments
@@ -429,27 +473,14 @@ class BatchedSim:
         _check(self.lib, self.lib.mate_b200_set_state(self.handle, ctypes.byref(view)))
 
     def _index_map(self, index, name, length, low, high):
-        """Environment / snapshot indices as an int32 tensor on the simulator's device (``None`` stays ``None``).  A host
-        sequence (or CPU tensor) is checked here: 1-D integers, ``length`` of them if given, each in ``[low, high)``,
-        else ``ValueError`` before any library call.  A device tensor is passed on without a synchronisation: the
-        library's kernels skip entries that are out of range."""
+        """Environment / snapshot indices as an int32 tensor on the simulator's device (``None`` stays ``None``), checked
+        by :func:`check_index_map`.  A device tensor is passed on without a synchronisation: the library's kernels skip
+        entries that are out of range."""
+        host = check_index_map(index, name, length, low, high)
         if index is None:
             return None
-        if torch.is_tensor(index) and index.is_cuda:
-            if index.dtype.is_floating_point or index.dtype.is_complex or index.dtype == torch.bool:
-                raise ValueError(f'{name} must hold integers, got {index.dtype}')
-            host = None
-        else:
-            host = index.numpy() if torch.is_tensor(index) else np.asarray(index)
-            if host.dtype.kind not in 'iu':
-                raise ValueError(f'{name} must hold integers, got {host.dtype}')
-        size = tuple(index.shape) if host is None else host.shape
-        if len(size) != 1 or size[0] == 0 or (length is not None and size[0] != length):
-            raise ValueError(f'{name} must be a 1-D sequence of {length if length is not None else "one or more"} indices, got shape {size}')
         if host is None:
             return index.to(self.device, torch.int32).contiguous()
-        if host.min() < low or host.max() >= high:
-            raise ValueError(f'{name} has entries outside [{low}, {high})')
         return torch.from_numpy(host.astype(np.int32)).to(self.device)
 
     def snapshot_bytes(self, count):
