@@ -531,11 +531,14 @@ __device__ __forceinline__ double sight_range_quad(const ObsRef ob, double cx, d
 // Camera.perceive (mate/entities.py:491-505) up to the stochastic draw, exact arithmetic of
 // the reference: returns 0 = not in range/sector, 1 = reached the draw.  The test itself is inline for callers
 // outside the step (the renderer): ptxas allocates registers across every caller of an out-of-line function, so
-// a new caller of `fov_reach_exact` would change the step kernel's code.
+// a new caller of `fov_reach_exact` would change the step kernel's code.  The distance is rounded like the C oracle
+// (oracle/mate_oracle.c, built with -ffp-contract=off) rounds it, without contracting the sum of squares into an FMA: a
+// target exactly on the arc of the sight range is one unit in the last place outside or inside depending on that
+// rounding.  (The Python reference's np.linalg.norm goes through a BLAS dot product, whose rounding is its own.)
 __device__ __forceinline__ int fov_reach_test(double cx, double cy, double phi, double theta, double rs,
                                               double qx, double qy) {
     const double relx = qx - cx, rely = qy - cy;
-    const double dist = norm2(relx, rely);
+    const double dist = sqrt(__dadd_rn(__dmul_rn(relx, relx), __dmul_rn(rely, rely)));
     if (dist > rs) return 0;
     const double ang = atan2_deg(rely, relx);
     double ra = fabs(phi - ang);

@@ -146,11 +146,12 @@ __device__ __forceinline__ void prefetch_discs64(const Params& p, int er) {
 }
 
 // ---- out-of-line exact (fp64) decisions, state re-read from global memory -------------------
-// ||a - b|| <= thr (or <), entities a / b given by their SoA rows
+// ||a - b|| <= thr (or <), entities a / b given by their SoA rows.  The sum of squares is not contracted into an FMA, like
+// fov_reach_test: a partner exactly at the sight range is decided by the rounding of the C oracle.
 __device__ __noinline__ bool sense_exact(const double* ax, const double* ay, const double* bx, const double* by,
                                          double thr, bool strict) {
     const double ex = *ax - *bx, ey = *ay - *by;
-    const double d2 = ex * ex + ey * ey, t2 = thr * thr;
+    const double d2 = __dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)), t2 = thr * thr;
     return strict ? dist_lt(d2, thr, t2 * (1.0 - 1e-12), t2 * (1.0 + 1e-12)) : dist_le(d2, thr, t2 * (1.0 - 1e-12), t2 * (1.0 + 1e-12));
 }
 

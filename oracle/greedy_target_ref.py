@@ -7,15 +7,11 @@ import numpy as np
 WAREHOUSES = np.array([[925.0, 925.0], [-925.0, 925.0], [-925.0, -925.0], [925.0, -925.0]])   # constants.py:70-72
 
 
-def team_step(xy, step_size, goal_bits, empty_bits, memory, draws, noise_scale):
-    """One group_step of the Nt target agents of one environment.
-
-    xy [Nt, 2], step_size [Nt], goal_bits [Nt, 4] (weights), empty_bits [Nt, 4] bool: the agents' private states;
-    memory = dict(goal [Nt], non_empty [Nt] bit sets, prev_xy [Nt, 2], prev_noise [Nt, 2]) BEFORE the step;
-    draws = dict(binomial [Nt], sample [Nt, 2], choice [Nt]) recorded outcomes.  Returns (actions [Nt, 2], memory after)."""
-    nt = len(xy)
-    goal = memory['goal'].copy()
-    non_empty = memory['non_empty'].copy()
+def communicated_non_empty(empty_bits, non_empty):
+    """The remembered non-empty warehouse sets [Nt] after observe -> process_messages -> communicate, from the sets
+    before the step; the goal choice of the act phase draws from these."""
+    nt = len(empty_bits)
+    non_empty = non_empty.copy()
     # observe -> process_messages (greedy.py:330-336)
     sends = np.zeros(nt, dtype=bool)
     for t in range(nt):
@@ -28,6 +24,18 @@ def team_step(xy, step_size, goal_bits, empty_bits, memory, draws, noise_scale):
     for t in range(nt):
         for s in sent:
             non_empty[t] &= s
+    return non_empty
+
+
+def team_step(xy, step_size, goal_bits, empty_bits, memory, draws, noise_scale):
+    """One group_step of the Nt target agents of one environment.
+
+    xy [Nt, 2], step_size [Nt], goal_bits [Nt, 4] (weights), empty_bits [Nt, 4] bool: the agents' private states;
+    memory = dict(goal [Nt], non_empty [Nt] bit sets, prev_xy [Nt, 2], prev_noise [Nt, 2]) BEFORE the step;
+    draws = dict(binomial [Nt], sample [Nt, 2], choice [Nt]) recorded outcomes.  Returns (actions [Nt, 2], memory after)."""
+    nt = len(xy)
+    goal = memory['goal'].copy()
+    non_empty = communicated_non_empty(empty_bits, memory['non_empty'])
     # act (greedy.py:289-328)
     actions = np.zeros((nt, 2))
     noise_out = np.zeros((nt, 2))

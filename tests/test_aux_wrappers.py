@@ -20,13 +20,27 @@ def terms_numpy(g, i):
     """Plain restatement of the terms (auxiliary_camera_rewards.py:140-149, auxiliary_target_rewards.py:135-177,
     more_training_information.py:61-82) from the recorded after-step pieces of sample i."""
     nc, nt, _ = (int(x) for x in g['cfg_counts'])
-    mask_ct, mask_tc = g['a_out_mask_ct'][i].astype(bool), g['a_out_mask_tc'][i].astype(bool)
-    cov = g['a_out_tgt_terms'][i][0, 1:4]
+    return terms_of(nc, nt, g['a_out_team_reward'][i], g['a_out_tgt_terms'][i][0, 1:4], g['a_out_mask_ct'][i], g['a_out_mask_tc'][i],
+                    g['a_out_tgt_xy'][i], g['a_out_tgt_empty_bits'][i], g['a_out_tgt_goal'][i], g['a_out_tgt_individual_done'][i],
+                    g['a_out_tgt_is_colliding'][i])
+
+
+def terms_of(nc, nt, team_reward, cov, mask_ct, mask_tc, xy, empty, goal, individual_done, is_colliding, soft=None):
+    """The terms of one environment: ``team_reward`` [2], ``cov`` the three coverage rates, masks [Nc, Nt] / [Nt, Nc],
+    target locations [Nt, 2], empty bits [Nt, 4], goals, individual done and collision flags [Nt]; ``soft`` [Nc, Nt]
+    (``None``: the soft_coverage_score columns stay 0) aggregated like auxiliary_camera_rewards.py:130-138 and
+    auxiliary_target_rewards.py:151-162."""
+    mask_ct, mask_tc = np.asarray(mask_ct).astype(bool), np.asarray(mask_tc).astype(bool)
+    cam_soft, tgt_soft = np.zeros(nc), np.zeros(nt)
+    if soft is not None and nc:
+        soft = np.asarray(soft, dtype=np.float64)
+        cam_soft = np.where(mask_ct.any(-1), (soft * mask_ct).sum(-1), np.tanh(soft.max(-1)))
+        tgt_soft = np.where(mask_ct.any(-2), (soft * mask_ct).sum(-2), np.tanh(soft.max(-2)))
     cam = np.zeros((nc, 8))
     for c in range(nc):
-        cam[c] = [g['a_out_team_reward'][i][0], cov[0], cov[1], cov[2], 0.0, mask_ct[c].sum(), 1.0, mask_tc[:, c].any()]
+        cam[c] = [team_reward[0], cov[0], cov[1], cov[2], cam_soft[c], mask_ct[c].sum(), 1.0, mask_tc[:, c].any()]
     tgt = np.zeros((nt, 16))
-    xy, empty, goal = g['a_out_tgt_xy'][i], g['a_out_tgt_empty_bits'][i].astype(bool), g['a_out_tgt_goal'][i]
+    empty = np.asarray(empty).astype(bool)
     for t in range(nt):
         wd = np.maximum(np.linalg.norm(xy[t] - WAREHOUSES, axis=-1) - 75.0, 0.0)
         if goal[t] >= 0:
@@ -35,8 +49,8 @@ def terms_numpy(g, i):
             goal_distance = wd[~empty[t]].min()
         else:
             goal_distance = 1000.0
-        tgt[t, :10] = [g['a_out_team_reward'][i][1], cov[0], cov[1], cov[2], goal_distance / 2000.0, g['a_out_tgt_individual_done'][i][t],
-                       0.0, mask_ct[:, t].any() if nc else 0.0, g['a_out_tgt_is_colliding'][i][t], 1.0]
+        tgt[t, :10] = [team_reward[1], cov[0], cov[1], cov[2], goal_distance / 2000.0, individual_done[t],
+                       tgt_soft[t], mask_ct[:, t].any() if nc else 0.0, is_colliding[t], 1.0]
         tgt[t, 10] = goal[t]
         tgt[t, 11] = wd[goal[t]] if goal[t] >= 0 else 1000.0
         tgt[t, 12:16] = wd

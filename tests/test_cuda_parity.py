@@ -126,7 +126,7 @@ def _goal_seeking_actions(rng, cfg, state, B, noise=0.3):
 
 
 CASES = [
-    # preset, B, steps, overrides
+    # preset, B, steps, overrides[, warp tile (MATE_B200_TILE)]; every compiled shape (tests/test_shape_matrix.py)
     ('MATE-4v8-9.yaml', 512, 160, {}),
     ('MATE-4v8-9.yaml', 256, 120, {'max_episode_steps': 37}),      # time-limit done + auto-reset
     ('MATE-8v8-9.yaml', 256, 100, {}),
@@ -136,15 +136,38 @@ CASES = [
     ('MATE-2v4-9.yaml', 130, 100, {'max_episode_steps': 51}),
     ('MATE-1v1-9.yaml', 200, 100, {}),
     ('MATE-4v4-0.yaml', 64, 60, {}),
+    ('MATE-1v1-0.yaml', 203, 90, {'max_episode_steps': 29}),
+    ('MATE-1v2-0.yaml', 157, 90, {}),                              # camera rows of 39 floats: scalar stores
+    ('MATE-1v2-9.yaml', 131, 90, {'max_episode_steps': 41}),       # camera rows of 75 floats: scalar stores
+    ('MATE-2v2-0.yaml', 99, 90, {'max_episode_steps': 33}),        # 4-float camera / 2-float target stores
+    ('MATE-2v2-9.yaml', 173, 90, {}),
+    ('MATE-2v4-0.yaml', 117, 90, {'max_episode_steps': 43}),
+    ('MATE-4v2-0.yaml', 101, 90, {}),
+    ('MATE-4v4-9.yaml', 141, 90, {'max_episode_steps': 39}),       # dense block copy, all three obstacle-round classes
+    ('MATE-8v8-0.yaml', 67, 80, {}),
+    # the odd-row shapes again in the warp tiles of large batches: below 8192 environments the step runs in tiles of 8
+    # (mate_sim_create), so every case above does, and MATE_B200_TILE picks 32 (from 24 576 environments on) or 16 here
+    ('MATE-1v1-0.yaml', 77, 60, {'max_episode_steps': 23}, 32),
+    ('MATE-1v2-0.yaml', 45, 60, {}, 32),
+    ('MATE-1v2-9.yaml', 53, 60, {'max_episode_steps': 27}, 32),
+    ('MATE-2v2-0.yaml', 39, 60, {}, 32),
+    ('MATE-2v2-9.yaml', 61, 60, {'max_episode_steps': 25}, 32),
+    ('MATE-1v2-9.yaml', 83, 60, {}, 16),
+    ('MATE-2v2-0.yaml', 71, 60, {'max_episode_steps': 31}, 16),
 ]
+# the ids of the cases without a tile stay those pytest gave the four-field tuples
+CASE_PARAMS = [case if len(case) == 5 else case + (None,) for case in CASES]
+CASE_IDS = [f'{p}-{b}-{s}-overrides{i}' + (f'-tile{tile}' if tile else '') for i, (p, b, s, _, tile) in enumerate(CASE_PARAMS)]
 
 
-@pytest.mark.parametrize('preset,B,steps,overrides', CASES)
-def test_cuda_vs_oracle(preset, B, steps, overrides):
+@pytest.mark.parametrize('preset,B,steps,overrides,tile', CASE_PARAMS, ids=CASE_IDS)
+def test_cuda_vs_oracle(preset, B, steps, overrides, tile, monkeypatch):
     """Reset + step + auto-reset on the GPU against the float64 C oracle, same Philox streams."""
     from mate_b200.config import flatten_config, read_config
     from oracle.oracle import Oracle
 
+    if tile:
+        monkeypatch.setenv('MATE_B200_TILE', str(tile))
     cfg = flatten_config(read_config(preset, **overrides))
     nc = cfg['num_cameras']
     seed = 1234
