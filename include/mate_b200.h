@@ -289,7 +289,10 @@ int mate_b200_episode_stats(MateSim* sim, float* out16, int32_t reset_after, voi
  *   MATE_OBS_SHARED_CAMERA / _TARGET    SharedFieldOfView.observation,   mate/wrappers/shared_field_of_view.py:74-145
  *   MATE_OBS_RELATIVE                   convert_coordinates,  mate/agents/utils.py:40-94  (RelativeCoordinates)
  *   MATE_OBS_RESCALED                   normalize_observation, mate/agents/utils.py:97-127 (RescaledObservation)
- * `ops` is a HOST array of num_ops <= MATE_MAX_OBS_OPS codes.  cam_affine [Dc][2] / tgt_affine [Dt][2] are dev
+ * `ops` is a HOST array of num_ops <= MATE_MAX_OBS_OPS codes, in the order the reference's wrappers admit:
+ *   (ENHANCED_* | SHARED_*)*  RELATIVE?  RESCALED?
+ * i.e. no mask code after RELATIVE or RESCALED, neither of those twice, and no RELATIVE after RESCALED; any other
+ * sequence is MATE_EINVAL and leaves the registered wrappers as they were.  cam_affine [Dc][2] / tgt_affine [Dt][2] are dev
  * arrays of (scale, shift) per observation column, needed (non-NULL) only with MATE_OBS_RESCALED.  cam_obs /
  * tgt_obs must hold the observations the last step/reset/observe call wrote for this handle.  float32 handles only
  * (MATE_EINVAL after MATE_OBS_FORMAT_F16). */
@@ -299,7 +302,7 @@ int mate_b200_episode_stats(MateSim* sim, float* out16, int32_t reset_after, voi
 #define MATE_OBS_SHARED_TARGET 4
 #define MATE_OBS_RELATIVE 5
 #define MATE_OBS_RESCALED 6
-#define MATE_MAX_OBS_OPS 8
+#define MATE_MAX_OBS_OPS 8   /* codes per stack, ordered (ENHANCED_* | SHARED_*)* RELATIVE? RESCALED? (above) */
 int mate_b200_transform_observations(MateSim* sim, float* cam_obs, float* tgt_obs, const int32_t* ops,
                                      int32_t num_ops, const float* cam_affine, const float* tgt_affine,
                                      void* stream);
@@ -307,7 +310,8 @@ int mate_b200_transform_observations(MateSim* sim, float* cam_obs, float* tgt_ob
 /* The same wrappers REGISTERED with the simulator: from now on every mate_b200_reset / _step / _step_host / _observe
  * applies them to an environment's rows while they are still in shared memory (the packer of the step kernel), i.e.
  * without the extra read + write pass over the observation tensors mate_b200_transform_observations costs.
- * num_ops = 0 unregisters.  The affine tables must stay valid until they are replaced. */
+ * num_ops = 0 unregisters.  The same order rule holds: a refused sequence leaves the registered wrappers in effect.
+ * The affine tables must stay valid until they are replaced. */
 int mate_b200_set_observation_ops(MateSim* sim, const int32_t* ops, int32_t num_ops,
                                   const float* cam_affine, const float* tgt_affine);
 

@@ -475,15 +475,21 @@ static int check_launch(const char* what) {
     return MATE_OK;
 }
 
-// the observation wrapper codes as an ObsOps (the count has been checked)
+// the observation wrapper codes as an ObsOps (the count has been checked), in the order the reference admits:
+// (Enhanced | Shared)* Relative? Rescaled? (MATE_MAX_OBS_OPS, include/mate_b200.h)
 static int parse_obs_ops(const MateSim* sim, const int32_t* ops, int32_t num_ops, const float* cam_affine, const float* tgt_affine,
                          ObsOps* o) {
     *o = ObsOps{};
     o->n = num_ops;
+    int stage = 0;   // 0 = mask codes, 1 = after MATE_OBS_RELATIVE, 2 = after MATE_OBS_RESCALED
     for (int i = 0; i < num_ops; ++i) {
         if (ops[i] < MATE_OBS_ENHANCED_CAMERA || ops[i] > MATE_OBS_RESCALED) return fail(MATE_EINVAL, "unknown observation wrapper code");
         if (ops[i] == MATE_OBS_RESCALED && (!tgt_affine || (sim->cfg.num_cameras > 0 && !cam_affine)))
             return fail(MATE_EINVAL, "MATE_OBS_RESCALED needs the affine tables");
+        const int at = ops[i] == MATE_OBS_RESCALED ? 2 : (ops[i] == MATE_OBS_RELATIVE ? 1 : 0);
+        if (at < stage || (at > 0 && at == stage))
+            return fail(MATE_EINVAL, "observation wrappers must be stacked as (Enhanced | Shared)* Relative? Rescaled?");
+        stage = at;
         o->op[i] = ops[i];
     }
     return MATE_OK;
@@ -554,13 +560,13 @@ extern "C" int mate_b200_set_observation_ops(MateSim* sim, const int32_t* ops, i
     if (num_ops < 0 || num_ops > MATE_MAX_OBS_OPS) return fail(MATE_EINVAL, "too many observation wrappers (MATE_MAX_OBS_OPS)");
     ObsOps o;
     if (int rc = parse_obs_ops(sim, ops, num_ops, cam_affine, tgt_affine, &o)) return rc;
-    // canonical stacks -- (Enhanced | Shared)* Relative? Rescaled? -- are applied while the rows are composed (FoldOps)
+    // the stack -- (Enhanced | Shared)* Relative? Rescaled?, checked above -- is applied while the rows are composed (FoldOps)
     FoldOps f{};
     int k = 0;
     while (k < num_ops && ops[k] >= MATE_OBS_ENHANCED_CAMERA && ops[k] <= MATE_OBS_SHARED_TARGET) f.mask_op[f.n_mask++] = ops[k++];
     if (k < num_ops && ops[k] == MATE_OBS_RELATIVE) { f.relative = 1; ++k; }
     if (k < num_ops && ops[k] == MATE_OBS_RESCALED) { f.rescaled = 1; ++k; }
-    f.fast = (num_ops > 0 && k == num_ops) ? 1 : 0;
+    f.fast = num_ops > 0 ? 1 : 0;
     if (f.fast && f.rescaled) {
         CUDA_TRY(cudaSetDevice(sim->device));
         const int nc = sim->cfg.num_cameras;

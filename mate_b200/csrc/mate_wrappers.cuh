@@ -139,7 +139,10 @@ __device__ __forceinline__ void apply_obs_ops(const Params& p, const ObsOps& ops
             __syncwarp();
         } else if (op == MATE_OBS_RELATIVE) {
             // locations still hold the simulator's values unless a rescale came first: subtract in fp64 from
-            // the state (entity - observer), else in place on whatever the entries hold now
+            // the state (entity - observer), else in place on whatever the entries hold now.  parse_obs_ops refuses
+            // RESCALED before RELATIVE, so `exact` always holds; the in-place branch stays only because removing it
+            // changes the register allocation of every step kernel, wrapper-free launches included (measured 0.15 -
+            // 0.3 % slower on a B200 at 1000 W)
             bool exact = true;
             for (int j = 0; j < i; ++j) exact = exact && ops.op[j] != MATE_OBS_RESCALED;
             auto relative = [&](auto k, float* row, const int r, const int idx, const int off) {

@@ -57,6 +57,24 @@ def check_observation_dtype(dtype):
     return dtype
 
 
+def check_observation_ops(ops):
+    """Observation wrapper codes (``_abi.OBS_*``) as a list of ints, else ``ValueError``: at most ``MAX_OBS_OPS`` known
+    codes in the order the reference's wrappers admit, ``(Enhanced | Shared)* Relative? Rescaled?`` (no mask code after
+    ``OBS_RELATIVE`` or ``OBS_RESCALED``, neither of those twice, no ``OBS_RELATIVE`` after ``OBS_RESCALED``)."""
+    ops = [int(op) for op in ops]
+    if len(ops) > _abi.MAX_OBS_OPS:
+        raise ValueError(f'at most {_abi.MAX_OBS_OPS} observation wrappers can be stacked')
+    stage = 0   # 0 = mask codes, 1 = after OBS_RELATIVE, 2 = after OBS_RESCALED
+    for op in ops:
+        if not _abi.OBS_ENHANCED_CAMERA <= op <= _abi.OBS_RESCALED:
+            raise ValueError(f'unknown observation wrapper code {op}')
+        at = {_abi.OBS_RELATIVE: 1, _abi.OBS_RESCALED: 2}.get(op, 0)
+        if at < stage or (at > 0 and at == stage):
+            raise ValueError(f'observation wrappers must be stacked as (Enhanced | Shared)* Relative? Rescaled?, got {ops}')
+        stage = at
+    return ops
+
+
 OBSERVED_TEAMS = ('both', 'camera', 'target')
 
 
@@ -235,9 +253,7 @@ class BatchedSim:
         """Observation wrapper codes (``_abi.OBS_*``), innermost first.  They are registered with the simulator
         (``mate_b200_set_observation_ops``): every reset / step / observe applies them to an environment's rows while
         the rows are still in shared memory, at no extra pass over the observation tensors."""
-        ops = [int(op) for op in ops]
-        if len(ops) > _abi.MAX_OBS_OPS:
-            raise ValueError(f'at most {_abi.MAX_OBS_OPS} observation wrappers can be stacked')
+        ops = check_observation_ops(ops)
         self._obs_ops = ops
         self._obs_ops_c = (ctypes.c_int32 * max(len(ops), 1))(*ops)
         if _abi.OBS_RESCALED in ops and self._affine is None:

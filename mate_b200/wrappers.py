@@ -145,6 +145,7 @@ class RelativeCoordinates(_ObservationWrapper):
 
     def __init__(self, env):
         assert not _has_wrapper(env, RelativeCoordinates), f'You should not use wrapper `{type(self)}` more than once.'
+        assert not _has_wrapper(env, RescaledObservation), f'You should use wrapper `{type(self)}` before `RescaledObservation`.'
         super().__init__(env)
         self._register([_abi.OBS_RELATIVE])
 
